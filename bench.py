@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload sym_solve3|sym_solve6|sym_invert6|sym_solve10|dense_inv4_f64|...]
+                    [--dump-outputs DIR]
 
 Metric (BASELINE.json): batched sym-solve matrices/s and achieved HBM GB/s
 vs peak.  A "step" is one pass of the hot path over the whole workload:
@@ -40,6 +41,7 @@ if ROOT not in sys.path:
 import torch  # noqa: E402
 
 L2_BYTES = 126 << 20
+DUMP_BUDGET = 60 << 20      # --dump-outputs: bytes written per invocation, all workloads and ranks together
 FALLBACK_HBM_GBS = 6650.0   # /opt/skills/guides/B200_PROFILING.md fallback
 
 # name -> (kind, n, dtype, voxels-per-side or batch, description)
@@ -130,6 +132,22 @@ def make_inputs(kind: str, n: int, dtype: torch.dtype, batch: int, device, seed:
     return [a]
 
 
+def operand_set_count(set_bytes: int) -> int:
+    """Distinct operand sets the steps rotate through: enough that consecutive steps never
+    find their data in L2 (one if a set is already several times L2)."""
+    return 1 if set_bytes >= 3 * L2_BYTES else min(8, math.ceil(3 * L2_BYTES / max(set_bytes, 1)))
+
+
+def operand_seed(rank: int, s: int) -> int:
+    """``make_inputs`` seed of operand set ``s`` of ``rank``."""
+    return 1000 * rank + s
+
+
+def timed_set(warmup: int, step: int, nsets: int) -> int:
+    """Operand set of timed step ``step`` (0-based): the rotation continues from the warm-up."""
+    return (warmup + step) % nsets
+
+
 ALGOS = {"auto": 0, "ldl": 1, "lu": 2, "warp": 3}
 
 
@@ -178,8 +196,8 @@ _REFERENCE = None
 
 def reference_impl():
     """(kind label, module-like namespace of callables): the reference's OWN code when it
-    can be imported (baseline/_ref, installed by oracle/install_reference.py; or
-    /root/reference in the build container), else the oracle port."""
+    can be imported (baseline/_ref, installed by oracle/install_reference.py, or the
+    directory NFM_REFERENCE_ROOT names), else the oracle port."""
     global _REFERENCE
     if _REFERENCE is None:
         try:
@@ -395,7 +413,16 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=None)
     ap.add_argument("--workloads", default=None,
                     help="comma-separated list: several workloads in one process, one JSON line each (saves start-up on multi-GPU boxes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output of the last timed step, shaped as the public API returns it, "
+                         "as DIR/<workload>.npy "
+                         "(DIR/<workload>.rank<R>.npy per rank when N > 1), in the workload's dtype; outputs above "
+                         f"{DUMP_BUDGET >> 20} MiB in all are cut to a fixed, seeded sample of rows (in ascending order)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -416,13 +443,27 @@ def main():
         if name not in WORKLOADS:
             raise SystemExit(f"unknown workload {name}")
         args.workload = name
-        run_workload(args, rank, local_rank, world, dist)
+        run_workload(args, rank, local_rank, world, dist, DUMP_BUDGET // (len(names) * world))
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
 
 
-def run_workload(args, rank, local_rank, world, dist):
+def dump_output(out: torch.Tensor, path: str, budget: int) -> None:
+    """Write ``out`` (one record per row) to ``path`` as .npy; above ``budget`` bytes, a
+    sample of rows drawn with a fixed seed, so that two runs with the same arguments write
+    the same rows."""
+    import numpy as np
+    rows = out.shape[0]
+    keep = max(1, budget // max(1, out[:1].numel() * out.element_size()))
+    if rows > keep:
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        out = out[idx.to(out.device)]
+    os.makedirs(os.path.dirname(path) or ".", exist_ok=True)
+    np.save(path, out.cpu().numpy())
+
+
+def run_workload(args, rank, local_rank, world, dist, dump_budget):
 
     w = dict(WORKLOADS[args.workload])
     if args.kind or args.n or args.dtype:
@@ -469,13 +510,11 @@ def run_workload(args, rank, local_rank, world, dist):
     code = 0 if dtype == torch.float32 else 1
     lens, olen = record_lengths(kind, n)
 
-    # operand sets: rotate enough distinct sets that consecutive steps never
-    # find their data in L2 (or one set if it is already several times L2)
     set_bytes = my * alg
-    nsets = 1 if set_bytes >= 3 * L2_BYTES else min(8, math.ceil(3 * L2_BYTES / max(set_bytes, 1)))
+    nsets = operand_set_count(set_bytes)
     sets = []
     for s in range(nsets):
-        ins = make_inputs(kind, n, dtype, my, dev, seed=1000 * rank + s)
+        ins = make_inputs(kind, n, dtype, my, dev, seed=operand_seed(rank, s))
         out = torch.empty(my, olen, device=dev, dtype=dtype) if olen > 1 else torch.empty(my, device=dev, dtype=dtype)
         sets.append((ins, out))
     timing["l2"] = (f"per-GPU working set {set_bytes / 2**20:.0f} MiB > L2" if nsets == 1 else
@@ -505,7 +544,7 @@ def run_workload(args, rank, local_rank, world, dist):
         step(i)
     clocks.wait_ready()
     # the timed loop is as tight as Python allows: pre-bound C-ABI calls, return codes checked afterwards
-    seq = [launchers[(args.warmup + i) % nsets] for i in range(args.steps)]
+    seq = [launchers[timed_set(args.warmup, i, nsets)] for i in range(args.steps)]
     sync()
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     rc_any = 0
@@ -549,6 +588,12 @@ def run_workload(args, rank, local_rank, world, dist):
             _lib.check(rc_any, "bench step")
         launches = _lib.launch_count() - launches0
         timing["launch"] = "eager: %d ctypes calls of the C ABI" % args.steps
+    if args.dump_outputs:
+        last_out = sets[timed_set(args.warmup, args.steps - 1, nsets)][1]
+        if kind == "batch_inv":         # the public batchinv returns (..., n, n)
+            last_out = last_out.view(my, n, n)
+        suffix = ".rank%d" % rank if world > 1 else ""
+        dump_output(last_out, os.path.join(args.dump_outputs, args.workload + suffix + ".npy"), dump_budget)
     elapsed_ms = ev0.elapsed_time(ev1)
     if dist is not None:
         t = torch.tensor([elapsed_ms], device=dev, dtype=torch.float64)

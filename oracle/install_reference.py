@@ -1,20 +1,20 @@
 #!/usr/bin/env python
 """Install the UNMODIFIED reference into the git-ignored ``baseline/_ref/`` so that
-it travels to the GPU box (where /root/reference does not exist) and
-``bench.py --impl reference`` can time the reference's own code.
+``bench.py --impl reference`` can time the reference's own code and
+``tests/test_oracle.py`` can compare the port with it bit for bit.
 
 TEST / MEASUREMENT INFRASTRUCTURE ONLY -- nothing under nitorch_fastmath_b200/
-imports it.  Run in the build container (needs /root/reference):
+imports it.  Needs a checkout of nitorch-fastmath, named by NFM_REFERENCE_SRC:
 
-    python oracle/install_reference.py
+    NFM_REFERENCE_SRC=<nitorch-fastmath checkout> python oracle/install_reference.py
 
 Steps (outcome recorded in baseline/_ref/INSTALL_LOG.txt and DESIGN.md section 7):
  1. ``pip install --no-index --no-build-isolation --no-deps --target baseline/_ref``
-    from a scratch copy of /root/reference (the source tree is read-only).
+    from a scratch copy of the checkout (which may be read-only).
  2. The reference's setup.py lists ``packages=['nitorch_fastmath']`` only, so the
     wheel omits the ``_impl`` (and ``tests``) sub-packages that ``batched.py`` and
     ``sugar.py`` import: the installed tree is completed by copying those
-    directories verbatim from /root/reference.  Nothing is edited.
+    directories verbatim from the checkout.  Nothing is edited.
 The un-vendored dependency ``jitfields`` is not installable offline; the loader
 (oracle/load_reference.py) registers an in-memory stand-in that binds the nine
 names of ``nitorch_fastmath/sym.py:30-34`` to the reference's own ``_impl/sym.py``.
@@ -28,13 +28,13 @@ import sys
 import tempfile
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SRC = os.environ.get("NFM_REFERENCE_SRC", "/root/reference")
+SRC = os.environ.get("NFM_REFERENCE_SRC", "")
 DST = os.path.join(ROOT, "baseline", "_ref")
 
 
 def main() -> int:
     if not os.path.isdir(os.path.join(SRC, "nitorch_fastmath")):
-        print(f"{SRC} not present: keeping whatever baseline/_ref holds")
+        print(f"NFM_REFERENCE_SRC={SRC!r} holds no nitorch_fastmath package: keeping whatever baseline/_ref holds")
         return 0
     shutil.rmtree(DST, ignore_errors=True)
     os.makedirs(DST, exist_ok=True)
@@ -43,7 +43,7 @@ def main() -> int:
         work = os.path.join(tmp, "reference")
         shutil.copytree(SRC, work)
         cmd = [sys.executable, "-m", "pip", "install", "--no-index", "--no-build-isolation", "--no-deps",
-               "--find-links", "/opt/wheelhouse", "--target", DST, work]
+               "--target", DST, work]
         r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
         log.append("$ " + " ".join(cmd))
         log.append(r.stdout[-2000:])

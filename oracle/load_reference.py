@@ -1,6 +1,8 @@
-"""Import the *real*, unmodified reference: from /root/reference in the build
-container, else from the git-ignored install ``baseline/_ref/`` that
-``oracle/install_reference.py`` makes (it travels to the GPU box).
+"""Import the *real*, unmodified reference: from the directory that the
+environment variable NFM_REFERENCE_ROOT names, else from the git-ignored
+install ``baseline/_ref/`` that ``oracle/install_reference.py`` makes.  The
+reference is not part of this repository; without it the callers fall back to
+the stored fixtures in ``tests/golden/`` or to the pinned port.
 
 TEST / MEASUREMENT INFRASTRUCTURE ONLY -- used by
 ``oracle/validate_against_reference.py``, ``tests/golden/make_golden.py`` and
@@ -27,10 +29,11 @@ _REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 def _find_root() -> str:
     env = os.environ.get("NFM_REFERENCE_ROOT")
-    for root in ([env] if env else []) + ["/root/reference", os.path.join(_REPO, "baseline", "_ref")]:
+    local = os.path.join(_REPO, "baseline", "_ref")
+    for root in ([env] if env else []) + [local]:
         if os.path.isfile(os.path.join(root, "nitorch_fastmath", "_impl", "sym.py")):
             return root
-    return env or "/root/reference"
+    return env or local
 
 
 REFERENCE_ROOT = _find_root()

@@ -1,13 +1,23 @@
-"""Generate the golden fixtures from the REAL reference (build container only).
+"""Generate the golden fixtures from the REAL reference.
 
-    python tests/golden/make_golden.py
+    NFM_REFERENCE_ROOT=<nitorch-fastmath checkout> python tests/golden/make_golden.py
 
-Imports /root/reference through oracle/load_reference.py, feeds it seeded
+Imports the reference through oracle/load_reference.py, feeds it seeded
 inputs and stores inputs + reference outputs in ``tests/golden/*.npz``.  The
 reference itself holds no golden vectors for this path (SURVEY.md section 8c)
-and cannot travel to the GPU box, so these files are the travelling pin:
+and is not part of this repository, so these files are the stored pin:
 tests/test_oracle.py checks the oracle against them on CPU and
 tests/test_gpu_parity.py checks the CUDA path against them on the B200.
+
+``oracle_pin_{f32,f64}.npz`` hold the inputs (samples) and reference outputs
+of the 370 checks of oracle/validate_against_reference.py; ``--oracle-pin``
+rewrites only those two files.  The copies in this repository were written
+without the reference at hand: each stored output is the output of
+oracle/ref_port.py, unchanged since commit 7225f88, where
+validate_against_reference.py found it identical to the reference on exactly
+these inputs (370 checks, 0 mismatches: 354 bit for bit, the 16 sym_matmul /
+sym_det checks to rounding).  Rewrite them with ``--oracle-pin`` where the
+reference is installed.
 """
 from __future__ import annotations
 
@@ -22,6 +32,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 
 from oracle import generators as G          # noqa: E402
 from oracle import load_reference           # noqa: E402
+from oracle import validate_against_reference  # noqa: E402
 
 BATCH = (3, 8)
 
@@ -100,9 +111,24 @@ def main():
     np.savez_compressed(os.path.join(HERE, "extra_golden.npz"), **extra)
     np.savez_compressed(os.path.join(HERE, "sym_golden.npz"), **sym)
     np.savez_compressed(os.path.join(HERE, "dense_golden.npz"), **dense)
-    for f in ("sym_golden.npz", "dense_golden.npz", "extra_golden.npz"):
+    write_oracle_pin()
+    for f in ("sym_golden.npz", "dense_golden.npz", "extra_golden.npz", "oracle_pin_f32.npz", "oracle_pin_f64.npz"):
         print(f, os.path.getsize(os.path.join(HERE, f)), "bytes")
 
 
+def write_oracle_pin():
+    """Inputs and reference outputs of every check of oracle/validate_against_reference.py,
+    replayed by tests/test_oracle.py::test_oracle_is_bit_identical_to_reference."""
+    rec = {}
+    if validate_against_reference.run(record=rec):
+        raise SystemExit("the oracle disagrees with the reference: not storing its outputs")
+    for tag in ("f32", "f64"):
+        part = {k: v for k, v in rec.items() if k.endswith(" " + tag)}
+        validate_against_reference.save_pin(os.path.join(HERE, f"oracle_pin_{tag}.npz"), part)
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["--oracle-pin"]:
+        write_oracle_pin()
+    else:
+        main()

@@ -1,11 +1,14 @@
 """The oracle (oracle/ref_port.py) against the fixtures the REAL reference
-produced (tests/golden/make_golden.py), and -- when /root/reference is
-present, i.e. in the build container -- against the reference itself, bit for
-bit.  CPU only."""
+produced (tests/golden/make_golden.py), bit for bit against the stored outputs
+of oracle/validate_against_reference.py, and -- when the unmodified reference
+is installed (oracle/load_reference.py: NFM_REFERENCE_ROOT or baseline/_ref) --
+against the reference itself.  CPU only."""
+import os
+
 import pytest
 import torch
 
-from conftest import TAGS
+from conftest import GOLDEN, TAGS
 from oracle import generators as G
 from oracle import load_reference
 from oracle import ref_port as P
@@ -101,7 +104,12 @@ def test_singular_closed_forms_do_not_raise():
     assert not torch.isfinite(x).any()
 
 
-@pytest.mark.skipif(not load_reference.available(), reason="reference not present (GPU box)")
 def test_oracle_is_bit_identical_to_reference():
-    from oracle import validate_against_reference
-    assert validate_against_reference.run(verbose=False) == 0
+    """The 370 checks of oracle/validate_against_reference.py, each at its own exactness,
+    against the reference outputs stored in tests/golden/oracle_pin_*.npz -- and against
+    the reference itself where it is installed."""
+    from oracle import validate_against_reference as V
+    stored = V.load_pin(*(os.path.join(GOLDEN, f"oracle_pin_{t}.npz") for t in ("f32", "f64")))
+    assert V.run(verbose=False, stored=stored) == 0
+    if load_reference.available():
+        assert V.run(verbose=False) == 0
