@@ -247,6 +247,43 @@ int nfm_sym_solve_update_reg(int dtype, int n, int algo, int64_t batch,
                              double lam, double alpha,
                              void *out, int64_t out_stride, void *stream);
 
+/* ---- gradients (backward passes of sym_matvec / sym_solve / sym_invert / sym_det) ----
+ * p = the stored coefficients of A, g = the incoming gradient.  S(u, w), the
+ * gradient of u^T A w with respect to p, is  S_ii = u_i w_i  and
+ * S_ij = u_i w_j + u_j w_i (i < j) in the packed layout (the diagonal is not
+ * doubled), u_i w_i in the diagonal layout and sum_i u_i w_i in the
+ * scaled-identity layout.  The gradients with respect to the vectors are the
+ * forward routines: A g (nfm_sym_matvec) and (A + diag d)^-1 g (nfm_sym_solve). */
+
+/* out = sign * S(u, w), records of 1 / n / n(n+1)/2 according to `layout`
+ * (NFM_LAYOUT_SCALED_IDENTITY, NFM_LAYOUT_DIAG or NFM_LAYOUT_SYM; sign = +1 or -1);
+ * u, w: records of n.
+ *   y = inp +/- A v :        d_p = +/- S(g, v)
+ *   x = (A + diag d)^-1 v :  d_p = -S(u, x), d_d = -S_diag(u, x)  with u = (A + diag d)^-1 g */
+int nfm_sym_outer2(int dtype, int n, int layout, int64_t batch,
+                   const void *u, int64_t u_stride,
+                   const void *w, int64_t w_stride, int sign,
+                   void *out, int64_t out_stride, void *stream);
+
+/* Gradient of B = A^-1 with respect to p:  M = B G B with G_ii = g_ii,
+ * G_ij = g_ij / 2 (G = diag(g) when diag_only != 0, the gradient of diag(A^-1));
+ * out_ii = -M_ii, out_ij = -2 M_ij.
+ * inv: the packed inverse B (records of n(n+1)/2, also when diag_only);
+ * grad: records of n(n+1)/2, or n when diag_only; out: records of n(n+1)/2. */
+int nfm_sym_invert_backward(int dtype, int n, int diag_only, int64_t batch,
+                            const void *inv, int64_t inv_stride,
+                            const void *grad, int64_t grad_stride,
+                            void *out, int64_t out_stride, void *stream);
+
+/* Gradient of t = det A with respect to p:  out_ii = g adj_ii, out_ij = 2 g adj_ij
+ * with adj = t A^-1 the adjugate.  n <= 4: closed-form adjugate (finite for
+ * singular A); n > 4: checked LDL^T with a pivoted-elimination fallback.
+ * mat, out: records of n(n+1)/2; grad: one value per matrix. */
+int nfm_sym_det_backward(int dtype, int n, int64_t batch,
+                         const void *mat, int64_t mat_stride,
+                         const void *grad, int64_t grad_stride,
+                         void *out, int64_t out_stride, void *stream);
+
 /* ---- host-buffer pipelines (end-to-end path) --------------------------- */
 
 /* Bytes of device workspace the host pipelines want for `chunk` matrices per

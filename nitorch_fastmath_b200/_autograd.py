@@ -1,0 +1,285 @@
+"""Gradients of the packed-symmetric routines (sym_matvec family, sym_solve,
+sym_invert, sym_det).
+
+The public functions in ``sym.py`` route here only when grad mode is on and a
+tensor operand requires grad; otherwise they run their plain path untouched.
+Each ``torch.autograd.Function`` runs the plain implementation in ``forward``
+and the library's backward kernels (``nfm_sym_outer2``,
+``nfm_sym_invert_backward``, ``nfm_sym_det_backward``, plus the forward
+``nfm_sym_matvec`` / ``nfm_sym_solve`` for the vector gradients) in
+``backward``, on the current stream.  torch allocates, casts between the
+compute dtype and the operands' dtypes, and sums a gradient over the batch
+dimensions its operand was broadcast along (``sum_to_size``).
+
+Notation (DESIGN.md, "Gradients"): p = the stored coefficients of A, g = the
+incoming gradient, S(u, w) = the gradient of u^T A w with respect to p.
+
+  y = inp +/- A v        d_inp = g, d_v = +/- A g, d_p = +/- S(g, v)
+  x = (A + diag d)^-1 v  u = (A + diag d)^-1 g: d_v = u, d_p = -S(u, x), d_d = -u * x
+  B = A^-1               d_p from M = B G B (nfm_sym_invert_backward)
+  t = det A              d_p = g * adjugate, off-diagonal doubled (nfm_sym_det_backward)
+
+Backward passes are once-differentiable: a second-order gradient raises.
+"""
+from __future__ import annotations
+
+from typing import Optional
+
+import torch
+from torch import Tensor
+from torch.autograd.function import once_differentiable
+
+from . import _dispatch as D
+from . import _host, _lib
+from . import sym as S
+
+
+def needs_grad(*operands) -> bool:
+    for t in operands:
+        if getattr(t, "requires_grad", False):
+            return True
+    return False
+
+
+def _layout_len(layout: int, n: int) -> int:
+    return {_lib.LAYOUT_SCALED_IDENTITY: 1, _lib.LAYOUT_DIAG: n, _lib.LAYOUT_SYM: n * (n + 1) // 2}[layout]
+
+
+def _launch(name: str, n: int, out_len: int, batch, operands, *args, before=(), dtype, device) -> Tensor:
+    """Run one backward kernel over ``batch``: every operand (trailing dim = its record) is
+    broadcast to ``batch`` and handed over as (pointer, batch stride); ``before`` / ``args`` are
+    the scalar arguments ahead of / between the operands and the output."""
+    out = torch.empty((*batch, out_len), dtype=dtype, device=device)
+    nb = D.batch_count(batch)
+    if nb > 0:
+        ops = [D.as_operand(t, batch, 1, dtype) for t in operands]
+        ptrs = [x for o in ops for x in (o.ptr, o.stride)]
+        with D.device_of(device):
+            rc = getattr(_lib.load(), name)(D.dtype_code(dtype), n, *before, nb, *ptrs, *args, out.data_ptr(), out_len,
+                                           D.current_stream_ptr(device))
+        _lib.check(rc, name)
+    return out
+
+
+def outer2(u: Tensor, w: Tensor, layout: int, sign: int) -> Tensor:
+    """``sign * S(u, w)`` in ``layout``: records of 1 / N / N(N+1)/2 over the broadcast batch of u, w."""
+    n = u.shape[-1]
+    batch = tuple(torch.broadcast_shapes(u.shape[:-1], w.shape[:-1]))
+    return _launch("nfm_sym_outer2", n, _layout_len(layout, n), batch, [u, w], sign,
+                   before=(layout,), dtype=u.dtype, device=u.device)
+
+
+def invert_backward(inv: Tensor, grad: Tensor, diag_only: bool) -> Tensor:
+    """Gradient of ``sym_invert`` with respect to the packed matrix, from the packed inverse."""
+    nn = inv.shape[-1]
+    n = D.packed_order(nn)
+    batch = tuple(torch.broadcast_shapes(inv.shape[:-1], grad.shape[:-1]))
+    return _launch("nfm_sym_invert_backward", n, nn, batch, [inv, grad],
+                   before=(int(bool(diag_only)),), dtype=inv.dtype, device=inv.device)
+
+
+def det_backward(mat: Tensor, grad: Tensor) -> Tensor:
+    """Gradient of ``sym_det`` with respect to the packed matrix; ``grad`` has the batch shape."""
+    nn = mat.shape[-1]
+    batch = tuple(torch.broadcast_shapes(mat.shape[:-1], grad.shape))
+    return _launch("nfm_sym_det_backward", D.packed_order(nn), nn, batch, [mat, grad.unsqueeze(-1)],
+                   dtype=mat.dtype, device=mat.device)
+
+
+def _work_device(dev: torch.device) -> torch.device:
+    """CPU operands compute their gradients on the CUDA device their forward streamed through."""
+    return dev if dev.type == "cuda" else _host.offload_device()
+
+
+def _grad_for(grad: Optional[Tensor], like: Tensor) -> Optional[Tensor]:
+    """Sum over the dims ``like`` was broadcast along, back to its dtype and device."""
+    if grad is None:
+        return None
+    if tuple(grad.shape) != tuple(like.shape):
+        grad = grad.sum_to_size(like.shape)
+    return grad.to(device=like.device, dtype=like.dtype)
+
+
+def _check_layout(layout: int, what: str, *operands) -> None:
+    """A full N*N `mat` is a general matrix to the kernels: its gradients (and those of the vector and the
+    regulariser of a solve) would need transposed products and solves."""
+    if layout == _lib.LAYOUT_FULL and needs_grad(*operands):
+        raise NotImplementedError(f"{what}: gradients with a full (N*N) matrix are not supported; "
+                                  "use the packed, diagonal or scaled-identity layout")
+
+
+def _check_out(out: Optional[Tensor], what: str) -> None:
+    if out is not None:
+        raise RuntimeError(f"{what}(): functions with out=... arguments don't support automatic differentiation, "
+                           "but one of the arguments requires grad")
+
+
+# ---------------------------------------------------------------------------
+# matvec family:  y = [inp +/-] A v
+# ---------------------------------------------------------------------------
+
+class _Matvec(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, inp, mat, vec, sign, dtype, inplace):
+        res = S._matvec(inp, mat, vec, sign, dtype, inp if inplace else None)
+        if inplace:
+            ctx.mark_dirty(inp)
+        ctx.save_for_backward(mat, vec)
+        ctx.sign = sign
+        ctx.cdt = D.compute_dtype(*[t for t in (mat, vec, inp) if t is not None], dtype=dtype)
+        ctx.inp_meta = None if inp is None else (inp.shape, inp.dtype, inp.device)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        mat, vec = ctx.saved_tensors
+        need_inp, need_mat, need_vec = ctx.needs_input_grad[:3]
+        dev = _work_device(vec.device)
+        cdt = ctx.cdt
+        n = vec.shape[-1]
+        g = g.to(device=dev, dtype=cdt)
+        d_inp = d_mat = d_vec = None
+        if need_inp:
+            shape, dt, idev = ctx.inp_meta
+            d_inp = g.sum_to_size(shape) if tuple(g.shape) != tuple(shape) else g
+            d_inp = d_inp.to(device=idev, dtype=dt)
+        if need_vec:
+            m = mat.to(device=dev, dtype=cdt)
+            if ctx.sign < 0:   # -A g as 0 - A g: a broadcast zero addend, no extra pass
+                d_vec = S._matvec(torch.zeros(n, dtype=cdt, device=dev), m, g, -1, cdt, None)
+            else:
+                d_vec = S._matvec(None, m, g, 0, cdt, None)
+            d_vec = _grad_for(d_vec, vec)
+        if need_mat:
+            layout = D.detect_layout(mat.shape[-1], n)
+            d_mat = _grad_for(outer2(g, vec.to(device=dev, dtype=cdt), layout, -1 if ctx.sign < 0 else 1), mat)
+        return d_inp, d_mat, d_vec, None, None, None
+
+
+def matvec(inp, mat, vec, sign: int, dtype, out, inplace: bool = False) -> Tensor:
+    what = {0: "sym_matvec", 1: "sym_addmatvec", -1: "sym_submatvec"}[sign] + ("_" if inplace else "")
+    _check_out(out, what)
+    mat, vec = torch.as_tensor(mat), torch.as_tensor(vec)
+    inp = None if inp is None else torch.as_tensor(inp)
+    _check_layout(D.detect_layout(mat.shape[-1], vec.shape[-1]), what, mat, vec)
+    return _Matvec.apply(inp, mat, vec, sign, dtype, inplace)
+
+
+# ---------------------------------------------------------------------------
+# solve:  x = (A + diag d)^-1 v
+# ---------------------------------------------------------------------------
+
+class _Solve(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, mat, vec, diag, dtype, method, inplace):
+        res = S._solve(mat, vec, diag, dtype=dtype, out=vec if inplace else None, method=method)
+        if inplace:
+            ctx.mark_dirty(vec)
+        reg_t = diag if torch.is_tensor(diag) else None
+        ctx.save_for_backward(mat, res, reg_t)
+        ctx.reg = None if reg_t is not None else diag   # scalar / sequence regulariser: no gradient
+        ctx.method = method
+        ctx.cdt = D.compute_dtype(mat, vec, dtype=dtype)
+        ctx.vec_meta = (vec.shape, vec.dtype, vec.device)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        mat, x, reg_t = ctx.saved_tensors
+        need_mat, need_vec, need_diag = ctx.needs_input_grad[:3]
+        dev = _work_device(mat.device)
+        cdt = ctx.cdt
+        m = mat.to(device=dev, dtype=cdt)
+        reg = reg_t.to(device=dev) if reg_t is not None else ctx.reg
+        u = S._solve(m, g.to(device=dev, dtype=cdt), reg, dtype=cdt, method=ctx.method)
+        d_mat = d_vec = d_diag = None
+        if need_vec:
+            shape, dt, vdev = ctx.vec_meta
+            d_vec = (u.sum_to_size(shape) if tuple(u.shape) != tuple(shape) else u).to(device=vdev, dtype=dt)
+        if need_mat or need_diag:
+            xc = x.to(device=dev, dtype=cdt)
+            layout = D.detect_layout(mat.shape[-1], x.shape[-1])
+            full = outer2(u, xc, layout, -1) if need_mat else None
+            if need_mat:
+                d_mat = _grad_for(full, mat)
+            if need_diag:
+                # -u * x, the diagonal part of d_p: the D-layout record is that already
+                dd = full if layout == _lib.LAYOUT_DIAG and full is not None else outer2(u, xc, _lib.LAYOUT_DIAG, -1)
+                d_diag = _grad_for(dd, reg_t)
+        return d_mat, d_vec, d_diag, None, None, None
+
+
+def solve(mat, vec, diag, dtype, out, eps, method, inplace: bool = False) -> Tensor:
+    what = "sym_solve_" if inplace else "sym_solve"
+    _check_out(out, what)
+    if eps is not None:
+        if diag is not None:
+            raise TypeError("give the regulariser as `diag` or as `eps`, not both")
+        diag = eps
+    mat, vec = torch.as_tensor(mat), torch.as_tensor(vec)
+    _check_layout(D.detect_layout(mat.shape[-1], vec.shape[-1]), what, mat, vec, diag)
+    return _Solve.apply(mat, vec, diag, dtype, method, inplace)
+
+
+# ---------------------------------------------------------------------------
+# invert:  B = A^-1  (or diag(A^-1))
+# ---------------------------------------------------------------------------
+
+class _Invert(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, mat, diag, dtype, method, inplace):
+        res = S._invert(mat, diag, dtype, mat if inplace else None, method=method)
+        if inplace:
+            ctx.mark_dirty(mat)
+        # the diagonal-only forward does not produce the packed inverse the backward needs:
+        # keep A and invert it again in backward
+        ctx.save_for_backward(mat if diag else res)
+        ctx.diag = bool(diag)
+        ctx.method = method
+        ctx.cdt = D.compute_dtype(mat, dtype=dtype)
+        ctx.mat_meta = (mat.shape, mat.dtype, mat.device)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        saved, = ctx.saved_tensors
+        _, dt, mdev = ctx.mat_meta
+        dev = _work_device(mdev)
+        cdt = ctx.cdt
+        inv = saved.to(device=dev, dtype=cdt)
+        if ctx.diag:
+            inv = S._invert(inv, False, cdt, method=ctx.method)
+        d = invert_backward(inv, g.to(device=dev, dtype=cdt), ctx.diag)
+        return d.to(device=mdev, dtype=dt), None, None, None, None
+
+
+def invert(mat, diag, dtype, out, method, inplace: bool = False) -> Tensor:
+    _check_out(out, "sym_invert_" if inplace else "sym_invert")
+    return _Invert.apply(torch.as_tensor(mat), diag, dtype, method, inplace)
+
+
+# ---------------------------------------------------------------------------
+# det:  t = det A
+# ---------------------------------------------------------------------------
+
+class _Det(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, mat):
+        ctx.save_for_backward(mat)
+        return S._det(mat)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        mat, = ctx.saved_tensors
+        dev = _work_device(mat.device)
+        cdt = D.compute_dtype(mat)
+        d = det_backward(mat.to(device=dev, dtype=cdt), g.to(device=dev, dtype=cdt))
+        return d.to(device=mat.device, dtype=mat.dtype)
+
+
+def det(mat) -> Tensor:
+    return _Det.apply(torch.as_tensor(mat))

@@ -222,6 +222,52 @@ int nfm_sym_invert(int dtype, int n, int algo, int diag_only, int64_t batch, con
   return nfm_sym_invert_ex(dtype, n, algo, diag_only, batch, &m, &o, stream);
 }
 
+int nfm_sym_outer2(int dtype, int n, int layout, int64_t batch, const void* u, int64_t u_stride, const void* w,
+                   int64_t w_stride, int sign, void* out, int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  if (layout < 0 || layout > 2) return fail(NFM_E_UNSUPPORTED, "layout must be scaled identity, diagonal or packed");
+  if (sign != 1 && sign != -1) return fail(NFM_E_BADARG, "sign must be +1 or -1");
+  Args a;
+  a.in(0, u, u_stride, true);
+  a.in(1, w, w_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  a.p.flags = sign < 0 ? 1 : 0;  // kFlagSubtract
+  auto s = static_cast<cudaStream_t>(stream);
+  return finish(dtype == NFM_F32 ? sym_outer2_impl<float>(n, layout, a.p, s) : sym_outer2_impl<double>(n, layout, a.p, s));
+}
+
+int nfm_sym_invert_backward(int dtype, int n, int diag_only, int64_t batch, const void* inv, int64_t inv_stride,
+                            const void* grad, int64_t grad_stride, void* out, int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  Args a;
+  a.in(0, inv, inv_stride, true);
+  a.in(1, grad, grad_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  auto s = static_cast<cudaStream_t>(stream);
+  return finish(dtype == NFM_F32 ? sym_invert_backward_impl<float>(n, diag_only, a.p, s)
+                                 : sym_invert_backward_impl<double>(n, diag_only, a.p, s));
+}
+
+int nfm_sym_det_backward(int dtype, int n, int64_t batch, const void* mat, int64_t mat_stride, const void* grad,
+                         int64_t grad_stride, void* out, int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  Args a;
+  a.in(0, mat, mat_stride, true);
+  a.in(1, grad, grad_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  auto s = static_cast<cudaStream_t>(stream);
+  return finish(dtype == NFM_F32 ? sym_det_backward_impl<float>(n, a.p, s) : sym_det_backward_impl<double>(n, a.p, s));
+}
+
 int nfm_batch_inv(int dtype, int n, int algo, int closed_form_reg, int64_t batch, const void* mat, int64_t a_stride,
                   void* out, int64_t out_stride, void* stream) {
   int rc = NFM_OK;

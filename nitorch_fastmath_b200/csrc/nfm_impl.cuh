@@ -27,6 +27,12 @@ template <typename T> int sym_invert_part0(int n, int diag_only, const KParams& 
 template <typename T> int sym_invert_part1(int n, int diag_only, const KParams& p, cudaStream_t s);
 template <typename T> int sym_invert_part2(int n, int diag_only, const KParams& p, cudaStream_t s);
 
+// backward kernels (nfm_sym_grad.cu): sign * S(u, w) in layout E / D / S, gradient of
+// sym_invert (packed or diagonal-only) and of sym_det with respect to the packed coefficients
+template <typename T> int sym_outer2_impl(int n, int layout, const KParams& p, cudaStream_t s);
+template <typename T> int sym_invert_backward_impl(int n, int diag_only, const KParams& p, cudaStream_t s);
+template <typename T> int sym_det_backward_impl(int n, const KParams& p, cudaStream_t s);
+
 // dense: part 0 = inverse (closed / Gauss-Jordan), part 1 = inverse (LDL^T) + det + matvec,
 // part 2 = solve LU, part 3 = solve LDL^T
 template <typename T> int batch_inv_lu_impl(int n, const KParams& p, cudaStream_t s);

@@ -17,6 +17,11 @@ There is no TorchScript, Triton, cupy or CPU fallback: CUDA tensors run on
 their device, CPU tensors are streamed through the current CUDA device, and
 without a CUDA device or without the built library every call raises.
 
+Gradients: sym_matvec, sym_addmatvec(_), sym_submatvec(_), sym_solve(_), sym_invert(_)
+and sym_det are differentiable (packed, diagonal and scaled-identity layouts); the
+backward passes run on the library's kernels (``_autograd.py``).  Without a needed
+gradient each function runs its plain path unchanged.
+
 Signatures are the union of the reference's in-repo implementation
 (nitorch_fastmath/_impl/sym.py) and the ``jitfields.sym`` functions that
 ``nitorch_fastmath.sym`` re-exports (sym.py:30-37).
@@ -30,6 +35,7 @@ from typing import Optional, Sequence, Union
 import torch
 from torch import Tensor
 
+from . import _autograd as A
 from . import _dispatch as D
 from . import _host, _lib
 
@@ -178,28 +184,42 @@ def sym_matvec(mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None, ou
     -------
     matvec : `(..., M) tensor`, dtype = promotion of the inputs
     """
+    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.matvec(None, mat, vec, 0, dtype, out)
     return _matvec(None, mat, vec, 0, dtype, out)
 
 
 def sym_addmatvec(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None,
                   out: Optional[Tensor] = None) -> Tensor:
     """``inp + mat @ vec``  (reference name: sym.py:31)."""
+    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
+            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.matvec(inp, mat, vec, +1, dtype, out)
     return _matvec(torch.as_tensor(inp), mat, vec, +1, dtype, out)
 
 
 def sym_addmatvec_(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None) -> Tensor:
     """In-place ``inp += mat @ vec``; returns ``inp``  (sym.py:31)."""
+    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
+            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.matvec(inp, mat, vec, +1, inp.dtype if dtype is None else dtype, None, inplace=True)
     return _matvec(inp, mat, vec, +1, inp.dtype if dtype is None else dtype, inp)
 
 
 def sym_submatvec(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None,
                   out: Optional[Tensor] = None) -> Tensor:
     """``inp - mat @ vec``  (sym.py:32)."""
+    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
+            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.matvec(inp, mat, vec, -1, dtype, out)
     return _matvec(torch.as_tensor(inp), mat, vec, -1, dtype, out)
 
 
 def sym_submatvec_(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None) -> Tensor:
     """In-place ``inp -= mat @ vec``; returns ``inp``  (sym.py:32)."""
+    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
+            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.matvec(inp, mat, vec, -1, inp.dtype if dtype is None else dtype, None, inplace=True)
     return _matvec(inp, mat, vec, -1, inp.dtype if dtype is None else dtype, inp)
 
 
@@ -268,6 +288,14 @@ def sym_solve(mat: Tensor, vec: Tensor,
     -------
     result : `(..., M) tensor` with ``vec``'s dtype (as the reference).
     """
+    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
+            or getattr(diag, "requires_grad", False) or getattr(eps, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.solve(mat, vec, diag, dtype, out, eps, method)
+    return _solve(mat, vec, diag, dtype, out, eps=eps, method=method)
+
+
+def _solve(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = None, out: Optional[Tensor] = None, *,
+           eps=None, method: Optional[str] = None) -> Tensor:
     if eps is not None:
         if diag is not None:
             raise TypeError("give the regulariser as `diag` or as `eps`, not both")
@@ -324,7 +352,7 @@ def sym_solve(mat: Tensor, vec: Tensor,
                     res.data_ptr(), ws, wsb, chunk, nbuf, streams))
             return res
         (dm, dv), cuda_dev = _to_device_inputs(mat, vec)
-        r = sym_solve(dm, dv, None if reg is None else reg.to(cuda_dev), dtype=dtype, method=method)
+        r = _solve(dm, dv, None if reg is None else reg.to(cuda_dev), dtype=dtype, method=method)
         if out is not None:
             out.copy_(r)
             return out
@@ -337,8 +365,8 @@ def sym_solve(mat: Tensor, vec: Tensor,
         full = out if (out is not None and out.dtype == cdt and tuple(out.shape) == (*batch, n)) else \
             torch.empty((*batch, n), dtype=cdt, device=dev)
         for idx in itertools.product(*[range(k) for k in batch[:split]]):
-            sym_solve(D.outer_views(mat, batch, 1, idx), D.outer_views(vec, batch, 1, idx),
-                      D.outer_views(reg, batch, 1, idx), dtype=cdt, out=full[idx], method=method)
+            _solve(D.outer_views(mat, batch, 1, idx), D.outer_views(vec, batch, 1, idx),
+                   D.outer_views(reg, batch, 1, idx), dtype=cdt, out=full[idx], method=method)
         if out is not None and full is not out:
             out.copy_(full)
             return out
@@ -367,7 +395,10 @@ def sym_solve(mat: Tensor, vec: Tensor,
 def sym_solve_(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = None, *,
                eps=None, method: Optional[str] = None) -> Tensor:
     r"""In-place ``vec <- mat \ vec``; returns ``vec``  (reference name sym.py:33)."""
-    return sym_solve(mat, vec, diag, dtype=dtype, out=vec, eps=eps, method=method)
+    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
+            or getattr(diag, "requires_grad", False) or getattr(eps, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.solve(mat, vec, diag, dtype, None, eps, method, inplace=True)
+    return _solve(mat, vec, diag, dtype=dtype, out=vec, eps=eps, method=method)
 
 
 # ---------------------------------------------------------------------------
@@ -489,6 +520,13 @@ def sym_invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = N
     -------
     imat : `(..., M or M*(M+1)//2) tensor` (compact storage, same ordering)
     """
+    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+        return A.invert(mat, diag, dtype, out, method)
+    return _invert(mat, diag, dtype, out, method=method)
+
+
+def _invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = None,
+            out: Optional[Tensor] = None, *, method: Optional[str] = None) -> Tensor:
     if _algo(method) == _lib.ALGO_WARP:
         raise ValueError("method='warp' is a sym_solve A/B kernel (SPD input, no pivoting); sym_invert has no such variant")
     if dtype is None and torch.is_tensor(mat) and D.plain_cuda(mat) and (
@@ -530,7 +568,7 @@ def sym_invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = N
                     code, n, algo, int(bool(diag)), nb, mat.data_ptr(), res.data_ptr(), ws, wsb, chunk, nbuf, streams))
             return res
         (dm,), _ = _to_device_inputs(mat)
-        r = sym_invert(dm, diag, dtype=dtype, method=method)
+        r = _invert(dm, diag, dtype=dtype, method=method)
         if out is not None:
             out.copy_(r)
             return out
@@ -552,7 +590,9 @@ def sym_invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = N
 
 def sym_invert_(mat: Tensor, dtype: Optional[torch.dtype] = None, *, method: Optional[str] = None) -> Tensor:
     """In-place inversion; returns ``mat``  (reference name sym.py:34)."""
-    return sym_invert(mat, False, dtype=dtype, out=mat, method=method)
+    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+        return A.invert(mat, False, dtype, None, method, inplace=True)
+    return _invert(mat, False, dtype=dtype, out=mat, method=method)
 
 
 # ---------------------------------------------------------------------------
@@ -603,6 +643,12 @@ def sym_outer(x: Tensor) -> Tensor:
 def sym_det(mat: Tensor) -> Tensor:
     """Determinant of a compact symmetric matrix `(...)`  (reference _impl/sym.py:401-452;
     the reference's batched N >= 3 result is wrong (:434), this one is not)."""
+    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+        return A.det(mat)
+    return _det(mat)
+
+
+def _det(mat: Tensor) -> Tensor:
     mat = torch.as_tensor(mat)
     n = D.packed_order(mat.shape[-1])
     _check_n(n)

@@ -1,0 +1,195 @@
+#!/usr/bin/env python
+"""Forward / backward time of the differentiable packed-symmetric routines, and the
+bandwidth of the backward kernels (nfm_sym_outer2, nfm_sym_invert_backward,
+nfm_sym_det_backward) against the measured copy peak.
+
+CUDA events around many calls after a warm-up; every field is larger than the
+126 MB L2 of a B200 (except the tiny-batch gate-cost rows, which time host work).
+Prints a report; ``--out FILE`` also writes it there."""
+import argparse
+import os
+import subprocess
+import sys
+import time
+
+import torch
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import nitorch_fastmath_b200 as nfm  # noqa: E402
+from nitorch_fastmath_b200 import _autograd as A  # noqa: E402
+from nitorch_fastmath_b200 import _lib, sym  # noqa: E402
+from oracle import generators as G  # noqa: E402
+from oracle import ref_port as P  # noqa: E402
+
+DEV = "cuda:0"
+LINES = []
+
+
+def say(s=""):
+    print(s, flush=True)
+    LINES.append(s)
+
+
+def ev_time(fn, reps=20, warm=3):
+    """Mean milliseconds per call of fn() (CUDA events, after warm-up)."""
+    for _ in range(warm):
+        fn()
+    torch.cuda.synchronize()
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.record()
+    for _ in range(reps):
+        fn()
+    b.record()
+    b.synchronize()
+    return a.elapsed_time(b) / reps
+
+
+def copy_peak():
+    x = torch.empty(1 << 29, dtype=torch.float32, device=DEV)   # 2 GiB
+    y = torch.empty_like(x)
+    ms = ev_time(lambda: y.copy_(x), reps=20)
+    return 2 * x.numel() * 4 / ms / 1e6   # GB/s
+
+
+def field(shape, n, dtype, seed):
+    """SPD packed field built on the GPU: (G G^T + n I) from a seeded normal field."""
+    g = torch.Generator(device=DEV)
+    g.manual_seed(seed)
+    a = torch.randn(*shape, n, n, device=DEV, dtype=dtype, generator=g) * 0.3
+    full = a @ a.mT
+    full.diagonal(0, -1, -2).add_(n)
+    iu = torch.triu_indices(n, n, 1, device=DEV)
+    m = torch.cat([full.diagonal(0, -1, -2), full[..., iu[0], iu[1]]], -1).contiguous()
+    del a, full
+    return m
+
+
+def vecs(shape, n, dtype, seed):
+    g = torch.Generator(device=DEV)
+    g.manual_seed(seed)
+    return torch.randn(*shape, n, device=DEV, dtype=dtype, generator=g)
+
+
+def fwd_bwd(name, fwd, leaves, gout):
+    """Forward with grad-requiring inputs, and the backward alone (graph rebuilt per call, untimed)."""
+    t_plain = ev_time(lambda: fwd(*[t.detach() for t in leaves]))
+    t_fwd = ev_time(lambda: fwd(*leaves))
+    out = [None]
+
+    def bwd():
+        torch.autograd.grad(out[0], leaves, gout)
+
+    for _ in range(3):
+        out[0] = fwd(*leaves)
+        bwd()
+    torch.cuda.synchronize()
+    total = 0.0
+    reps = 10
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(reps):
+        out[0] = fwd(*leaves)
+        torch.cuda.synchronize()
+        a.record()
+        bwd()
+        b.record()
+        b.synchronize()
+        total += a.elapsed_time(b)
+    say(f"{name:44s} forward no-grad {t_plain:8.3f} ms   forward with grad {t_fwd:8.3f} ms   backward {total / reps:8.3f} ms")
+
+
+def main():
+    ap = argparse.ArgumentParser(description=__doc__)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("grad_timing needs a CUDA device")
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
+                       capture_output=True, text=True).stdout.strip()
+    say(f"GPU 0: {q}   ({torch.cuda.get_device_name(0)}; torch {torch.__version__})")
+    peak = copy_peak()
+    say(f"measured copy peak (2 GiB device-to-device copy, read + write bytes): {peak:.0f} GB/s")
+    say()
+    say("== forward / backward, fp32, fields larger than L2 ==")
+    f32 = torch.float32
+    for side, n in ((256, 3), (192, 6), (160, 10)):
+        shape = (side, side, side)
+        m, v, g = field(shape, n, f32, 1), vecs(shape, n, f32, 2), vecs(shape, n, f32, 3)
+        fwd_bwd(f"sym_solve {side}^3 N={n} (d mat, d vec)", lambda m, v: nfm.sym_solve(m, v),
+                [m.requires_grad_(), v.requires_grad_()], g)
+        del m, v, g
+        torch.cuda.empty_cache()
+    shape, n = (192, 192, 192), 6
+    nn = n * (n + 1) // 2
+    m = field(shape, n, f32, 1)
+    fwd_bwd(f"sym_invert 192^3 N={n}", lambda m: nfm.sym_invert(m), [m.requires_grad_()], vecs(shape, nn, f32, 4))
+    fwd_bwd(f"sym_invert(diag=True) 192^3 N={n}", lambda m: nfm.sym_invert(m, True), [m], vecs(shape, n, f32, 4))
+    fwd_bwd(f"sym_det 192^3 N={n}", lambda m: nfm.sym_det(m), [m], vecs(shape, 1, f32, 5)[..., 0])
+    del m
+    torch.cuda.empty_cache()
+
+    say()
+    say("== N=3 reference: autograd through the oracle (eager torch) on the same GPU, 256^3 fp32 ==")
+    shape, n = (256, 256, 256), 3
+    m, v, g = field(shape, n, f32, 1), vecs(shape, n, f32, 2), vecs(shape, n, f32, 3)
+    fwd_bwd("oracle sym_solve 256^3 N=3", lambda m, v: P.sym_solve(m, v), [m.requires_grad_(), v.requires_grad_()], g)
+    fwd_bwd("nfm    sym_solve 256^3 N=3", lambda m, v: nfm.sym_solve(m, v), [m, v], g)
+    del m, v, g
+    torch.cuda.empty_cache()
+
+    say()
+    say("== backward kernels: algorithmic bytes / time, against the copy peak ==")
+    say(f"{'kernel':44s} {'dtype':8s} {'batch':>10s} {'us':>10s} {'GB/s':>8s} {'of peak':>8s} path")
+    lib = _lib.load()
+    for dtype in (torch.float32, torch.float64):
+        s = torch.tensor([], dtype=dtype).element_size()
+        for n in (3, 6, 10):
+            nn = n * (n + 1) // 2
+            batch = int(2e9 // ((2 * nn + n) * s))        # ~2 GB of traffic per call
+            u, w = vecs((batch,), n, dtype, 1), vecs((batch,), n, dtype, 2)
+            for lname, layout, ln in (("S", _lib.LAYOUT_SYM, nn), ("D", _lib.LAYOUT_DIAG, n), ("E", _lib.LAYOUT_SCALED_IDENTITY, 1)):
+                if lname != "S" and n != 6:
+                    continue
+                ms = ev_time(lambda: A.outer2(u, w, layout, -1))
+                path = lib.nfm_last_path_was_tma()
+                gbs = (2 * n + ln) * s * batch / ms / 1e6
+                say(f"{'outer2 N=%d layout %s' % (n, lname):44s} {str(dtype)[6:]:8s} {batch:10d} {ms * 1e3:10.1f} {gbs:8.0f} {gbs / peak:8.2f} {path}")
+            del u, w
+            b = field((batch // 2,), n, dtype, 3)
+            gp, gd, gs = vecs((batch // 2,), nn, dtype, 4), vecs((batch // 2,), n, dtype, 5), vecs((batch // 2,), 1, dtype, 6)[:, 0]
+            for label, fn, nbytes in (("invert backward N=%d" % n, lambda: A.invert_backward(b, gp, False), 3 * nn),
+                                      ("invert backward diag_only N=%d" % n, lambda: A.invert_backward(b, gd, True), 2 * nn + n),
+                                      ("det backward N=%d" % n, lambda: A.det_backward(b, gs), 2 * nn + 1)):
+                ms = ev_time(fn)
+                path = lib.nfm_last_path_was_tma()
+                gbs = nbytes * s * (batch // 2) / ms / 1e6
+                say(f"{label:44s} {str(dtype)[6:]:8s} {batch // 2:10d} {ms * 1e3:10.1f} {gbs:8.0f} {gbs / peak:8.2f} {path}")
+            del b, gp, gd, gs
+            torch.cuda.empty_cache()
+
+    say()
+    say("== cost of the no-grad gate: public call vs the implementation behind it (1024 x N=3 fp32, host-bound) ==")
+    m, v = field((1024,), 3, f32, 1), vecs((1024,), 3, f32, 2)
+    pairs = [("sym_solve", lambda: nfm.sym_solve(m, v), lambda: sym._solve(m, v)),
+             ("sym_matvec", lambda: nfm.sym_matvec(m, v), lambda: sym._matvec(None, m, v, 0, None, None)),
+             ("sym_invert", lambda: nfm.sym_invert(m), lambda: sym._invert(m)),
+             ("sym_det", lambda: nfm.sym_det(m), lambda: sym._det(m))]
+    for name, pub, impl in pairs:
+        res = []
+        for f in (pub, impl, pub, impl):       # alternate, keep the better of two rounds
+            for _ in range(200):
+                f()
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            for _ in range(5000):
+                f()
+            torch.cuda.synchronize()
+            res.append((time.perf_counter() - t0) / 5000 * 1e6)
+        say(f"{name:12s} public {min(res[0], res[2]):6.2f} us/call   implementation {min(res[1], res[3]):6.2f} us/call   "
+            f"gate {min(res[0], res[2]) - min(res[1], res[3]):+5.2f} us")
+    if args.out:
+        with open(args.out, "w") as fh:
+            fh.write("\n".join(LINES) + "\n")
+
+
+if __name__ == "__main__":
+    main()
