@@ -78,6 +78,18 @@ uint64_t nfm_launch_count(void);
  * dense 16-byte aligned operands),
  * 0 otherwise (strided kernel) */
 int nfm_last_path_was_tma(void);
+/* Shape of the bulk launch of the last call on this thread (host-side record, no
+ * device work), for tests and tuning:
+ *   out[0] kind: 1 tile kernel, 3 warp-pool kernel, 4 many-right-hand-sides kernel,
+ *          0 none (strided kernel, sub-warp kernel, or no launch yet)
+ *   out[1] threads per CTA      out[2] matrices per thread
+ *   out[3] stages (tile), buffers (pool), ring depth per warp (many right-hand sides)
+ *   out[4] warps per CTA (pool, many right-hand sides; 0 for the tile kernel)
+ *   out[5] segmented shared-memory layout (0/1); many right-hand sides: the
+ *          re-layout mask (1 matrices, 2 right-hand sides)
+ *   out[6] grid (CTAs)          out[7] tiles (tile kernel) or warp tiles
+ * Returns NFM_OK, or NFM_E_BADARG when out is NULL. */
+int nfm_last_launch_shape(int64_t out[8]);
 
 /* y = A v            (inp == NULL, sign ignored)
  * y = inp + A v      (sign = +1)      y = inp - A v   (sign = -1)

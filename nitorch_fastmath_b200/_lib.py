@@ -34,6 +34,7 @@ SIGNATURES = {
     "nfm_last_error_string": (ctypes.c_char_p, []),
     "nfm_launch_count": (c_uint64, []),
     "nfm_last_path_was_tma": (c_int, []),
+    "nfm_last_launch_shape": (c_int, [ctypes.POINTER(c_int64)]),
     "nfm_sym_matvec": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _I, _P, _L, _P]),
     "nfm_sym_solve": (c_int, [_I, _I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P, _L, _P]),
     "nfm_sym_invert": (c_int, [_I, _I, _I, _I, _L, _P, _L, _P, _L, _P]),
@@ -96,3 +97,13 @@ def check(rc: int, what: str) -> None:
 
 def launch_count() -> int:
     return int(load().nfm_launch_count())
+
+
+LAUNCH_FIELDS = ("kind", "threads", "mpt", "stages", "warps", "seg", "grid", "tiles")
+
+
+def last_launch_shape() -> dict:
+    """The bulk launch of the last call on this thread (``nfm_last_launch_shape``)."""
+    buf = (c_int64 * 8)()
+    check(load().nfm_last_launch_shape(buf), "nfm_last_launch_shape")
+    return dict(zip(LAUNCH_FIELDS, (int(v) for v in buf)))

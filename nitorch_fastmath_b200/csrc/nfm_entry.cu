@@ -12,6 +12,7 @@ namespace nfm {
 
 std::atomic<unsigned long long> g_launch_count{0};
 thread_local int t_last_path_tma = 0;
+thread_local long long t_last_launch[8] = {};
 static thread_local char t_error[512] = "";
 
 void set_error(const char* fmt, ...) {
@@ -137,6 +138,11 @@ int nfm_version(void) { return NFM_VERSION; }
 const char* nfm_last_error_string(void) { return nfm::t_error; }
 uint64_t nfm_launch_count(void) { return g_launch_count.load(); }
 int nfm_last_path_was_tma(void) { return t_last_path_tma; }
+int nfm_last_launch_shape(int64_t out[8]) {
+  if (out == nullptr) return fail(NFM_E_BADARG, "output is NULL");
+  for (int i = 0; i < 8; ++i) out[i] = t_last_launch[i];
+  return NFM_OK;
+}
 
 int nfm_sym_matvec_ex(int dtype, int n, int layout, int64_t batch, const nfm_operand* mat, const nfm_operand* vec,
                       const nfm_operand* inp, int sign, const nfm_operand* out, void* stream) {

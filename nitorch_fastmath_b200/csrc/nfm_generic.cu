@@ -406,6 +406,7 @@ bool many_staged_enabled() {  // NFM_DISABLE_MANY_STAGED=1: always the one-threa
 template <typename T, int N, bool CHOL>
 static int solve_many_launch(int nrhs, int right, i64 batch, const T* a, i64 as, const T* b, i64 bs, T* out, i64 os, cudaStream_t s) {
   t_last_path_tma = 0;
+  reset_launch_record();
   constexpr int es = int(sizeof(T));
   const i64 brec = i64(N) * nrhs;
   const bool dense = as == N * N && bs == brec && os == brec && aligned16(a) && aligned16(b) && aligned16(out);
@@ -466,6 +467,7 @@ static int solve_many_launch(int nrhs, int right, i64 batch, const T* a, i64 as,
       g_launch_count.fetch_add(1, std::memory_order_relaxed);
       if (e != cudaSuccess) return int(e);
       t_last_path_tma = 4;
+      record_launch(4, nwarps * 32, 1, depth, nwarps, transpose, grid, ntiles);  // slot 5: the re-layout mask
       done = ntiles * 32;
       if (done == batch) return 0;
     }

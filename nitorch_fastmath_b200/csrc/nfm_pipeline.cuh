@@ -54,6 +54,17 @@ namespace nfm {
 
 extern std::atomic<unsigned long long> g_launch_count;
 extern thread_local int t_last_path_tma;
+// Shape of the last bulk launch on this thread (nfm_last_launch_shape): kind (1 tile, 3 pool,
+// 4 many right-hand sides, 0 none), threads per CTA, matrices per thread, stages / buffers /
+// ring depth, warps, segmented layout, grid, tiles.  Host stores only.
+extern thread_local long long t_last_launch[8];
+inline void record_launch(int kind, int threads, int mpt, int stages, int warps, int seg, long long grid, long long tiles) {
+  const long long v[8] = {kind, threads, mpt, stages, warps, seg, grid, tiles};
+  for (int i = 0; i < 8; ++i) t_last_launch[i] = v[i];
+}
+inline void reset_launch_record() {
+  for (int i = 0; i < 8; ++i) t_last_launch[i] = 0;
+}
 void set_error(const char* fmt, ...);
 
 // Ops that take the two scalar parameters of KParams declare `kScalars`.
@@ -878,7 +889,7 @@ inline int balanced_tile(i64 batch, i64 grid_max, int capacity) {
   return int(t < capacity ? t : capacity);
 }
 
-bool balance_enabled();  // nfm_entry.cu: false when the environment has NFM_DISABLE_BALANCE=1
+bool balance_enabled();  // nfm_entry.cu: true only when the environment has NFM_BALANCE=1
 
 template <class Op, int THREADS, int MPT, int STAGES, bool SEG>
 int launch_tile(const KParams& p, cudaStream_t stream) {
@@ -922,6 +933,7 @@ int launch_tile(const KParams& p, cudaStream_t stream) {
     cudaError_t e = launch_pdl(kern, unsigned(grid), THREADS, size_t(smem), stream, q, ntiles, tile_m, part_m);
     g_launch_count.fetch_add(1, std::memory_order_relaxed);
     if (e != cudaSuccess) return int(e);
+    record_launch(1, THREADS, MPT, STAGES, 0, SEG, grid, ntiles_all);
   }
   if (covered < p.batch) return launch_tail<Op>(p, covered, stream);  // < kGran matrices
   return 0;
@@ -956,6 +968,7 @@ int launch_pool(const KParams& p, int nwarps, int nbuf, cudaStream_t stream) {
   if (grid > ntiles_all) grid = ntiles_all;
   cudaError_t e = launch_pdl(kern, unsigned(grid), unsigned(nwarps * 32), size_t(smem), stream, p, ntiles, nwarps, nbuf);
   g_launch_count.fetch_add(1, std::memory_order_relaxed);
+  if (e == cudaSuccess) record_launch(3, nwarps * 32, MPT, nbuf, nwarps, SEG, grid, ntiles_all);
   return int(e);
 }
 
@@ -977,6 +990,7 @@ template <class Op>
 int run_op(KParams p, cudaStream_t stream) {
   using Tn = Tune<Op>;
   t_last_path_tma = 0;
+  reset_launch_record();
   if (p.batch == 0) return NFM_OK;
   const int lens[kMaxIn] = {Op::kLen0, Op::kLen1, Op::kLen2, len3<Op>::value};
   bool fast = p.out_stride == Op::kOut && elem_stride(p.out_estride) == 1 && aligned16(p.out);
@@ -1036,8 +1050,11 @@ int run_op(KParams p, cudaStream_t stream) {
     } else if constexpr (TuneSmall<Op>::kEnabled) {
       using Ts = TuneSmall<Op>;
       const bool small = p.batch * Ts::kRec < Ts::kBelowBytes;
-      rc = small ? launch_tile<Op, Ts::kThreads, Ts::kMpt, Ts::kStages, Tn::kSeg>(p, stream)
-                 : launch_tile<Op, Tn::kThreads, Tn::kMpt, Tn::kStages, Tn::kSeg>(p, stream);
+      rc = small ? -1 : launch_tile<Op, Tn::kThreads, Tn::kMpt, Tn::kStages, Tn::kSeg>(p, stream);
+      // the large geometry's ring is sized for the mandatory operands; with the optional ones staged
+      // as well it can pass the shared-memory limit (fp32 7x7 scaled-identity addmatvec: 241,704 B):
+      // the small geometry then keeps the batch on the TMA path
+      if (rc < 0) rc = launch_tile<Op, Ts::kThreads, Ts::kMpt, Ts::kStages, Tn::kSeg>(p, stream);
     } else {
       rc = launch_tile<Op, Tn::kThreads, Tn::kMpt, Tn::kStages, Tn::kSeg>(p, stream);
     }

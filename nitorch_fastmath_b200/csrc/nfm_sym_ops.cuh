@@ -17,6 +17,11 @@ __host__ __device__ constexpr int layout_len(int layout, int n) {
 
 constexpr int kFlagSubtract = 1;  // matvec: out = inp - A v
 
+__device__ __forceinline__ float add_rn(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ double add_rn(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ float sub_rn(float a, float b) { return __fsub_rn(a, b); }
+__device__ __forceinline__ double sub_rn(double a, double b) { return __dsub_rn(a, b); }
+
 // out = [inp +/-] A v        in0 = mat, in1 = vec, in2 = inp (optional)
 template <typename T, int N, int LAYOUT>
 struct SymMatvecOp {
@@ -43,9 +48,12 @@ struct SymMatvecOp {
       dense_matvec_reg<T, N, N>(m, v, y);
     }
     if (present & 4) {
+      // the addend is added to the rounded product by an add the compiler may not fuse: left to
+      // it, `inp + m v` became an FMA in some tile geometries and not in others (diagonal layout,
+      // fp32 order 6, fp64 order 3), so one call gave other bits above the large-batch switch
       const bool sub = flags & kFlagSubtract;
 #pragma unroll
-      for (int i = 0; i < N; ++i) out[i] = sub ? inp[i] - y[i] : inp[i] + y[i];
+      for (int i = 0; i < N; ++i) out[i] = sub ? sub_rn(inp[i], y[i]) : add_rn(inp[i], y[i]);
     } else {
 #pragma unroll
       for (int i = 0; i < N; ++i) out[i] = y[i];

@@ -42,7 +42,10 @@ int sym_solve_warp(int n, const KParams& p0, cudaStream_t s) {
   }
   const int warp_flag = t_last_path_tma;
   const int rc = sym_solve_part1<T>(n, p, s);
-  if (warp_flag == 2) t_last_path_tma = 2;
+  if (warp_flag == 2) {  // the bulk went to the sub-warp kernel, not the tile launch of the remainder
+    t_last_path_tma = 2;
+    reset_launch_record();
+  }
   return rc;
 }
 

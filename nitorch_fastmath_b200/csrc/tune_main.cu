@@ -15,6 +15,7 @@
 namespace nfm {
 std::atomic<unsigned long long> g_launch_count{0};
 thread_local int t_last_path_tma = 0;
+thread_local long long t_last_launch[8] = {};
 void set_error(const char*, ...) {}
 const DeviceInfo& device_info() {
   static DeviceInfo d{};

@@ -159,7 +159,10 @@ def test_ragged_tile_boundaries(nfm, batch):
     """Batches around the tile size: full tiles go by TMA, and so does the partial
     last tile (a smaller byte count); only the batch % 4 (% 32 in the segmented layout)
     matrices that break the 16-byte granularity of bulk copies go to the strided
-    kernel -- 3x3 fp32 (tile 1024), 6x6 fp32 (tile 512), dense 4x4 fp64 (segmented)."""
+    kernel -- 3x3 fp32, 6x6 fp32, dense 4x4 fp64 (segmented).  All of these batches
+    stay below the large-batch switch, so the packed solves run in the small tile
+    geometry (3x3: 512-matrix tiles, 6x6: 128); the largest gives each CTA only a few
+    tiles.  The large geometry and ring wrap-around are covered by test_steady_state.py."""
     from nitorch_fastmath_b200 import _lib
     for n in (3, 6):
         mat = G.spd_packed(batch, n, torch.float32, seed=batch + n)
@@ -222,7 +225,9 @@ def test_pivoting_differs_between_lanes_of_a_warp(nfm, dtype, n):
 def test_pool_kernel_tile_boundaries(nfm, batch):
     """Heavy ops with large records run on the warp-pool kernel (32-matrix warp
     tiles, buffers handed from warp to warp): batches around the warp tile and
-    around one / several rounds of the pool."""
+    around one round of the grid.  The largest gives each CTA about three warp
+    tiles, fewer than its buffers, so no buffer is refilled here; recycling is
+    covered by test_steady_state.py."""
     from nitorch_fastmath_b200 import _lib
     for n, dtype in ((8, torch.float64), (9, torch.float64), (10, torch.float32), (10, torch.float64)):
         a = _row_permuted(G.dense_shifted(batch, n, dtype, seed=batch + n), seed=batch)
