@@ -118,6 +118,13 @@ def as_operand(t: torch.Tensor, batch_shape: Tuple[int, ...], rec_ndim: int, dty
     return Operand(full, stride, estride)
 
 
+def check_out_shape(out: Optional[torch.Tensor], shape: Sequence[int]) -> None:
+    """``out`` must have exactly the result's shape: the host pipelines write ``batch x record``
+    elements through its pointer, and ``copy_`` would broadcast into a larger tensor."""
+    if out is not None and tuple(out.shape) != tuple(shape):
+        raise RuntimeError(f"out has shape {tuple(out.shape)}, expected {tuple(shape)}")
+
+
 def out_operand(out: Optional[torch.Tensor], shape: Tuple[int, ...], rec_ndim: int, dtype: torch.dtype,
                 device: torch.device, allow_estride: bool = False):
     """Returns (operand to write into, tensor to return, needs_copy_back)."""
@@ -125,8 +132,7 @@ def out_operand(out: Optional[torch.Tensor], shape: Tuple[int, ...], rec_ndim: i
         res = torch.empty(shape, dtype=dtype, device=device)
         rec_len = math.prod(shape[len(shape) - rec_ndim:]) if rec_ndim else 1
         return Operand(res, rec_len), res, False
-    if tuple(out.shape) != tuple(shape):
-        raise RuntimeError(f"out has shape {tuple(out.shape)}, expected {tuple(shape)}")
+    check_out_shape(out, shape)
     if out.device != device:
         raise RuntimeError("out lives on a different device")
     nb = len(shape) - rec_ndim

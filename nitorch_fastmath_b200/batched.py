@@ -54,7 +54,8 @@ def batchdet(a: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
     if a.device.type != "cuda":
         n = _square_order(a)
         nb = a.numel() // (n * n)
-        if _plain_host(a) and nb > 0 and (out is None or (_plain_host(a, out) and out.shape == a.shape[:-2])):
+        D.check_out_shape(out, a.shape[:-2])
+        if _plain_host(a) and nb > 0 and (out is None or _plain_host(a, out)):
             code = D.dtype_code(a.dtype)
             res = out if out is not None else torch.empty(a.shape[:-2], dtype=a.dtype, pin_memory=True)
             _host.run_host("nfm_batch_det_host", code, a.dtype, n * n, 1, nb,
@@ -107,7 +108,8 @@ def batchinv(a: Tensor, *, method: str = 'auto', regularise: bool = True, out: O
     if a.device.type != "cuda":
         n = _square_order(a)
         nb = a.numel() // (n * n)
-        if _plain_host(a) and nb > 0 and (out is None or (_plain_host(a, out) and out.shape == a.shape)):
+        D.check_out_shape(out, a.shape)
+        if _plain_host(a) and nb > 0 and (out is None or _plain_host(a, out)):
             code = D.dtype_code(a.dtype)
             res = out if out is not None else torch.empty(a.shape, dtype=a.dtype, pin_memory=True)
             _host.run_host("nfm_batch_inv_host", code, a.dtype, n * n, n * n, nb,
@@ -152,6 +154,7 @@ def batchmatvec(mat: Tensor, vec: Tensor, *, out: Optional[Tensor] = None) -> Te
     mat, vec = torch.as_tensor(mat), torch.as_tensor(vec)
     dev = D.common_device(mat, vec)
     if dev.type != "cuda":
+        D.check_out_shape(out, (*torch.broadcast_shapes(mat.shape[:-2], vec.shape[:-1]), mat.shape[-2]))
         r = batchmatvec(*_upload(mat, vec))
         if out is not None:
             out.copy_(r)

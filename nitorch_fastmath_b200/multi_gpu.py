@@ -14,6 +14,7 @@ from typing import Callable, Optional, Sequence
 import torch
 from torch import Tensor
 
+from . import _dispatch as D
 from . import sym
 from .shard import shard_bounds
 
@@ -60,6 +61,7 @@ def sym_solve_multi(mat: Tensor, vec: Tensor, diag: Optional[Tensor] = None, *, 
     r"""``mat \ vec`` for CPU tensors ``mat (B, N(N+1)/2)``, ``vec (B, N)`` (and an optional
     per-matrix regulariser ``diag (B, N)``), sharded over ``devices``."""
     _check_host(mat, vec, diag, out)
+    D.check_out_shape(out, vec.shape)
     devices = _devices(devices)
     flat_m, flat_v = mat.reshape(-1, mat.shape[-1]), vec.reshape(-1, vec.shape[-1])
     flat_d = diag.reshape(-1, diag.shape[-1]) if diag is not None else None
@@ -78,10 +80,11 @@ def sym_invert_multi(mat: Tensor, diag: bool = False, *, devices: Optional[Seque
                      out: Optional[Tensor] = None, method: Optional[str] = None) -> Tensor:
     """Packed inverse (or its diagonal) of CPU ``mat (B, N(N+1)/2)``, sharded over ``devices``."""
     _check_host(mat, out)
+    width = D.packed_order(mat.shape[-1]) if diag else mat.shape[-1]
+    D.check_out_shape(out, (*mat.shape[:-1], width))
     devices = _devices(devices)
     flat_m = mat.reshape(-1, mat.shape[-1])
     if out is None:
-        width = sym.D.packed_order(mat.shape[-1]) if diag else mat.shape[-1]
         out = torch.empty((*mat.shape[:-1], width), dtype=mat.dtype, pin_memory=True)
     flat_o = out.reshape(-1, out.shape[-1])
 
@@ -96,6 +99,7 @@ def sym_matvec_multi(mat: Tensor, vec: Tensor, *, devices: Optional[Sequence[int
                      out: Optional[Tensor] = None) -> Tensor:
     """``mat @ vec`` for CPU tensors, sharded over ``devices``."""
     _check_host(mat, vec, out)
+    D.check_out_shape(out, vec.shape)
     devices = _devices(devices)
     flat_m, flat_v = mat.reshape(-1, mat.shape[-1]), vec.reshape(-1, vec.shape[-1])
     if out is None:

@@ -43,10 +43,11 @@ def lmdiv(a: Tensor, b: Tensor, method: str = 'lu', rcond: float = 1e-15, out: O
     if dev.type != "cuda":
         cuda = _host.offload_device()
         n, k = a.shape[-1], b.shape[-1]
+        if b.dim() >= 2 and b.shape[-2] == n:     # anything else is rejected by the device call
+            D.check_out_shape(out, (*torch.broadcast_shapes(a.shape[:-2], b.shape[:-2]), n, k))
         plain = (a.dtype == b.dtype and a.dtype in D._DTYPE_CODE and a.is_contiguous() and b.is_contiguous()
                  and 1 <= n <= _lib.MAX_N and b.shape[-2] == n and a.shape[:-2] == b.shape[:-2] and k > 0 and a.numel() > 0
-                 and (out is None or (out.device.type == "cpu" and out.is_contiguous() and out.dtype == a.dtype
-                                      and out.shape == b.shape)))
+                 and (out is None or (out.device.type == "cpu" and out.is_contiguous() and out.dtype == a.dtype)))
         if plain:
             # dense host batches are streamed through the GPU in chunks (nfm_batch_solve_host)
             code = D.dtype_code(a.dtype)
@@ -97,6 +98,8 @@ def rmdiv(a: Tensor, b: Tensor, method: str = 'lu', rcond: float = 1e-15, out: O
     dev = D.common_device(a, b)
     if dev.type != "cuda":
         cuda = _host.offload_device()
+        if a.dim() >= 2 and a.shape[-1] == b.shape[-1]:     # anything else is rejected by the device call
+            D.check_out_shape(out, (*torch.broadcast_shapes(a.shape[:-2], b.shape[:-2]), a.shape[-2], b.shape[-1]))
         r = rmdiv(a.to(cuda), b.to(cuda), method=method).cpu()
         if out is not None:
             out.copy_(r)

@@ -115,6 +115,7 @@ def _matvec(inp: Optional[Tensor], mat: Tensor, vec: Tensor, sign: int,
 
     if dev.type != "cuda":
         _host.offload_device()   # raises when there is no CUDA device: no CPU path
+        D.check_out_shape(out, (*batch, n))
         plain = (layout == _lib.LAYOUT_SYM and all(_host.is_plain(t) and tuple(t.shape[:-1]) == batch and t.dtype == cdt
                                                    for t in tensors)
                  and (out is None or (_host.is_plain(out) and out.dtype == cdt)))
@@ -336,6 +337,7 @@ def _solve(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = N
 
     if dev.type != "cuda":
         _host.offload_device()   # raises when there is no CUDA device: no CPU path
+        D.check_out_shape(out, (*batch, n))
         per_voxel_reg = reg is not None and reg.dim() > 1
         plain = (layout == _lib.LAYOUT_SYM and _host.is_plain(mat) and _host.is_plain(vec)
                  and tuple(mat.shape[:-1]) == batch and tuple(vec.shape[:-1]) == batch
@@ -558,6 +560,7 @@ def _invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = None
 
     if dev.type != "cuda":
         _host.offload_device()   # raises when there is no CUDA device: no CPU path
+        D.check_out_shape(out, (*batch, no))
         plain = (_host.is_plain(mat) and mat.dtype == cdt
                  and (out is None or (_host.is_plain(out) and out.dtype == cdt)))
         if plain and nb > 0:
