@@ -296,6 +296,54 @@ int nfm_sym_det_backward(int dtype, int n, int64_t batch,
                          const void *grad, int64_t grad_stride,
                          void *out, int64_t out_stride, void *stream);
 
+/* ---- gradients of the dense routines (batchdet, batchinv, batchmatvec, lmdiv, rmdiv) ----
+ * Records are dense row-major.  G is the incoming gradient.  For the LDL^T path
+ * (method 'chol') the gradient is the symmetric part of the general formula. */
+
+/* Gradient of t = det A:  out = g * adj(A)^T (the cofactor matrix).  n <= 3:
+ * closed-form cofactors (finite for singular A); n >= 4: one pivoted Gauss-Jordan
+ * elimination, out = g t A^-T (non-finite for a singular A).
+ * mat, out: records of n*n; grad: one value per matrix. */
+int nfm_batch_det_backward(int dtype, int n, int64_t batch,
+                           const void *mat, int64_t mat_stride,
+                           const void *grad, int64_t grad_stride,
+                           void *out, int64_t out_stride, void *stream);
+
+/* Gradient of Y = A^-1 from Y:  out = -Y^T G Y^T  (sym == 0: lu / auto), or
+ * out = -Y (G + G^T) Y / 2  (sym == 1: 'chol', Y symmetric).  Records of n*n. */
+int nfm_batch_inv_backward(int dtype, int n, int sym, int64_t batch,
+                           const void *inv, int64_t inv_stride,
+                           const void *grad, int64_t grad_stride,
+                           void *out, int64_t out_stride, void *stream);
+
+/* order 0: out = sign * U W^T   (U: m x k, W: n x k)
+ * order 1: out = sign * U^T W   (U: k x m, W: k x n)
+ * out: m x n; sym == 1 (m == n only): sign * (M + M^T) / 2; sign = +1 or -1.
+ *   X = A^-1 B  (lmdiv):       dA = -U X^T with U = A^-T G      (order 0, sign -1)
+ *   Y = B A^-1  (rmdiv):       dA = -Y^T U with U = G A^-T      (order 1, sign -1)
+ *   y = A v     (batchmatvec): dA = g v^T                        (order 0, k = 1)
+ * m == n <= 10 with k <= 4 run on the TMA-staged register kernels, other shapes on
+ * a run-time-sized kernel. */
+int nfm_batch_outer(int dtype, int m, int n, int k, int order, int sym, int sign,
+                    int64_t batch, const void *u, int64_t u_stride,
+                    const void *w, int64_t w_stride,
+                    void *out, int64_t out_stride, void *stream);
+
+/* right == 0: X = A^-T B  (B, X: n x k row-major)
+ * right == 1: X = B A^-T  (B, X: k x n row-major)
+ * algo: NFM_ALGO_LU (AUTO is LU) or NFM_ALGO_LDL (A symmetric: the same as
+ * nfm_batch_solve / nfm_batch_rsolve). */
+int nfm_batch_tsolve(int dtype, int n, int k, int right, int algo, int64_t batch,
+                     const void *mat, int64_t a_stride,
+                     const void *b, int64_t b_stride,
+                     void *out, int64_t out_stride, void *stream);
+
+/* y = A^T v ; A: m x n row-major, v: m, y: n. */
+int nfm_batch_tmatvec(int dtype, int m, int n, int64_t batch,
+                      const void *mat, int64_t mat_stride,
+                      const void *vec, int64_t vec_stride,
+                      void *out, int64_t out_stride, void *stream);
+
 /* ---- host-buffer pipelines (end-to-end path) --------------------------- */
 
 /* Bytes of device workspace the host pipelines want for `chunk` matrices per

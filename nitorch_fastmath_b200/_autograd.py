@@ -1,8 +1,10 @@
 """Gradients of the packed-symmetric routines (sym_matvec family, sym_solve,
-sym_invert, sym_det).
+sym_invert, sym_det) and of the dense ones (batchdet, batchinv, batchmatvec,
+lmdiv, rmdiv; through them inv, solvevec and matvec).
 
-The public functions in ``sym.py`` route here only when grad mode is on and a
-tensor operand requires grad; otherwise they run their plain path untouched.
+The public functions in ``sym.py``, ``batched.py`` and ``sugar.py`` route here
+only when grad mode is on and a tensor operand requires grad; otherwise they run
+their plain path untouched.
 Each ``torch.autograd.Function`` runs the plain implementation in ``forward``
 and the library's backward kernels (``nfm_sym_outer2``,
 ``nfm_sym_invert_backward``, ``nfm_sym_det_backward``, plus the forward
@@ -19,10 +21,20 @@ incoming gradient, S(u, w) = the gradient of u^T A w with respect to p.
   B = A^-1               d_p from M = B G B (nfm_sym_invert_backward)
   t = det A              d_p = g * adjugate, off-diagonal doubled (nfm_sym_det_backward)
 
+Dense (G = the incoming gradient; for method 'chol' the symmetric part of each matrix
+gradient, torch's convention for cholesky + cholesky_solve / cholesky_inverse):
+
+  t = det A              dA = g adj(A)^T                       (nfm_batch_det_backward)
+  Y = A^-1               dA = -Y^T G Y^T                       (nfm_batch_inv_backward)
+  X = A^-1 B             U = A^-T G: dB = U, dA = -U X^T       (nfm_batch_tsolve, nfm_batch_outer)
+  Y = B A^-1             U = G A^-T: dB = U, dA = -Y^T U
+  y = A v                dA = g v^T, dv = A^T g                (nfm_batch_outer, nfm_batch_tmatvec)
+
 Backward passes are once-differentiable: a second-order gradient raises.
 """
 from __future__ import annotations
 
+from types import SimpleNamespace
 from typing import Optional
 
 import torch
@@ -31,6 +43,7 @@ from torch.autograd.function import once_differentiable
 
 from . import _dispatch as D
 from . import _host, _lib
+from . import batched as B
 from . import sym as S
 
 
@@ -51,7 +64,7 @@ def _launch(name: str, n: int, out_len: int, batch, operands, *args, before=(), 
     the scalar arguments ahead of / between the operands and the output."""
     out = torch.empty((*batch, out_len), dtype=dtype, device=device)
     nb = D.batch_count(batch)
-    if nb > 0:
+    if nb > 0 and out_len > 0:
         ops = [D.as_operand(t, batch, 1, dtype) for t in operands]
         ptrs = [x for o in ops for x in (o.ptr, o.stride)]
         with D.device_of(device):
@@ -283,3 +296,172 @@ class _Det(torch.autograd.Function):
 
 def det(mat) -> Tensor:
     return _Det.apply(torch.as_tensor(mat))
+
+
+# ---------------------------------------------------------------------------
+# dense routines: records (..., n, n), (..., n, k), (..., k, n), (..., n)
+# ---------------------------------------------------------------------------
+
+def _meta(t: Tensor) -> SimpleNamespace:
+    """What ``_grad_for`` needs of an operand, without keeping it alive."""
+    return SimpleNamespace(shape=t.shape, dtype=t.dtype, device=t.device)
+
+
+def _batch(*records) -> tuple:
+    return tuple(torch.broadcast_shapes(*[t.shape[:t.dim() - nd] for t, nd in records]))
+
+
+def dense_det_backward(a: Tensor, g: Tensor) -> Tensor:
+    """g * adj(A)^T for (..., n, n) matrices and (...) incoming gradients."""
+    n = a.shape[-1]
+    batch = _batch((a, 2), (g, 0))
+    return _launch("nfm_batch_det_backward", n, n * n, batch, [a.flatten(-2), g.unsqueeze(-1)],
+                   dtype=a.dtype, device=a.device).view(*batch, n, n)
+
+
+def dense_inv_backward(y: Tensor, g: Tensor, sym: bool) -> Tensor:
+    """-Y^T G Y^T, or -Y (G + G^T) Y / 2 when ``sym``, from the inverse Y."""
+    n = y.shape[-1]
+    batch = _batch((y, 2), (g, 2))
+    return _launch("nfm_batch_inv_backward", n, n * n, batch, [y.flatten(-2), g.flatten(-2)], before=(int(sym),),
+                   dtype=y.dtype, device=y.device).view(*batch, n, n)
+
+
+def dense_outer(u: Tensor, w: Tensor, rows: bool, sym: bool, sign: int) -> Tensor:
+    """``sign * U W^T`` (U: (..., m, k), W: (..., n, k)) or, with ``rows``, ``sign * U^T W``
+    (U: (..., k, m), W: (..., k, n)); the symmetric part when ``sym``."""
+    k, m = (u.shape[-2], u.shape[-1]) if rows else (u.shape[-1], u.shape[-2])
+    n = w.shape[-1] if rows else w.shape[-2]
+    batch = _batch((u, 2), (w, 2))
+    if k == 0:
+        return torch.zeros((*batch, m, n), dtype=u.dtype, device=u.device)
+    return _launch("nfm_batch_outer", m, m * n, batch, [u.flatten(-2), w.flatten(-2)],
+                   before=(n, k, int(rows), int(sym), sign), dtype=u.dtype, device=u.device).view(*batch, m, n)
+
+
+def dense_tsolve(a: Tensor, b: Tensor, right: bool, algo: int) -> Tensor:
+    """``A^-T B`` (B: (..., n, k)) or, with ``right``, ``B A^-T`` (B: (..., k, n))."""
+    n = a.shape[-1]
+    k = b.shape[-2] if right else b.shape[-1]
+    batch = _batch((a, 2), (b, 2))
+    return _launch("nfm_batch_tsolve", n, n * k, batch, [a.flatten(-2), b.flatten(-2)], before=(k, int(right), algo),
+                   dtype=a.dtype, device=a.device).view(*batch, *b.shape[-2:])
+
+
+def dense_tmatvec(a: Tensor, v: Tensor) -> Tensor:
+    """``A^T v`` for A: (..., m, n), v: (..., m)."""
+    m, n = a.shape[-2:]
+    batch = _batch((a, 2), (v, 1))
+    return _launch("nfm_batch_tmatvec", m, n, batch, [a.flatten(-2), v], before=(n,), dtype=a.dtype, device=a.device)
+
+
+class _BatchDet(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, a):
+        ctx.save_for_backward(a)
+        return B._batchdet(a)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        a, = ctx.saved_tensors
+        dev, cdt = _work_device(a.device), D.compute_dtype(a)
+        return _grad_for(dense_det_backward(a.to(device=dev, dtype=cdt), g.to(device=dev, dtype=cdt)), a)
+
+
+def batchdet(a, out) -> Tensor:
+    _check_out(out, "batchdet")
+    return _BatchDet.apply(torch.as_tensor(a))
+
+
+class _BatchInv(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, a, method, regularise):
+        res = B._batchinv(a, method=method, regularise=regularise)
+        # n = 2, 3 with `regularise`: the determinant shift is a constant, the gradient is that of the returned Y
+        ctx.save_for_backward(res)
+        ctx.sym = method.lower() in ("chol", "ldl")
+        ctx.a = _meta(a)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        y, = ctx.saved_tensors
+        dev = _work_device(y.device)
+        d = dense_inv_backward(y.to(device=dev), g.to(device=dev, dtype=y.dtype), ctx.sym)
+        return _grad_for(d, ctx.a), None, None
+
+
+def batchinv(a, method, regularise, out) -> Tensor:
+    _check_out(out, "batchinv")
+    return _BatchInv.apply(torch.as_tensor(a), method, regularise)
+
+
+class _BatchMatvec(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, mat, vec):
+        ctx.save_for_backward(mat, vec)
+        return B._batchmatvec(mat, vec)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        mat, vec = ctx.saved_tensors
+        need_mat, need_vec = ctx.needs_input_grad[:2]
+        dev, cdt = _work_device(mat.device), D.compute_dtype(mat, vec)
+        g = g.to(device=dev, dtype=cdt)
+        d_mat = d_vec = None
+        if need_mat:
+            d_mat = _grad_for(dense_outer(g.unsqueeze(-1), vec.to(device=dev, dtype=cdt).unsqueeze(-1), False, False, 1), mat)
+        if need_vec:
+            d_vec = _grad_for(dense_tmatvec(mat.to(device=dev, dtype=cdt), g), vec)
+        return d_mat, d_vec
+
+
+def batchmatvec(mat, vec, out) -> Tensor:
+    _check_out(out, "batchmatvec")
+    return _BatchMatvec.apply(torch.as_tensor(mat), torch.as_tensor(vec))
+
+
+class _Division(torch.autograd.Function):
+    """X = A^-1 B (lmdiv, ``right`` False) or Y = B A^-1 (rmdiv: sugar.rmdiv(b, a) in its own names)."""
+
+    @staticmethod
+    def forward(ctx, a, b, method, right):
+        from . import sugar
+        res = sugar._rmdiv(b, a, method) if right else sugar._lmdiv(a, b, method)
+        ctx.save_for_backward(a, res)
+        ctx.right = right
+        ctx.algo = sugar._algo(method)
+        ctx.b = _meta(b)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        a, x = ctx.saved_tensors
+        need_a, need_b = ctx.needs_input_grad[:2]
+        dev, cdt = _work_device(a.device), x.dtype
+        ac = a.to(device=dev, dtype=cdt)
+        u = dense_tsolve(ac, g.to(device=dev, dtype=cdt), ctx.right, ctx.algo)
+        d_a = d_b = None
+        if need_b:
+            d_b = _grad_for(u, ctx.b)
+        if need_a:
+            xc = x.to(device=dev)
+            sym = ctx.algo == _lib.ALGO_LDL
+            d = dense_outer(xc, u, True, sym, -1) if ctx.right else dense_outer(u, xc, False, sym, -1)
+            d_a = _grad_for(d, a)
+        return d_a, d_b, None, None
+
+
+def lmdiv(a, b, method, out) -> Tensor:
+    _check_out(out, "lmdiv")
+    return _Division.apply(torch.as_tensor(a), torch.as_tensor(b), method, False)
+
+
+def rmdiv(a, b, method, out) -> Tensor:
+    """``a b^-1``: the Function's matrix is ``b``."""
+    _check_out(out, "rmdiv")
+    return _Division.apply(torch.as_tensor(b), torch.as_tensor(a), method, True)

@@ -56,6 +56,11 @@ SIGNATURES = {
     "nfm_sym_outer2": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _I, _P, _L, _P]),
     "nfm_sym_invert_backward": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
     "nfm_sym_det_backward": (c_int, [_I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_batch_det_backward": (c_int, [_I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_batch_inv_backward": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_batch_outer": (c_int, [_I, _I, _I, _I, _I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_batch_tsolve": (c_int, [_I, _I, _I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_batch_tmatvec": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
     "nfm_host_workspace_bytes": (c_size_t, [_I, _L, _I, _I, _I]),
     "nfm_sym_solve_host": (c_int, [_I, _I, _I, _L, _P, _P, _P, _P, _P, c_size_t, _L, _I, ctypes.POINTER(c_void_p)]),
     "nfm_sym_invert_host": (c_int, [_I, _I, _I, _I, _L, _P, _P, _P, c_size_t, _L, _I, ctypes.POINTER(c_void_p)]),

@@ -10,6 +10,7 @@ from typing import Optional
 import torch
 from torch import Tensor
 
+from . import _autograd as A
 from . import _dispatch as D
 from . import _host, _lib
 
@@ -41,6 +42,8 @@ def batchdet(a: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
     """Batched determinant of small matrices.
 
     Reference: _impl/batched.py:35-63 (closed forms det2/det3 :22-32; LU above).
+    Differentiable (``nfm_batch_det_backward``): exact cofactors for n <= 3, also for
+    singular matrices; above, g det(A) A^-T, which is not finite for a singular matrix.
 
     Parameters
     ----------
@@ -50,6 +53,12 @@ def batchdet(a: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
     -------
     d : (...) tensor
     """
+    if getattr(a, "requires_grad", False) and torch.is_grad_enabled():
+        return A.batchdet(a, out)
+    return _batchdet(a, out=out)
+
+
+def _batchdet(a: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
     a = torch.as_tensor(a)
     if a.device.type != "cuda":
         n = _square_order(a)
@@ -99,7 +108,16 @@ def batchinv(a: Tensor, *, method: str = 'auto', regularise: bool = True, out: O
     Returns
     -------
     a : (..., n, n) tensor
+
+    Differentiable (``nfm_batch_inv_backward``); for orders 2 and 3 the determinant shift of
+    ``regularise`` is treated as a constant.
     """
+    if getattr(a, "requires_grad", False) and torch.is_grad_enabled():
+        return A.batchinv(a, method, regularise, out)
+    return _batchinv(a, method=method, regularise=regularise, out=out)
+
+
+def _batchinv(a: Tensor, *, method: str = 'auto', regularise: bool = True, out: Optional[Tensor] = None) -> Tensor:
     a = torch.as_tensor(a)
     kind = method.lower()
     algo = {'auto': _lib.ALGO_AUTO, 'lu': _lib.ALGO_LU, 'chol': _lib.ALGO_LDL, 'ldl': _lib.ALGO_LDL}.get(kind)
@@ -151,6 +169,12 @@ def batchmatvec(mat: Tensor, vec: Tensor, *, out: Optional[Tensor] = None) -> Te
     -------
     matvec : (..., m) tensor
     """
+    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.batchmatvec(mat, vec, out)
+    return _batchmatvec(mat, vec, out=out)
+
+
+def _batchmatvec(mat: Tensor, vec: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
     mat, vec = torch.as_tensor(mat), torch.as_tensor(vec)
     dev = D.common_device(mat, vec)
     if dev.type != "cuda":

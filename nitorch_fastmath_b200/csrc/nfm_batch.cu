@@ -10,7 +10,7 @@ namespace nfm {
 
 template <typename T, int ALGO> struct InvBind { template <int N> using Op = BatchInvOp<T, N, ALGO>; };
 template <typename T> struct DetBind { template <int N> using Op = BatchDetOp<T, N>; };
-template <typename T> struct MvBind { template <int N> using Op = BatchMatvecOp<T, N>; };
+template <typename T, bool TRANSPOSE> struct MvBind { template <int N> using Op = BatchMatvecOp<T, N, TRANSPOSE>; };
 template <typename T, int ALGO> struct SolBind { template <int N> using Op = BatchSolveOp<T, N, ALGO>; };
 template <typename T, int K, int ALGO> struct SolKBind { template <int N> using Op = BatchSolveKOp<T, N, K, ALGO>; };
 
@@ -48,8 +48,13 @@ int batch_det_impl(int n, const KParams& p, cudaStream_t s) {
 }
 template <typename T>
 int batch_matvec_impl(int n, const KParams& p, cudaStream_t s) {
-  return DispatchN<MvBind<T>::template Op, 1, NFM_MAX_N>::run(n, p, s);
+  return DispatchN<MvBind<T, false>::template Op, 1, NFM_MAX_N>::run(n, p, s);
 }
+template <typename T>
+int batch_tmatvec_impl(int n, const KParams& p, cudaStream_t s) {
+  return DispatchN<MvBind<T, true>::template Op, 1, NFM_MAX_N>::run(n, p, s);
+}
+template int batch_tmatvec_impl<NFM_SCALAR>(int, const KParams&, cudaStream_t);
 template int batch_inv_ldl_impl<NFM_SCALAR>(int, const KParams&, cudaStream_t);
 template int batch_det_impl<NFM_SCALAR>(int, const KParams&, cudaStream_t);
 template int batch_matvec_impl<NFM_SCALAR>(int, const KParams&, cudaStream_t);

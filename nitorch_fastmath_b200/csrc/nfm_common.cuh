@@ -42,6 +42,9 @@ struct KParams {
 
 // KParams::flags of BatchSolveKOp: X = B A^-1 with B, X  K x N row-major (one system A^T x = b per row)
 constexpr int kFlagRightDivision = 2;
+// ... and, independent of the record order, solve with A^T: X = A^-T B (left) or B A^-T (right).
+// The transposed solves are the gradients of lmdiv / rmdiv with respect to B.
+constexpr int kFlagTransposeA = 4;
 
 // ---------------------------------------------------------------------------
 // PTX wrappers

@@ -75,11 +75,15 @@ __device__ __forceinline__ void dense_inv_closed(const T (&a)[N * N], bool regul
 }
 
 // in-place Gauss-Jordan inverse with partial (row) pivoting.  N*N registers.
+// invert<true>() also returns det A (product of the pivots, sign of the row exchanges): the
+// determinant backward gets both from one elimination.  invert<false>() returns 1.
 template <typename T, int N>
 struct GaussJordan {
   T a[N][N];
 
-  __device__ __forceinline__ void invert() {
+  template <bool DET = false>
+  __device__ __forceinline__ T invert() {
+    T det = T(1);
     int piv[N];
     static_for<0, N>([&](auto K) {
       constexpr int k = K;
@@ -106,6 +110,7 @@ struct GaussJordan {
           });
         });
       }
+      if constexpr (DET) det *= (p != k) ? -a[k][k] : a[k][k];
       const T rp = T(1) / a[k][k];
       a[k][k] = T(1);
       static_for<0, N>([&](auto J) { a[k][J] *= rp; });
@@ -137,6 +142,7 @@ struct GaussJordan {
         });
       }
     });
+    return det;
   }
 };
 

@@ -134,9 +134,11 @@ struct BatchSolveOp {
 
 // X = A^-1 B with K right-hand sides; B and X are N x K row-major records.
 // With kFlagRightDivision (sugar.rmdiv, K rows): X = B A^-1, B and X are K x N row-major -- the same
-// records read with the other index order (A transposed, one right-hand side per ROW of B).  The
-// flag is uniform over the launch: one branch picks between two fully static instantiations (per-element
-// selects between the two orders cost the 4x4 fp32 left division 7 %).
+// records read with the other index order (A transposed, one right-hand side per ROW of B).
+// kFlagTransposeA solves with A^T instead, in either order: X = A^-T B or X = B A^-T (the gradients of
+// lmdiv / rmdiv; LDL^T reads a symmetric matrix, so it ignores the bit).  The flags are uniform over the
+// launch: one branch picks between fully static instantiations (per-element selects between the two
+// orders cost the 4x4 fp32 left division 7 %).
 template <typename T, int N, int K, int ALGO>
 struct BatchSolveKOp {
   using scalar = T;
@@ -149,11 +151,20 @@ struct BatchSolveKOp {
 
   __device__ static __forceinline__ void apply(const T (&a)[kLen0], const T (&b)[kLen1], const T (&z)[1], int present,
                                                int flags, T (&x)[kOut]) {
-    if (flags & kFlagRightDivision) apply_order<true>(a, b, x);
-    else apply_order<false>(a, b, x);
+    const bool right = flags & kFlagRightDivision;
+    if constexpr (ALGO != NFM_ALGO_LDL) {
+      if (flags & kFlagTransposeA) {
+        if (right) apply_order<true, false>(a, b, x);
+        else apply_order<false, true>(a, b, x);
+        return;
+      }
+    }
+    if (right) apply_order<true, true>(a, b, x);
+    else apply_order<false, false>(a, b, x);
   }
 
-  template <bool right>
+  // right: record order of B and X; ta: eliminate with A^T (right division without kFlagTransposeA)
+  template <bool right, bool ta>
   __device__ static __forceinline__ void apply_order(const T (&a)[kLen0], const T (&b)[kLen1], T (&x)[kOut]) {
     T sol[N][K];  // sol[i][c]: component i of the solution for right-hand side c
     if constexpr (ALGO == NFM_ALGO_LDL) {
@@ -174,7 +185,7 @@ struct BatchSolveKOp {
 #pragma unroll
       for (int i = 0; i < N; ++i) {
 #pragma unroll
-        for (int j = 0; j < N; ++j) g.a[i][j] = right ? a[j * N + i] : a[i * N + j];
+        for (int j = 0; j < N; ++j) g.a[i][j] = ta ? a[j * N + i] : a[i * N + j];
 #pragma unroll
         for (int c = 0; c < K; ++c) g.b[i][c] = right ? b[c * N + i] : b[i * K + c];
       }
@@ -190,7 +201,8 @@ struct BatchSolveKOp {
   }
 };
 
-template <typename T, int N>
+// y = A v, or y = A^T v when TRANSPOSE (the gradient of batchmatvec with respect to v)
+template <typename T, int N, bool TRANSPOSE = false>
 struct BatchMatvecOp {
   using scalar = T;
   static constexpr int kLen0 = N * N;
@@ -202,7 +214,17 @@ struct BatchMatvecOp {
 
   __device__ static __forceinline__ void apply(const T (&a)[kLen0], const T (&v)[N], const T (&)[1], int present,
                                                int flags, T (&y)[N]) {
-    dense_matvec_reg<T, N, N>(a, v, y);
+    if constexpr (TRANSPOSE) {
+#pragma unroll
+      for (int j = 0; j < N; ++j) {
+        T s = a[j] * v[0];
+#pragma unroll
+        for (int i = 1; i < N; ++i) s += a[i * N + j] * v[i];
+        y[j] = s;
+      }
+    } else {
+      dense_matvec_reg<T, N, N>(a, v, y);
+    }
   }
 };
 

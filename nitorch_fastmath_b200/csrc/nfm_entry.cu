@@ -391,8 +391,129 @@ int nfm_batch_matvec(int dtype, int m, int n, int64_t batch, const void* mat, in
   }
   if (mat == nullptr || vec == nullptr || out == nullptr) return fail(NFM_E_BADARG, "NULL operand");
   if (mat_stride < 0 || vec_stride < 0 || out_stride < 0) return fail(NFM_E_BADARG, "negative batch stride");
-  int rc = dtype == NFM_F32 ? batch_matvec_rt<float>(m, n, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s)
-                            : batch_matvec_rt<double>(m, n, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s);
+  int rc = dtype == NFM_F32 ? batch_matvec_rt<float>(m, n, 0, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s)
+                            : batch_matvec_rt<double>(m, n, 0, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s);
+  if (rc) set_error("matvec kernel launch failed: %s", cudaGetErrorString(cudaError_t(rc)));
+  return rc;
+}
+
+int nfm_batch_det_backward(int dtype, int n, int64_t batch, const void* mat, int64_t mat_stride, const void* grad,
+                           int64_t grad_stride, void* out, int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  Args a;
+  a.in(0, mat, mat_stride, true);
+  a.in(1, grad, grad_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  auto s = static_cast<cudaStream_t>(stream);
+  return finish(dtype == NFM_F32 ? batch_det_backward_impl<float>(n, a.p, s) : batch_det_backward_impl<double>(n, a.p, s));
+}
+
+int nfm_batch_inv_backward(int dtype, int n, int sym, int64_t batch, const void* inv, int64_t inv_stride, const void* grad,
+                           int64_t grad_stride, void* out, int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  if (sym != 0 && sym != 1) return fail(NFM_E_UNSUPPORTED, "sym must be 0 or 1");
+  Args a;
+  a.in(0, inv, inv_stride, true);
+  a.in(1, grad, grad_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  auto s = static_cast<cudaStream_t>(stream);
+  return finish(dtype == NFM_F32 ? batch_inv_backward_impl<float>(n, sym, a.p, s) : batch_inv_backward_impl<double>(n, sym, a.p, s));
+}
+
+int nfm_batch_outer(int dtype, int m, int n, int k, int order, int sym, int sign, int64_t batch, const void* u, int64_t u_stride,
+                    const void* w, int64_t w_stride, void* out, int64_t out_stride, void* stream) {
+  if (dtype != NFM_F32 && dtype != NFM_F64) return fail(NFM_E_UNSUPPORTED, "dtype must be NFM_F32 or NFM_F64");
+  if (m < 1 || n < 1 || k < 1) return fail(NFM_E_BADARG, "matrix shape must be positive");
+  if (order != 0 && order != 1) return fail(NFM_E_UNSUPPORTED, "order must be 0 (U W^T) or 1 (U^T W)");
+  if (sym != 0 && sym != 1) return fail(NFM_E_UNSUPPORTED, "sym must be 0 or 1");
+  if (sym && m != n) return fail(NFM_E_UNSUPPORTED, "sym needs a square result");
+  if (sign != 1 && sign != -1) return fail(NFM_E_BADARG, "sign must be +1 or -1");
+  if (batch < 0) return fail(NFM_E_BADARG, "negative batch");
+  auto s = static_cast<cudaStream_t>(stream);
+  if (m == n && n <= NFM_MAX_N && k <= 4) {  // register kernels through the TMA pipeline
+    Args a;
+    a.in(0, u, u_stride, true);
+    a.in(1, w, w_stride, true);
+    a.out(out, out_stride);
+    if (a.rc) return a.rc;
+    a.p.batch = batch;
+    a.p.flags = (sign < 0 ? 1 : 0) | (order ? kFlagRightDivision : 0) | (sym ? 8 : 0);  // kFlagOuterNegate, kFlagOuterSym
+    if (k <= 2)
+      return finish(dtype == NFM_F32 ? batch_outer_k12_impl<float>(n, k, a.p, s) : batch_outer_k12_impl<double>(n, k, a.p, s));
+    return finish(dtype == NFM_F32 ? batch_outer_k34_impl<float>(n, k, a.p, s) : batch_outer_k34_impl<double>(n, k, a.p, s));
+  }
+  if (u == nullptr || w == nullptr || out == nullptr) return fail(NFM_E_BADARG, "NULL operand");
+  if (u_stride < 0 || w_stride < 0 || out_stride < 0) return fail(NFM_E_BADARG, "negative batch stride");
+  t_last_path_tma = 0;
+  reset_launch_record();
+  int rc = dtype == NFM_F32 ? batch_outer_rt<float>(m, n, k, order, sym, sign, batch, u, u_stride, w, w_stride, out, out_stride, s)
+                            : batch_outer_rt<double>(m, n, k, order, sym, sign, batch, u, u_stride, w, w_stride, out, out_stride, s);
+  if (rc) set_error("outer kernel launch failed: %s", cudaGetErrorString(cudaError_t(rc)));
+  return rc;
+}
+
+int nfm_batch_tsolve(int dtype, int n, int k, int right, int algo, int64_t batch, const void* mat, int64_t a_stride, const void* b,
+                     int64_t b_stride, void* out, int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  if (k < 1) return fail(NFM_E_BADARG, "k must be >= 1");
+  if (right != 0 && right != 1) return fail(NFM_E_UNSUPPORTED, "right must be 0 (A^-T B) or 1 (B A^-T)");
+  if (algo == NFM_ALGO_AUTO) algo = NFM_ALGO_LU;
+  if (algo != NFM_ALGO_LU && algo != NFM_ALGO_LDL) return fail(NFM_E_UNSUPPORTED, "batch_tsolve: algo must be LU or LDL");
+  if (mat == nullptr || b == nullptr || out == nullptr) return fail(NFM_E_BADARG, "NULL operand");
+  if (a_stride < 0 || b_stride < 0 || out_stride < 0) return fail(NFM_E_BADARG, "negative batch stride");
+  // one right-hand side: a record of n either way, and A^-T b is the right division of one row
+  // (B A^-T = (A^-1 B^T)^T the left division of one column)
+  if (k == 1)
+    return right ? nfm_batch_solve(dtype, n, 1, algo, batch, mat, a_stride, b, b_stride, out, out_stride, stream)
+                 : nfm_batch_rsolve(dtype, n, 1, algo, batch, mat, a_stride, b, b_stride, out, out_stride, stream);
+  auto s = static_cast<cudaStream_t>(stream);
+  if (k <= 4) {  // the register kernels of nfm_batch_solve with kFlagTransposeA
+    Args a;
+    a.in(0, mat, a_stride, true);
+    a.in(1, b, b_stride, true);
+    a.out(out, out_stride);
+    if (a.rc) return a.rc;
+    a.p.batch = batch;
+    a.p.flags = kFlagTransposeA | (right ? kFlagRightDivision : 0);
+    if (algo == NFM_ALGO_LDL)
+      return finish(dtype == NFM_F32 ? batch_solvek_ldl_impl<float>(n, k, a.p, s) : batch_solvek_ldl_impl<double>(n, k, a.p, s));
+    return finish(dtype == NFM_F32 ? batch_solvek_lu_impl<float>(n, k, a.p, s) : batch_solvek_lu_impl<double>(n, k, a.p, s));
+  }
+  const int chol = algo == NFM_ALGO_LDL, mode = right | 2;  // bit 1: solve with A^T (kRightTransposeA)
+  rc = dtype == NFM_F32 ? batch_solve_many<float>(n, k, chol, mode, batch, mat, a_stride, b, b_stride, out, out_stride, s)
+                        : batch_solve_many<double>(n, k, chol, mode, batch, mat, a_stride, b, b_stride, out, out_stride, s);
+  if (rc) set_error("solve kernel launch failed: %s", cudaGetErrorString(cudaError_t(rc)));
+  return rc;
+}
+
+int nfm_batch_tmatvec(int dtype, int m, int n, int64_t batch, const void* mat, int64_t mat_stride, const void* vec,
+                      int64_t vec_stride, void* out, int64_t out_stride, void* stream) {
+  if (dtype != NFM_F32 && dtype != NFM_F64) return fail(NFM_E_UNSUPPORTED, "dtype must be NFM_F32 or NFM_F64");
+  if (m < 1 || n < 1) return fail(NFM_E_BADARG, "matrix shape must be positive");
+  if (batch < 0) return fail(NFM_E_BADARG, "negative batch");
+  auto s = static_cast<cudaStream_t>(stream);
+  if (m == n && n <= NFM_MAX_N) {
+    Args a;
+    a.in(0, mat, mat_stride, true);
+    a.in(1, vec, vec_stride, true);
+    a.out(out, out_stride);
+    if (a.rc) return a.rc;
+    a.p.batch = batch;
+    return finish(dtype == NFM_F32 ? batch_tmatvec_impl<float>(n, a.p, s) : batch_tmatvec_impl<double>(n, a.p, s));
+  }
+  if (mat == nullptr || vec == nullptr || out == nullptr) return fail(NFM_E_BADARG, "NULL operand");
+  if (mat_stride < 0 || vec_stride < 0 || out_stride < 0) return fail(NFM_E_BADARG, "negative batch stride");
+  t_last_path_tma = 0;
+  reset_launch_record();
+  int rc = dtype == NFM_F32 ? batch_matvec_rt<float>(m, n, 1, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s)
+                            : batch_matvec_rt<double>(m, n, 1, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s);
   if (rc) set_error("matvec kernel launch failed: %s", cudaGetErrorString(cudaError_t(rc)));
   return rc;
 }

@@ -11,18 +11,45 @@
 
 namespace nfm {
 
+// y = A v (A: m x n, y: m), or y = A^T v (v: m, y: n) when `trans` (the gradient of batchmatvec
+// with respect to v)
 template <typename T>
 __global__ void __launch_bounds__(128) matvec_rt_kernel(const T* __restrict__ mat, i64 ms, const T* __restrict__ vec,
-                                                        i64 vs, T* __restrict__ out, i64 os, int m, int n, i64 batch) {
-  const i64 total = batch * m;
+                                                        i64 vs, T* __restrict__ out, i64 os, int m, int n, int trans,
+                                                        i64 batch) {
+  const int rows = trans ? n : m, len = trans ? m : n, step = trans ? n : 1;
+  const i64 total = batch * rows;
   for (i64 t = i64(blockIdx.x) * blockDim.x + threadIdx.x; t < total; t += i64(gridDim.x) * blockDim.x) {
-    const i64 b = t / m;
-    const int i = int(t - b * m);
-    const T* a = mat + b * ms + i64(i) * n;
+    const i64 b = t / rows;
+    const int i = int(t - b * rows);
+    const T* a = mat + b * ms + (trans ? i64(i) : i64(i) * n);
     const T* v = vec + b * vs;
     T s = a[0] * v[0];
-    for (int j = 1; j < n; ++j) s += a[j] * v[j];
+    for (int j = 1; j < len; ++j) s += a[i64(j) * step] * v[j];
     out[b * os + i] = s;
+  }
+}
+
+// out = sign * U W^T (U: m x k, W: n x k row-major; `rows` == 0) or sign * U^T W (U: k x m, W: k x n;
+// `rows` == 1), out: m x n row-major; `sym` (m == n): sign * (M + M^T) / 2.  The run-time-sized
+// form of BatchOuterOp (nfm_dense_grad.cu) for k > 4 and rectangular shapes.  One thread per element.
+template <typename T>
+__global__ void __launch_bounds__(128) outer_rt_kernel(const T* __restrict__ u, i64 us, const T* __restrict__ w, i64 ws,
+                                                       T* __restrict__ out, i64 os, int m, int n, int k, int rows, int sym,
+                                                       T sign, i64 batch) {
+  const i64 total = batch * m * n;
+  for (i64 t = i64(blockIdx.x) * blockDim.x + threadIdx.x; t < total; t += i64(gridDim.x) * blockDim.x) {
+    const i64 b = t / (i64(m) * n);
+    const int e = int(t - b * m * n), i = e / n, j = e - (e / n) * n;
+    const T* ub = u + b * us;
+    const T* wb = w + b * ws;
+    auto dot = [&](int r, int c) {  // sum_q U(r, q) W(c, q)
+      T s = rows ? ub[r] * wb[c] : ub[i64(r) * k] * wb[i64(c) * k];
+      for (int q = 1; q < k; ++q) s += rows ? ub[i64(q) * m + r] * wb[i64(q) * n + c] : ub[i64(r) * k + q] * wb[i64(c) * k + q];
+      return s;
+    };
+    const T v = sym ? T(0.5) * (dot(i, j) + dot(j, i)) : dot(i, j);
+    out[b * os + e] = sign * v;
   }
 }
 
@@ -34,6 +61,8 @@ __global__ void __launch_bounds__(128) matvec_rt_kernel(const T* __restrict__ ma
 //   left  (right == 0): X = A^-1 B,  B and X  n x nrhs row-major  (column c: b[i*nrhs + c])
 //   right (right == 1): X = B A^-1,  B and X  nrhs x n row-major  (row c: b[c*n + i]), i.e.
 //                       A^T x_c = b_c for every row c -- no transposed copies of A or B.
+//   bit 1 of `right` (kRightTransposeA) solves with A^T in either order: X = A^-T B, X = B A^-T
+//   (the gradients of lmdiv / rmdiv).  LDL^T reads a symmetric matrix and ignores it.
 // LU with partial pivoting keeps the multipliers in the lower triangle and the pivot
 // rows in piv[]; a column replays the exchanges with predicated swaps (skipped by a
 // warp vote when no matrix of the warp pivoted in that step).
@@ -134,15 +163,18 @@ __device__ __forceinline__ void substitute_in_registers(const T (&a)[N][N], cons
   }
 }
 
-// the matrix of one system out of its row-major record (transposed for right division;
-// the lower triangle mirrored for the symmetric LDL^T path)
+constexpr int kRightTransposeA = 2;
+
+// the matrix of one system out of its row-major record (transposed for right division, and once more
+// for kRightTransposeA; the lower triangle mirrored for the symmetric LDL^T path)
 template <typename T, int N, bool CHOL, int PITCH = 1>
 __device__ __forceinline__ void load_system(const T* src, int right, T (&a)[N][N]) {
+  const bool ta = (right & 1) != ((right & kRightTransposeA) != 0);
   static_for<0, N>([&](auto I) {
     static_for<0, N>([&](auto J) {
       constexpr int i = I, j = J;
       if constexpr (CHOL) a[i][j] = src[((i > j ? i : j) * N + (i > j ? j : i)) * PITCH];  // lower triangle, symmetric
-      else a[i][j] = right ? src[(j * N + i) * PITCH] : src[(i * N + j) * PITCH];
+      else a[i][j] = ta ? src[(j * N + i) * PITCH] : src[(i * N + j) * PITCH];
     });
   });
 }
@@ -161,9 +193,9 @@ __global__ void __launch_bounds__(128) solve_many_kernel(const T* mat, i64 as, c
     T* xx = out + b * os;
     for (int c = 0; c < nrhs; ++c) {
       T x[N];
-      static_for<0, N>([&](auto I) { x[I] = right ? bb[c * N + I] : bb[I * nrhs + c]; });
+      static_for<0, N>([&](auto I) { x[I] = (right & 1) ? bb[c * N + I] : bb[I * nrhs + c]; });
       substitute_in_registers<T, N, CHOL>(a, piv, x);
-      if (valid) static_for<0, N>([&](auto I) { (right ? xx[c * N + I] : xx[I * nrhs + c]) = x[I]; });
+      if (valid) static_for<0, N>([&](auto I) { ((right & 1) ? xx[c * N + I] : xx[I * nrhs + c]) = x[I]; });
     }
   }
 }
@@ -301,9 +333,9 @@ __global__ void __launch_bounds__(many_max_warps<T, N>() * 32, 1)
       int c = (lane >> rot_shift) % nrhs;
       for (int done = 0; done < nrhs; ++done) {
         T x[N];
-        static_for<0, N>([&](auto I) { x[I] = right ? bb[c * N + I] : bb[I * nrhs + c]; });
+        static_for<0, N>([&](auto I) { x[I] = (right & 1) ? bb[c * N + I] : bb[I * nrhs + c]; });
         substitute_in_registers<T, N, CHOL>(a, piv, x);
-        static_for<0, N>([&](auto I) { (right ? bb[c * N + I] : bb[I * nrhs + c]) = x[I]; });
+        static_for<0, N>([&](auto I) { ((right & 1) ? bb[c * N + I] : bb[I * nrhs + c]) = x[I]; });
         c = c + 1 == nrhs ? 0 : c + 1;
       }
     } else {
@@ -311,9 +343,9 @@ __global__ void __launch_bounds__(many_max_warps<T, N>() * 32, 1)
       T* bb = scratch + lane;
       for (int c = 0; c < nrhs; ++c) {
         T x[N];
-        static_for<0, N>([&](auto I) { x[I] = right ? bb[(c * N + I) * kPitch] : bb[(I * nrhs + c) * kPitch]; });
+        static_for<0, N>([&](auto I) { x[I] = (right & 1) ? bb[(c * N + I) * kPitch] : bb[(I * nrhs + c) * kPitch]; });
         substitute_in_registers<T, N, CHOL>(a, piv, x);
-        static_for<0, N>([&](auto I) { (right ? bb[(c * N + I) * kPitch] : bb[(I * nrhs + c) * kPitch]) = x[I]; });
+        static_for<0, N>([&](auto I) { ((right & 1) ? bb[(c * N + I) * kPitch] : bb[(I * nrhs + c) * kPitch]) = x[I]; });
       }
       __syncwarp();
       scratch_to_tile(scratch, reinterpret_cast<T*>(buf + a_bytes), brec, lane);
@@ -386,14 +418,26 @@ static unsigned grid_for(i64 work) {
 }
 
 template <typename T>
-int batch_matvec_rt(int m, int n, i64 batch, const void* mat, i64 ms, const void* vec, i64 vs, void* out, i64 os,
+int batch_matvec_rt(int m, int n, int trans, i64 batch, const void* mat, i64 ms, const void* vec, i64 vs, void* out, i64 os,
                     cudaStream_t s) {
   if (batch == 0) return 0;
-  matvec_rt_kernel<T><<<grid_for(batch * m), 128, 0, s>>>(static_cast<const T*>(mat), ms, static_cast<const T*>(vec), vs,
-                                                          static_cast<T*>(out), os, m, n, batch);
+  matvec_rt_kernel<T><<<grid_for(batch * (trans ? n : m)), 128, 0, s>>>(static_cast<const T*>(mat), ms, static_cast<const T*>(vec),
+                                                                        vs, static_cast<T*>(out), os, m, n, trans, batch);
   g_launch_count.fetch_add(1, std::memory_order_relaxed);
   return int(cudaGetLastError());
 }
+
+template <typename T>
+int batch_outer_rt(int m, int n, int k, int rows, int sym, int sign, i64 batch, const void* u, i64 us, const void* w, i64 ws,
+                   void* out, i64 os, cudaStream_t s) {
+  if (batch == 0) return 0;
+  outer_rt_kernel<T><<<grid_for(batch * m * n), 128, 0, s>>>(static_cast<const T*>(u), us, static_cast<const T*>(w), ws,
+                                                             static_cast<T*>(out), os, m, n, k, rows, sym, T(sign), batch);
+  g_launch_count.fetch_add(1, std::memory_order_relaxed);
+  return int(cudaGetLastError());
+}
+template int batch_outer_rt<float>(int, int, int, int, int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
+template int batch_outer_rt<double>(int, int, int, int, int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
 
 bool many_staged_enabled() {  // NFM_DISABLE_MANY_STAGED=1: always the one-thread-per-system global-memory kernel
   static const bool on = [] {
@@ -500,7 +544,7 @@ int batch_solve_many(int n, int nrhs, int chol, int right, i64 batch, const void
 template int batch_solve_many<float>(int, int, int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
 template int batch_solve_many<double>(int, int, int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
 
-template int batch_matvec_rt<float>(int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
-template int batch_matvec_rt<double>(int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
+template int batch_matvec_rt<float>(int, int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
+template int batch_matvec_rt<double>(int, int, int, i64, const void*, i64, const void*, i64, void*, i64, cudaStream_t);
 
 }  // namespace nfm

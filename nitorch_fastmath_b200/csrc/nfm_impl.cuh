@@ -45,11 +45,23 @@ template <typename T> int batch_solve_ldl_impl(int n, const KParams& p, cudaStre
 // parts 4 / 5: 2..4 right-hand sides (register kernels); more go to the run-time-sized kernel
 template <typename T> int batch_solvek_lu_impl(int n, int k, const KParams& p, cudaStream_t s);
 template <typename T> int batch_solvek_ldl_impl(int n, int k, const KParams& p, cudaStream_t s);
+template <typename T> int batch_tmatvec_impl(int n, const KParams& p, cudaStream_t s);  // part 1: y = A^T v
+
+// backward kernels of the dense routines (nfm_dense_grad.cu): part 0 = inverse and determinant
+// gradients; parts 1 / 2 = sign * U W^T or U^T W (optionally symmetrised) for k = 1..2 / 3..4
+template <typename T> int batch_inv_backward_impl(int n, int sym, const KParams& p, cudaStream_t s);
+template <typename T> int batch_det_backward_impl(int n, const KParams& p, cudaStream_t s);
+template <typename T> int batch_outer_k12_impl(int n, int k, const KParams& p, cudaStream_t s);
+template <typename T> int batch_outer_k34_impl(int n, int k, const KParams& p, cudaStream_t s);
 
 // run-time-sized fallbacks (nfm_generic.cu)
+// (trans: y = A^T v; out = sign * U W^T or U^T W (rows), optionally symmetrised, for k > 4 / m != n)
 template <typename T>
-int batch_matvec_rt(int m, int n, i64 batch, const void* mat, i64 ms, const void* vec, i64 vs, void* out, i64 os,
+int batch_matvec_rt(int m, int n, int trans, i64 batch, const void* mat, i64 ms, const void* vec, i64 vs, void* out, i64 os,
                     cudaStream_t s);
+template <typename T>
+int batch_outer_rt(int m, int n, int k, int rows, int sym, int sign, i64 batch, const void* u, i64 us, const void* w, i64 ws,
+                   void* out, i64 os, cudaStream_t s);
 
 // nfm_fused.cu: register kernels for 1 <= k, d <= 6 and for tall Jacobians k <= 10, d <= 3
 constexpr int kFusedMaxOrder = 6;

@@ -12,6 +12,7 @@ from typing import Optional
 import torch
 from torch import Tensor
 
+from . import _autograd as A
 from . import _dispatch as D
 from . import _host, _lib
 from .batched import batchinv, batchmatvec
@@ -33,8 +34,14 @@ def _algo(method: str) -> int:
 def lmdiv(a: Tensor, b: Tensor, method: str = 'lu', rcond: float = 1e-15, out: Optional[Tensor] = None) -> Tensor:
     r"""Left matrix division ``inv(a) @ b``  (reference sugar.py:75-137).
 
-    a : `(..., n, n)`, b : `(..., n, k)` -> `(..., n, k)`
+    a : `(..., n, n)`, b : `(..., n, k)` -> `(..., n, k)`.  Differentiable in both operands.
     """
+    if (getattr(a, "requires_grad", False) or getattr(b, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.lmdiv(a, b, method, out)
+    return _lmdiv(a, b, method, out)
+
+
+def _lmdiv(a: Tensor, b: Tensor, method: str = 'lu', out: Optional[Tensor] = None) -> Tensor:
     a, b = torch.as_tensor(a), torch.as_tensor(b)
     if a.shape[-1] != a.shape[-2]:
         raise NotImplementedError("non-square systems (pseudo-inverse) are outside the B200 hot path")
@@ -89,8 +96,14 @@ def rmdiv(a: Tensor, b: Tensor, method: str = 'lu', rcond: float = 1e-15, out: O
     as written the reference returns ``lmdiv(b, a)^T = (inv(b) @ a)^T`` and only runs for square ``a``).
 
     a : `(..., k, n)`, b : `(..., n, n)` -> `(..., k, n)`.  Solved natively as ``b^T x_r = a_r`` for every
-    row ``r`` (``nfm_batch_rsolve``): neither operand is transposed or copied.
+    row ``r`` (``nfm_batch_rsolve``): neither operand is transposed or copied.  Differentiable in both operands.
     """
+    if (getattr(a, "requires_grad", False) or getattr(b, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.rmdiv(a, b, method, out)
+    return _rmdiv(a, b, method, out)
+
+
+def _rmdiv(a: Tensor, b: Tensor, method: str = 'lu', out: Optional[Tensor] = None) -> Tensor:
     a, b = torch.as_tensor(a), torch.as_tensor(b)
     if b.shape[-1] != b.shape[-2]:
         raise NotImplementedError("non-square systems (pseudo-inverse) are outside the B200 hot path")

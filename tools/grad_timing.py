@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """Forward / backward time of the differentiable packed-symmetric routines, and the
 bandwidth of the backward kernels (nfm_sym_outer2, nfm_sym_invert_backward,
-nfm_sym_det_backward) against the measured copy peak.
+nfm_sym_det_backward) against the measured copy peak.  ``--dense`` measures the dense
+routines instead (batchdet, batchinv, solvevec, lmdiv, rmdiv; nfm_batch_inv_backward,
+nfm_batch_det_backward, nfm_batch_outer, nfm_batch_tsolve) and autograd through torch's
+own linalg functions on the same GPU.
 
 CUDA events around many calls after a warm-up; every field is larger than the
 126 MB L2 of a B200 (except the tiny-batch gate-cost rows, which time host work).
@@ -97,9 +100,90 @@ def fwd_bwd(name, fwd, leaves, gout):
     say(f"{name:44s} forward no-grad {t_plain:8.3f} ms   forward with grad {t_fwd:8.3f} ms   backward {total / reps:8.3f} ms")
 
 
+def dense_field(batch, n, dtype, seed, spd=False):
+    """randn + n I (or G G^T + n I with ``spd``), built on the GPU."""
+    g = torch.Generator(device=DEV)
+    g.manual_seed(seed)
+    a = torch.randn(*batch, n, n, device=DEV, dtype=dtype, generator=g)
+    if spd:
+        a = a @ a.mT * 0.1
+    a.diagonal(0, -1, -2).add_(n)
+    return a
+
+
+def dense(peak):
+    lib = _lib.load()
+    f32, f64 = torch.float32, torch.float64
+    say("== dense routines: forward / backward, fields larger than L2 ==")
+    cube = (256, 256, 256)
+    a = dense_field(cube, 3, f32, 1)
+    fwd_bwd("batchdet 256^3 3x3 fp32", nfm.batchdet, [a.requires_grad_()], vecs(cube[:-1], cube[-1], f32, 2))
+    fwd_bwd("torch.linalg.det 256^3 3x3 fp32", torch.linalg.det, [a], vecs(cube[:-1], cube[-1], f32, 2))
+    gi = dense_field(cube, 3, f32, 3)
+    fwd_bwd("batchinv 256^3 3x3 fp32", nfm.batchinv, [a], gi)
+    fwd_bwd("torch.linalg.inv 256^3 3x3 fp32", torch.linalg.inv, [a], gi)
+    del a, gi
+    torch.cuda.empty_cache()
+    b16 = (16 << 20,)
+    a = dense_field(b16, 4, f64, 1).requires_grad_()
+    gi = dense_field(b16, 4, f64, 2)
+    fwd_bwd("batchinv 16M 4x4 fp64", nfm.batchinv, [a], gi)
+    fwd_bwd("torch.linalg.inv 16M 4x4 fp64", torch.linalg.inv, [a], gi)
+    del gi
+    v, g = vecs(b16, 4, f64, 3).requires_grad_(), vecs(b16, 4, f64, 4)
+    fwd_bwd("solvevec 16M 4x4 fp64 (d mat, d vec)", nfm.solvevec, [a, v], g)
+    fwd_bwd("torch.linalg.solve 16M 4x4 fp64 (d mat, d vec)", lambda a, v: torch.linalg.solve(a, v), [a, v], g)
+    del a, v, g
+    torch.cuda.empty_cache()
+    b4 = (4 << 20,)
+    a = dense_field(b4, 4, f32, 1).requires_grad_()
+    for k in (3, 8):
+        b, g = vecs(b4 + (4,), k, f32, 2).requires_grad_(), vecs(b4 + (4,), k, f32, 3)
+        fwd_bwd(f"lmdiv 4M 4x4 k={k} fp32", nfm.lmdiv, [a, b], g)
+        fwd_bwd(f"torch.linalg.solve 4M 4x4 k={k} fp32", torch.linalg.solve, [a, b], g)
+    x, g = vecs(b4 + (3,), 4, f32, 4).requires_grad_(), vecs(b4 + (3,), 4, f32, 5)
+    fwd_bwd("rmdiv 4M 3 rows x 4x4 fp32", nfm.rmdiv, [x, a], g)
+    fwd_bwd("torch.linalg.solve(left=False) 4M 3 rows fp32", lambda x, a: torch.linalg.solve(a, x, left=False), [x, a], g)
+    del a, b, g, x
+    torch.cuda.empty_cache()
+
+    say()
+    say("== dense backward kernels: algorithmic bytes / time, against the copy peak ==")
+    say("   inverse backward 3n^2 s, det backward (2n^2+1) s, outer (2nk+n^2) s, transposed solve (n^2+2nk) s")
+    say(f"{'kernel':44s} {'dtype':8s} {'batch':>10s} {'us':>10s} {'GB/s':>8s} {'of peak':>8s} path")
+    for dtype in (f32, f64):
+        s = torch.tensor([], dtype=dtype).element_size()
+        for n in (3, 4, 6, 8, 10):
+            batch = int(2e9 // (3 * n * n * s))        # ~2 GB of traffic per call
+            y, gm = dense_field((batch,), n, dtype, 1), vecs((batch, n), n, dtype, 2)
+            rows = [("inverse backward n=%d" % n, lambda: A.dense_inv_backward(y, gm, False), 3 * n * n),
+                    ("inverse backward chol n=%d" % n, lambda: A.dense_inv_backward(y, gm, True), 3 * n * n)]
+            gd = gm[:, 0, 0].contiguous()
+            rows.append(("det backward n=%d" % n, lambda: A.dense_det_backward(y, gd), 2 * n * n + 1))
+            for label, fn, nb in rows:
+                ms = ev_time(fn)
+                path = lib.nfm_last_path_was_tma()
+                gbs = nb * s * batch / ms / 1e6
+                say(f"{label:44s} {str(dtype)[6:]:8s} {batch:10d} {ms * 1e3:10.1f} {gbs:8.0f} {gbs / peak:8.2f} {path}")
+            del gm, gd
+            for k in (1, 3):
+                u, w = vecs((batch, n), k, dtype, 3), vecs((batch, n), k, dtype, 4)
+                for label, fn, nb in (("outer n=%d k=%d" % (n, k), lambda: A.dense_outer(u, w, False, False, -1), 2 * n * k + n * n),
+                                      ("transposed solve lu n=%d k=%d" % (n, k), lambda: A.dense_tsolve(y, u, False, _lib.ALGO_LU),
+                                       n * n + 2 * n * k)):
+                    ms = ev_time(fn)
+                    path = lib.nfm_last_path_was_tma()
+                    gbs = nb * s * batch / ms / 1e6
+                    say(f"{label:44s} {str(dtype)[6:]:8s} {batch:10d} {ms * 1e3:10.1f} {gbs:8.0f} {gbs / peak:8.2f} {path}")
+                del u, w
+            del y
+            torch.cuda.empty_cache()
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--dense", action="store_true", help="measure the dense routines instead of the packed ones")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("grad_timing needs a CUDA device")
@@ -109,6 +193,12 @@ def main():
     peak = copy_peak()
     say(f"measured copy peak (2 GiB device-to-device copy, read + write bytes): {peak:.0f} GB/s")
     say()
+    if args.dense:
+        dense(peak)
+        if args.out:
+            with open(args.out, "w") as fh:
+                fh.write("\n".join(LINES) + "\n")
+        return
     say("== forward / backward, fp32, fields larger than L2 ==")
     f32 = torch.float32
     for side, n in ((256, 3), (192, 6), (160, 10)):
