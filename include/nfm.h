@@ -296,6 +296,38 @@ int nfm_sym_det_backward(int dtype, int n, int64_t batch,
                          const void *grad, int64_t grad_stride,
                          void *out, int64_t out_stride, void *stream);
 
+/* ---- gradients of the Gauss-Newton builders (sym_matmul, sym_outer, sym_to_full) ----
+ * g = the incoming gradient of a packed result of order n; G^ = its full symmetric
+ * matrix with the off-diagonals halved (G^_ii = g_ii, G^_ij = g_ij / 2);
+ * pack(M) = M_ii, 2 M_ij (i < j).  The fused sym_matmul_solve / sym_solve_update
+ * differentiate through nfm_sym_matmul, nfm_sym_solve, nfm_sym_outer2 and
+ * nfm_sym_matmul_backward. */
+
+/* Gradient of nfm_sym_matmul (same k, d, mode and the same shapes):
+ *   mode 0, Y = J^T H J:  dJ = 2 H J G^,  dH = pack(J G^ J^T)
+ *   mode 1, Y = J H J^T:  dJ = 2 G^ J H,  dH = pack(J^T G^ J)      (k == d)
+ * jac: k x d row-major, hess: packed, grad: packed records of the result's order.
+ * which = 1: out = dJ (records of k*d); 2: out = dH (packed records of H);
+ * 3: out = [dJ | dH] (records of k*d + the packed length of H). */
+int nfm_sym_matmul_backward(int dtype, int k, int d, int mode, int which, int64_t batch,
+                            const void *jac, int64_t jac_stride,
+                            const void *hess, int64_t hess_stride,
+                            const void *grad, int64_t grad_stride,
+                            void *out, int64_t out_stride, void *stream);
+
+/* Gradient of y = x x^T (nfm_sym_outer):  out = 2 G^ x.
+ * vec, out: records of n; grad: records of n(n+1)/2. */
+int nfm_sym_outer_backward(int dtype, int n, int64_t batch,
+                           const void *vec, int64_t vec_stride,
+                           const void *grad, int64_t grad_stride,
+                           void *out, int64_t out_stride, void *stream);
+
+/* Gradient of F = nfm_sym_to_full(p):  out_ii = G_ii, out_ij = G_ij + G_ji.
+ * grad: n x n row-major records; out: records of n(n+1)/2. */
+int nfm_sym_to_full_backward(int dtype, int n, int64_t batch,
+                             const void *grad, int64_t grad_stride,
+                             void *out, int64_t out_stride, void *stream);
+
 /* ---- gradients of the dense routines (batchdet, batchinv, batchmatvec, lmdiv, rmdiv) ----
  * Records are dense row-major.  G is the incoming gradient.  For the LDL^T path
  * (method 'chol') the gradient is the symmetric part of the general formula. */

@@ -1,6 +1,7 @@
 """Gradients of the packed-symmetric routines (sym_matvec family, sym_solve,
-sym_invert, sym_det) and of the dense ones (batchdet, batchinv, batchmatvec,
-lmdiv, rmdiv; through them inv, solvevec and matvec).
+sym_invert, sym_det), of the Gauss-Newton builders (sym_matmul, sym_outer,
+sym_to_full, sym_matmul_solve, sym_solve_update(_)) and of the dense ones
+(batchdet, batchinv, batchmatvec, lmdiv, rmdiv; through them inv, solvevec and matvec).
 
 The public functions in ``sym.py``, ``batched.py`` and ``sugar.py`` route here
 only when grad mode is on and a tensor operand requires grad; otherwise they run
@@ -20,6 +21,16 @@ incoming gradient, S(u, w) = the gradient of u^T A w with respect to p.
   x = (A + diag d)^-1 v  u = (A + diag d)^-1 g: d_v = u, d_p = -S(u, x), d_d = -u * x
   B = A^-1               d_p from M = B G B (nfm_sym_invert_backward)
   t = det A              d_p = g * adjugate, off-diagonal doubled (nfm_sym_det_backward)
+
+Gauss-Newton builders (G^ = the full symmetric form of a packed gradient with the
+off-diagonals halved, pack(M) = M_ii, 2 M_ij):
+
+  Y = J^T H J            dJ = 2 H J G^, dH = pack(J G^ J^T)     (nfm_sym_matmul_backward)
+  Y = J H J^T (k=d<=3)   dJ = 2 G^ J H, dH = pack(J^T G^ J)
+  y = x x^T              dx = 2 G^ x                            (nfm_sym_outer_backward)
+  F = sym_to_full(p)     dp_ii = G_ii, dp_ij = G_ij + G_ji      (nfm_sym_to_full_backward)
+  x = (J^T H J + diag d)^-1 g0, out = x - alpha (A + lam I + diag d)^-1 v: chains of
+                         nfm_sym_matmul, nfm_sym_solve, nfm_sym_outer2 and the matmul backward
 
 Dense (G = the incoming gradient; for method 'chol' the symmetric part of each matrix
 gradient, torch's convention for cholesky + cholesky_solve / cholesky_inverse):
@@ -465,3 +476,197 @@ def rmdiv(a, b, method, out) -> Tensor:
     """``a b^-1``: the Function's matrix is ``b``."""
     _check_out(out, "rmdiv")
     return _Division.apply(torch.as_tensor(b), torch.as_tensor(a), method, True)
+
+
+# ---------------------------------------------------------------------------
+# Gauss-Newton builders: sym_matmul, sym_outer, sym_to_full, sym_matmul_solve, sym_solve_update
+# ---------------------------------------------------------------------------
+
+def _mode(k: int, d: int) -> int:
+    """J H J^T for k == d <= 3 (the reference's unrolled branches), J^T H J otherwise."""
+    return 1 if (k == d and k <= 3) else 0
+
+
+def _packed_h(j: Tensor, h: Tensor) -> Tensor:
+    """A diagonal Hessian (k values) padded to packed form here, outside the Functions, so that
+    its gradient is the diagonal of the packed one (the backward of torch.cat)."""
+    k = j.shape[-2]
+    if h.shape[-1] == k and k > 1:
+        return torch.cat([h, h.new_zeros((*h.shape[:-1], k * (k - 1) // 2))], -1)
+    return h
+
+
+def matmul_backward(j: Tensor, h: Tensor, g: Tensor, which: int):
+    """(dJ, dH) of ``sym_matmul`` from J (..., k, d), packed H and the packed incoming gradient;
+    ``which`` bit 0 asks for dJ, bit 1 for dH (None where not asked).  With both, one record
+    [dJ | dH] per matrix is written and split into two views."""
+    k, d = j.shape[-2:]
+    kd, kk = k * d, h.shape[-1]
+    batch = _batch((j, 2), (h, 1), (g, 1))
+    out_len = (kd if which & 1 else 0) + (kk if which & 2 else 0)
+    out = _launch("nfm_sym_matmul_backward", k, out_len, batch, [j.flatten(-2), h, g], before=(d, _mode(k, d), which),
+                  dtype=h.dtype, device=h.device)
+    return (out[..., :kd].unflatten(-1, (k, d)) if which & 1 else None,
+            out[..., out_len - kk:] if which & 2 else None)
+
+
+def outer_backward(x: Tensor, g: Tensor) -> Tensor:
+    """Gradient of ``sym_outer``: 2 G^ x."""
+    n = x.shape[-1]
+    return _launch("nfm_sym_outer_backward", n, n, _batch((x, 1), (g, 1)), [x, g], dtype=x.dtype, device=x.device)
+
+
+def to_full_backward(g: Tensor) -> Tensor:
+    """Gradient of ``sym_to_full`` from the (..., n, n) incoming gradient: G_ii, G_ij + G_ji."""
+    n = g.shape[-1]
+    return _launch("nfm_sym_to_full_backward", n, n * (n + 1) // 2, tuple(g.shape[:-2]), [g.flatten(-2)],
+                   dtype=g.dtype, device=g.device)
+
+
+class _SymMatmul(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, j, h):
+        res = S._matmul(j, h)
+        ctx.save_for_backward(j, h)
+        ctx.cdt = res.dtype
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        j, h = ctx.saved_tensors
+        need_j, need_h = ctx.needs_input_grad[:2]
+        dev, cdt = _work_device(h.device), ctx.cdt
+        dj, dh = matmul_backward(j.to(device=dev, dtype=cdt), h.to(device=dev, dtype=cdt), g.to(device=dev, dtype=cdt),
+                                 int(need_j) | 2 * int(need_h))
+        return _grad_for(dj, j), _grad_for(dh, h)
+
+
+def matmul(j, h) -> Tensor:
+    j, h = torch.as_tensor(j), torch.as_tensor(h)
+    return _SymMatmul.apply(j, _packed_h(j, h))
+
+
+class _SymOuter(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x):
+        ctx.save_for_backward(x)
+        return S._outer(x)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        x, = ctx.saved_tensors
+        dev, cdt = _work_device(x.device), D.compute_dtype(x)
+        return _grad_for(outer_backward(x.to(device=dev, dtype=cdt), g.to(device=dev, dtype=cdt)), x)
+
+
+def outer(x) -> Tensor:
+    return _SymOuter.apply(torch.as_tensor(x))
+
+
+class _SymToFull(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, p):
+        ctx.p = _meta(p)
+        return S._to_full(p)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        dev, cdt = _work_device(ctx.p.device), D.compute_dtype(g)
+        return _grad_for(to_full_backward(g.to(device=dev, dtype=cdt)), ctx.p)
+
+
+def to_full(p) -> Tensor:
+    return _SymToFull.apply(torch.as_tensor(p))
+
+
+class _MatmulSolve(torch.autograd.Function):
+    """x = (A + diag d)^-1 g0 with A = sym_matmul(J, H).  Backward recomputes A (nfm_sym_matmul):
+    u = (A + diag d)^-1 G (nfm_sym_solve, 'auto' as the fused kernel), dg0 = u, dA = -S(u, x),
+    dd = -u * x (the diagonal of dA), and (dJ, dH) from dA by the sym_matmul backward."""
+
+    @staticmethod
+    def forward(ctx, j, h, g, diag):
+        res = S._matmul_solve(j, h, g, diag)
+        reg_t = diag if torch.is_tensor(diag) else None
+        ctx.save_for_backward(j, h, res, reg_t)
+        ctx.reg = None if reg_t is not None else diag   # float / sequence regulariser: no gradient
+        ctx.g = _meta(g)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gr):
+        j, h, x, reg_t = ctx.saved_tensors
+        need_j, need_h, need_g, need_d = ctx.needs_input_grad[:4]
+        cdt, d = x.dtype, x.shape[-1]
+        jc, hc = j.to(cdt), h.to(cdt)
+        u = S._solve(S._matmul(jc, hc), gr.to(cdt), reg_t if reg_t is not None else ctx.reg, method="auto")
+        d_j = d_h = d_g = d_d = None
+        if need_g:
+            d_g = _grad_for(u, ctx.g)
+        if need_j or need_h:
+            da = outer2(u, x, _lib.LAYOUT_SYM, -1)
+            dj, dh = matmul_backward(jc, hc, da, int(need_j) | 2 * int(need_h))
+            d_j, d_h = _grad_for(dj, j), _grad_for(dh, h)
+            if need_d:
+                d_d = _grad_for(da[..., :d], reg_t)
+        elif need_d:
+            d_d = _grad_for(outer2(u, x, _lib.LAYOUT_DIAG, -1), reg_t)
+        return d_j, d_h, d_g, d_d
+
+
+def matmul_solve(j, h, g, diag, out) -> Tensor:
+    _check_out(out, "sym_matmul_solve")
+    j, h, g = torch.as_tensor(j), torch.as_tensor(h), torch.as_tensor(g)
+    return _MatmulSolve.apply(j, _packed_h(j, h), g, diag)
+
+
+class _SolveUpdate(torch.autograd.Function):
+    """out = x - alpha s, s = (A + lam I + diag d)^-1 v.  Backward: dx = G; with
+    u = (A + lam I + diag d)^-1 G and s recomputed (nfm_sym_solve, regulariser lam + d, the same
+    method): dv = -alpha u, dp = alpha S(u, s), dd = alpha u * s (the diagonal of dp)."""
+
+    @staticmethod
+    def forward(ctx, x, mat, vec, diag, lam, alpha, method, inplace):
+        res = S._solve_update(x, mat, vec, lam, alpha, x if inplace else None, diag=diag, method=method)
+        if inplace:
+            ctx.mark_dirty(x)
+        reg_t = diag if torch.is_tensor(diag) else None
+        ctx.save_for_backward(mat, vec, reg_t)
+        ctx.reg = None if reg_t is not None else diag
+        ctx.lam, ctx.alpha, ctx.method = float(lam), float(alpha), method
+        ctx.cdt = D.compute_dtype(x, mat, vec)
+        ctx.x = _meta(x)
+        return res
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        mat, vec, reg_t = ctx.saved_tensors
+        need_x, need_m, need_v, need_d = ctx.needs_input_grad[:4]
+        cdt, n = ctx.cdt, vec.shape[-1]
+        d_x = d_m = d_v = d_d = None
+        if need_x:
+            d_x = _grad_for(g, ctx.x)
+        if need_m or need_v or need_d:
+            m = mat.to(cdt)
+            reg = S._as_diag(reg_t if reg_t is not None else ctx.reg, n, cdt, m.device)
+            reg = (ctx.lam or None) if reg is None else reg + ctx.lam
+            ua = S._solve(m, g.to(cdt), reg, method=ctx.method) * ctx.alpha
+            if need_v:
+                d_v = _grad_for(-ua, vec)
+            if need_m or need_d:
+                s = S._solve(m, vec.to(cdt), reg, method=ctx.method)
+                dp = outer2(ua, s, _lib.LAYOUT_SYM if need_m else _lib.LAYOUT_DIAG, 1)
+                d_m = _grad_for(dp, mat) if need_m else None
+                d_d = _grad_for(dp[..., :n], reg_t) if need_d else None
+        return d_x, d_m, d_v, d_d, None, None, None, None
+
+
+def solve_update(x, mat, vec, lam, alpha, out, diag, method, inplace: bool = False) -> Tensor:
+    _check_out(out, "sym_solve_update")
+    x, mat, vec = torch.as_tensor(x), torch.as_tensor(mat), torch.as_tensor(vec)
+    return _SolveUpdate.apply(x, mat, vec, diag, lam, alpha, method, inplace)

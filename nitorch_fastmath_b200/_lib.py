@@ -56,6 +56,9 @@ SIGNATURES = {
     "nfm_sym_outer2": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _I, _P, _L, _P]),
     "nfm_sym_invert_backward": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
     "nfm_sym_det_backward": (c_int, [_I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_sym_matmul_backward": (c_int, [_I, _I, _I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_sym_outer_backward": (c_int, [_I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
+    "nfm_sym_to_full_backward": (c_int, [_I, _I, _L, _P, _L, _P, _L, _P]),
     "nfm_batch_det_backward": (c_int, [_I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
     "nfm_batch_inv_backward": (c_int, [_I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),
     "nfm_batch_outer": (c_int, [_I, _I, _I, _I, _I, _I, _I, _L, _P, _L, _P, _L, _P, _L, _P]),

@@ -397,6 +397,71 @@ int nfm_batch_matvec(int dtype, int m, int n, int64_t batch, const void* mat, in
   return rc;
 }
 
+int nfm_sym_matmul_backward(int dtype, int k, int d, int mode, int which, int64_t batch, const void* jac, int64_t jac_stride,
+                            const void* hess, int64_t hess_stride, const void* grad, int64_t grad_stride, void* out,
+                            int64_t out_stride, void* stream) {
+  if (dtype != NFM_F32 && dtype != NFM_F64) return fail(NFM_E_UNSUPPORTED, "dtype must be NFM_F32 or NFM_F64");
+  if (k < 1 || k > NFM_MAX_N || d < 1 || d > NFM_MAX_N) return fail(NFM_E_UNSUPPORTED, "sym_matmul_backward: 1 <= k, d <= 10");
+  if (mode != 0 && mode != 1) return fail(NFM_E_UNSUPPORTED, "mode must be 0 (J^T H J) or 1 (J H J^T)");
+  if (mode == 1 && k != d) return fail(NFM_E_UNSUPPORTED, "mode 1 needs k == d");
+  if (which < 1 || which > 3) return fail(NFM_E_UNSUPPORTED, "which must be 1 (dJ), 2 (dH) or 3 (both)");
+  if (batch < 0) return fail(NFM_E_BADARG, "negative batch");
+  Args a;
+  a.in(0, jac, jac_stride, true);
+  a.in(1, hess, hess_stride, true);
+  a.in(2, grad, grad_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  auto s = static_cast<cudaStream_t>(stream);
+  if (!fused_shape_built(k, d) || (mode == 1 && k > 3)) {  // the shapes the forward runs on matmul_rt_kernel
+    t_last_path_tma = 0;
+    reset_launch_record();
+    const int rc = dtype == NFM_F32
+                       ? sym_matmul_backward_rt<float>(k, d, mode, which, batch, jac, jac_stride, hess, hess_stride, grad, grad_stride,
+                                                       out, out_stride, s)
+                       : sym_matmul_backward_rt<double>(k, d, mode, which, batch, jac, jac_stride, hess, hess_stride, grad,
+                                                        grad_stride, out, out_stride, s);
+    if (rc) set_error("sym_matmul_backward kernel launch failed: %s", cudaGetErrorString(cudaError_t(rc)));
+    return rc;
+  }
+  if (dtype == NFM_F32) {
+    if (which == 1) return finish(sym_matmul_backward_impl<float, 1>(k, d, mode, a.p, s));
+    if (which == 2) return finish(sym_matmul_backward_impl<float, 2>(k, d, mode, a.p, s));
+    return finish(sym_matmul_backward_impl<float, 3>(k, d, mode, a.p, s));
+  }
+  if (which == 1) return finish(sym_matmul_backward_impl<double, 1>(k, d, mode, a.p, s));
+  if (which == 2) return finish(sym_matmul_backward_impl<double, 2>(k, d, mode, a.p, s));
+  return finish(sym_matmul_backward_impl<double, 3>(k, d, mode, a.p, s));
+}
+
+int nfm_sym_outer_backward(int dtype, int n, int64_t batch, const void* vec, int64_t vec_stride, const void* grad,
+                           int64_t grad_stride, void* out, int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  Args a;
+  a.in(0, vec, vec_stride, true);
+  a.in(1, grad, grad_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  auto s = static_cast<cudaStream_t>(stream);
+  return finish(dtype == NFM_F32 ? sym_outer_backward_impl<float>(n, a.p, s) : sym_outer_backward_impl<double>(n, a.p, s));
+}
+
+int nfm_sym_to_full_backward(int dtype, int n, int64_t batch, const void* grad, int64_t grad_stride, void* out,
+                             int64_t out_stride, void* stream) {
+  int rc = NFM_OK;
+  if (!check_common(dtype, n, batch, rc)) return rc;
+  Args a;
+  a.in(0, grad, grad_stride, true);
+  a.out(out, out_stride);
+  if (a.rc) return a.rc;
+  a.p.batch = batch;
+  auto s = static_cast<cudaStream_t>(stream);
+  return finish(dtype == NFM_F32 ? sym_to_full_backward_impl<float>(n, a.p, s) : sym_to_full_backward_impl<double>(n, a.p, s));
+}
+
 int nfm_batch_det_backward(int dtype, int n, int64_t batch, const void* mat, int64_t mat_stride, const void* grad,
                            int64_t grad_stride, void* out, int64_t out_stride, void* stream) {
   int rc = NFM_OK;

@@ -395,7 +395,76 @@ __global__ void __launch_bounds__(128) matmul_rt_kernel(const T* __restrict__ ja
   }
 }
 
+__device__ __forceinline__ int pidx_rt(int n, int i, int j) {
+  const int lo = i < j ? i : j, hi = i < j ? j : i;
+  return lo == hi ? lo : n + lo * n - (lo * (lo + 1)) / 2 + (hi - lo - 1);
+}
+
+// Gradient of J^T H J (mode 0) / J H J^T (mode 1) for the shapes matmul_rt_kernel runs: the
+// run-time-sized form of SymMatmulBackwardOp (nfm_gn_grad.cu), same formulas, same record layout
+// (`which` 1 = dJ, 2 = dH, 3 = [dJ | dH]).  F(o, a) is the ON x HN factor of Y = F H F^T.
+template <typename T>
+__global__ void __launch_bounds__(128) matmul_backward_rt_kernel(const T* __restrict__ jac, i64 js, const T* __restrict__ hess,
+                                                                 i64 hs, const T* __restrict__ grad, i64 gs, T* __restrict__ out,
+                                                                 i64 os, int k, int d, int mode, int which, i64 batch) {
+  const int hn = mode == 0 ? k : d;  // order of H
+  const int on = mode == 0 ? d : k;  // order of Y
+  const int kj = (which & 1) ? k * d : 0;
+  for (i64 b = i64(blockIdx.x) * blockDim.x + threadIdx.x; b < batch; b += i64(gridDim.x) * blockDim.x) {
+    const T* j = jac + b * js;
+    const T* h = hess + b * hs;
+    const T* g = grad + b * gs;
+    T* dst = out + b * os;
+    auto f = [&](int o, int a) { return mode == 0 ? j[a * d + o] : j[o * d + a]; };
+    auto ghat = [&](int o, int q) { return o == q ? g[o] : T(0.5) * g[pidx_rt(on, o, q)]; };
+    T r[NFM_MAX_N];
+    if (which & 1) {
+      for (int o = 0; o < on; ++o) {  // row o of dF = 2 G^ F H
+        for (int a = 0; a < hn; ++a) {
+          T s = T(0);
+          for (int q = 0; q < on; ++q) s += ghat(o, q) * f(q, a);
+          r[a] = s;
+        }
+        for (int c = 0; c < hn; ++c) {
+          T s = T(0);
+          for (int a = 0; a < hn; ++a) s += r[a] * h[pidx_rt(hn, a, c)];
+          dst[mode == 0 ? c * d + o : o * d + c] = T(2) * s;
+        }
+      }
+    }
+    if (which & 2) {
+      for (int a = 0; a < hn; ++a) {  // row a of F^T G^ F, packed
+        for (int q = 0; q < on; ++q) {
+          T s = T(0);
+          for (int o = 0; o < on; ++o) s += f(o, a) * ghat(o, q);
+          r[q] = s;
+        }
+        for (int c = a; c < hn; ++c) {
+          T s = T(0);
+          for (int q = 0; q < on; ++q) s += r[q] * f(q, c);
+          dst[kj + pidx_rt(hn, a, c)] = a == c ? s : T(2) * s;
+        }
+      }
+    }
+  }
+}
+
 static unsigned grid_for(i64 work);
+
+template <typename T>
+int sym_matmul_backward_rt(int k, int d, int mode, int which, i64 batch, const void* jac, i64 js, const void* hess, i64 hs,
+                           const void* grad, i64 gs, void* out, i64 os, cudaStream_t s) {
+  if (batch == 0) return 0;
+  matmul_backward_rt_kernel<T><<<grid_for(batch), 128, 0, s>>>(static_cast<const T*>(jac), js, static_cast<const T*>(hess), hs,
+                                                               static_cast<const T*>(grad), gs, static_cast<T*>(out), os, k, d,
+                                                               mode, which, batch);
+  g_launch_count.fetch_add(1, std::memory_order_relaxed);
+  return int(cudaGetLastError());
+}
+template int sym_matmul_backward_rt<float>(int, int, int, int, i64, const void*, i64, const void*, i64, const void*, i64, void*, i64,
+                                           cudaStream_t);
+template int sym_matmul_backward_rt<double>(int, int, int, int, i64, const void*, i64, const void*, i64, const void*, i64, void*,
+                                            i64, cudaStream_t);
 
 template <typename T>
 int sym_matmul_rt(int k, int d, int mode, i64 batch, const void* jac, i64 js, const void* hess, i64 hs, void* out, i64 os,

@@ -65,12 +65,19 @@ int batch_outer_rt(int m, int n, int k, int rows, int sym, int sign, i64 batch, 
 
 // nfm_fused.cu: register kernels for 1 <= k, d <= 6 and for tall Jacobians k <= 10, d <= 3
 constexpr int kFusedMaxOrder = 6;
-inline bool fused_shape_built(int k, int d) {
+constexpr bool fused_shape_built(int k, int d) {
   return k >= 1 && d >= 1 && ((k <= kFusedMaxOrder && d <= kFusedMaxOrder) || (k <= NFM_MAX_N && d <= 3));
 }
 template <typename T> int sym_matmul_impl(int k, int d, int mode, const KParams& p, cudaStream_t s);
 template <typename T> int sym_matmul_solve_impl(int k, int d, int mode, const KParams& p, cudaStream_t s);
 template <typename T> int sym_solve_update_impl(int n, int algo, const KParams& p, cudaStream_t s);
+
+// backward kernels of the Gauss-Newton builders (nfm_gn_grad.cu): sym_matmul for the shapes of
+// fused_shape_built (WHICH 1 = dJ, 2 = dH, 3 = both in one record; parts 0 / 1 / 2), sym_outer and
+// sym_to_full (part 3)
+template <typename T, int WHICH> int sym_matmul_backward_impl(int k, int d, int mode, const KParams& p, cudaStream_t s);
+template <typename T> int sym_outer_backward_impl(int n, const KParams& p, cudaStream_t s);
+template <typename T> int sym_to_full_backward_impl(int n, const KParams& p, cudaStream_t s);
 
 // nrhs > 4 and right division: register factorisation (order templated), run-time loop over
 // the right-hand sides (nfm_generic.cu)
@@ -81,5 +88,9 @@ int batch_solve_many(int n, int nrhs, int chol, int right, i64 batch, const void
 template <typename T>
 int sym_matmul_rt(int k, int d, int mode, i64 batch, const void* jac, i64 js, const void* hess, i64 hs, void* out, i64 os,
                   cudaStream_t s);
+// the gradient of sym_matmul for the other shapes (records as SymMatmulBackwardOp)
+template <typename T>
+int sym_matmul_backward_rt(int k, int d, int mode, int which, i64 batch, const void* jac, i64 js, const void* hess, i64 hs,
+                           const void* grad, i64 gs, void* out, i64 os, cudaStream_t s);
 
 }  // namespace nfm

@@ -18,9 +18,10 @@ their device, CPU tensors are streamed through the current CUDA device, and
 without a CUDA device or without the built library every call raises.
 
 Gradients: sym_matvec, sym_addmatvec(_), sym_submatvec(_), sym_solve(_), sym_invert(_)
-and sym_det are differentiable (packed, diagonal and scaled-identity layouts); the
-backward passes run on the library's kernels (``_autograd.py``).  Without a needed
-gradient each function runs its plain path unchanged.
+and sym_det are differentiable (packed, diagonal and scaled-identity layouts), and so
+are the Gauss-Newton builders sym_matmul, sym_outer, sym_to_full, sym_matmul_solve and
+sym_solve_update(_); the backward passes run on the library's kernels
+(``_autograd.py``).  Without a needed gradient each function runs its plain path unchanged.
 
 Signatures are the union of the reference's in-repo implementation
 (nitorch_fastmath/_impl/sym.py) and the ``jitfields.sym`` functions that
@@ -417,7 +418,17 @@ def sym_solve_update(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alph
     sym.py:31-33); not a function of the reference.  CUDA tensors only;
     ``mat (..., M*(M+1)//2)``, ``vec`` and ``x`` ``(..., M)``; ``diag`` is the
     reference's per-voxel regulariser ``(..., M)`` (or anything broadcastable to it).
+    Differentiable with respect to ``x``, ``mat``, ``vec`` and a tensor ``diag``.
     """
+    if (getattr(x, "requires_grad", False) or getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
+            or getattr(diag, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.solve_update(x, mat, vec, lam, alpha, out, diag, method)
+    return _solve_update(x, mat, vec, lam, alpha, out, diag=diag, method=method)
+
+
+def _solve_update(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alpha: float = 1.0,
+                  out: Optional[Tensor] = None, *, diag: Optional[Tensor] = None,
+                  method: Optional[str] = None) -> Tensor:
     x, mat, vec = torch.as_tensor(x), torch.as_tensor(mat), torch.as_tensor(vec)
     dev = D.common_device(x, mat, vec)
     if dev.type != "cuda":
@@ -454,7 +465,10 @@ def sym_solve_update(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alph
 def sym_solve_update_(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alpha: float = 1.0, *,
                       diag: Optional[Tensor] = None, method: Optional[str] = None) -> Tensor:
     r"""In-place ``x -= alpha * (mat + lam*I + diag(d)) \ vec``; returns ``x``."""
-    return sym_solve_update(x, mat, vec, lam, alpha, out=x, diag=diag, method=method)
+    if (getattr(x, "requires_grad", False) or getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
+            or getattr(diag, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.solve_update(x, mat, vec, lam, alpha, None, diag, method, inplace=True)
+    return _solve_update(x, mat, vec, lam, alpha, out=x, diag=diag, method=method)
 
 
 def sym_matmul_solve(j: Tensor, h: Tensor, g: Tensor, diag=None, out: Optional[Tensor] = None) -> Tensor:
@@ -466,7 +480,15 @@ def sym_matmul_solve(j: Tensor, h: Tensor, g: Tensor, diag=None, out: Optional[T
     diagonal ``(..., k)``, ``g (..., d)``, ``diag`` float / sequence / ``(..., d)``;
     ``1 <= k, d <= 6`` or ``k <= 10`` with ``d <= 3``; CUDA tensors.  Like ``sym_matmul`` it evaluates ``J H J^T``
     for ``k == d <= 3`` (the reference's unrolled branches).  Not a function of the reference.
+    Differentiable with respect to ``j``, ``h``, ``g`` and a tensor ``diag``.
     """
+    if (getattr(j, "requires_grad", False) or getattr(h, "requires_grad", False) or getattr(g, "requires_grad", False)
+            or getattr(diag, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.matmul_solve(j, h, g, diag, out)
+    return _matmul_solve(j, h, g, diag, out)
+
+
+def _matmul_solve(j: Tensor, h: Tensor, g: Tensor, diag=None, out: Optional[Tensor] = None) -> Tensor:
     j, h, g = torch.as_tensor(j), torch.as_tensor(h), torch.as_tensor(g)
     dev = D.common_device(j, h, g)
     if dev.type != "cuda":
@@ -623,6 +645,12 @@ def _unary(fn_name: str, x: Tensor, n: int, out_shape, rec_ndim_out: int) -> Ten
 
 def sym_to_full(mat: Tensor) -> Tensor:
     """Compact symmetric -> full `(..., M, M)`  (reference _impl/sym.py:16-60)."""
+    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+        return A.to_full(mat)
+    return _to_full(mat)
+
+
+def _to_full(mat: Tensor) -> Tensor:
     mat = torch.as_tensor(mat)
     n = D.packed_order(mat.shape[-1])
     _check_n(n)
@@ -637,6 +665,12 @@ def sym_diag(mat: Tensor) -> Tensor:
 
 def sym_outer(x: Tensor) -> Tensor:
     """Symmetric outer product ``x x^T`` in compact storage (reference _impl/sym.py:496-528)."""
+    if getattr(x, "requires_grad", False) and torch.is_grad_enabled():
+        return A.outer(x)
+    return _outer(x)
+
+
+def _outer(x: Tensor) -> Tensor:
     x = torch.as_tensor(x)
     n = x.shape[-1]
     _check_n(n)
@@ -665,13 +699,20 @@ def sym_matmul(j: Tensor, h: Tensor) -> Tensor:
     ``h`` `(..., k*(k+1)//2)`, result `(..., d*(d+1)//2)`.  Note that for
     ``k == d <= 3`` the reference's unrolled branches (:532-593) evaluate
     :math:`J H J^T`; this drop-in reproduces that (C ABI ``mode=1``).
+    Differentiable with respect to ``j`` and ``h`` (also a diagonal ``h``).
     """
+    if (getattr(j, "requires_grad", False) or getattr(h, "requires_grad", False)) and torch.is_grad_enabled():
+        return A.matmul(j, h)
+    return _matmul(j, h)
+
+
+def _matmul(j: Tensor, h: Tensor) -> Tensor:
     j, h = torch.as_tensor(j), torch.as_tensor(h)
     dev = D.common_device(j, h)
     if dev.type != "cuda":
         _host.offload_device()   # raises when there is no CUDA device: no CPU path
         (dj, dh), _ = _to_device_inputs(j, h)
-        return sym_matmul(dj, dh).cpu()
+        return _matmul(dj, dh).cpu()
     k, d = j.shape[-2:]
     if not (1 <= k <= _lib.MAX_N and 1 <= d <= _lib.MAX_N):
         raise ValueError(f"sym_matmul supports 1 <= k, d <= {_lib.MAX_N}")

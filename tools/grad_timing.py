@@ -4,7 +4,10 @@ bandwidth of the backward kernels (nfm_sym_outer2, nfm_sym_invert_backward,
 nfm_sym_det_backward) against the measured copy peak.  ``--dense`` measures the dense
 routines instead (batchdet, batchinv, solvevec, lmdiv, rmdiv; nfm_batch_inv_backward,
 nfm_batch_det_backward, nfm_batch_outer, nfm_batch_tsolve) and autograd through torch's
-own linalg functions on the same GPU.
+own linalg functions on the same GPU.  ``--gn`` measures the Gauss-Newton builders
+(sym_matmul, sym_matmul_solve, sym_solve_update, sym_outer, sym_to_full;
+nfm_sym_matmul_backward, nfm_sym_outer_backward, nfm_sym_to_full_backward) and autograd
+through the oracle on the same GPU.
 
 CUDA events around many calls after a warm-up; every field is larger than the
 126 MB L2 of a B200 (except the tiny-batch gate-cost rows, which time host work).
@@ -180,10 +183,107 @@ def dense(peak):
             torch.cuda.empty_cache()
 
 
+def jacobian(shape, k, d, dtype, seed):
+    """0.1 randn plus ones on the leading diagonal, built on the GPU."""
+    j = vecs(shape + (k,), d, dtype, seed) * 0.1
+    j[..., range(min(k, d)), range(min(k, d))] += 1.0
+    return j
+
+
+def gn(peak):
+    lib = _lib.load()
+    f32 = torch.float32
+    say("== Gauss-Newton builders: forward / backward (all inputs), fp32, fields larger than L2 ==")
+    for side, k, d in ((160, 10, 3), (192, 6, 6), (256, 3, 3)):
+        shape = (side, side, side)
+        mode1 = k == d and k <= 3
+        kh, ko = (d, k) if mode1 else (k, d)
+        j, h = jacobian(shape, k, d, f32, 1).requires_grad_(), field(shape, kh, f32, 2).requires_grad_()
+        tag = f"{side}^3 k={k} d={d}" + (" (mode 1)" if mode1 else "")
+        fwd_bwd(f"sym_matmul {tag}", nfm.sym_matmul, [j, h], vecs(shape, ko * (ko + 1) // 2, f32, 3))
+        g0 = vecs(shape, ko, f32, 4).requires_grad_()
+        fwd_bwd(f"sym_matmul_solve {tag}", lambda j, h, g0: nfm.sym_matmul_solve(j, h, g0, 1.0), [j, h, g0], vecs(shape, ko, f32, 5))
+        del j, h, g0
+        torch.cuda.empty_cache()
+    shape = (256, 256, 256)
+    x, m, v = vecs(shape, 3, f32, 1).requires_grad_(), field(shape, 3, f32, 2).requires_grad_(), vecs(shape, 3, f32, 3).requires_grad_()
+    gs = vecs(shape, 3, f32, 4)
+    fwd_bwd("sym_solve_update 256^3 N=3", lambda x, m, v: nfm.sym_solve_update(x, m, v, 0.1, 0.5), [x, m, v], gs)
+    fwd_bwd("sym_outer 256^3 N=3", nfm.sym_outer, [x], vecs(shape, 6, f32, 5))
+    del x, m, v, gs
+    torch.cuda.empty_cache()
+    shape = (192, 192, 192)
+    m = field(shape, 6, f32, 1).requires_grad_()
+    fwd_bwd("sym_to_full 192^3 N=6", nfm.sym_to_full, [m], vecs(shape + (6,), 6, f32, 2))
+    del m
+    torch.cuda.empty_cache()
+
+    say()
+    say("== autograd through the oracle (eager torch, what the reference does), same GPU, fp32 ==")
+    shape = (192, 192, 192)
+    j, h = jacobian(shape, 6, 6, f32, 1).requires_grad_(), field(shape, 6, f32, 2).requires_grad_()
+    fwd_bwd("oracle sym_matmul 192^3 k=6 d=6", P.sym_matmul, [j, h], vecs(shape, 21, f32, 3))
+    del j, h
+    torch.cuda.empty_cache()
+    shape = (256, 256, 256)
+    j, h, g0 = jacobian(shape, 3, 3, f32, 1).requires_grad_(), field(shape, 3, f32, 2).requires_grad_(), vecs(shape, 3, f32, 4).requires_grad_()
+    one = torch.ones(3, device=DEV, dtype=f32)     # the oracle takes a float regulariser on the CPU only
+    fwd_bwd("oracle sym_matmul_solve 256^3 k=d=3 (mode 1)", lambda j, h, g0: P.sym_solve(P.sym_matmul(j, h), g0, one),
+            [j, h, g0], vecs(shape, 3, f32, 5))
+    del j, h
+    m, x = field(shape, 3, f32, 2).requires_grad_(), vecs(shape, 3, f32, 1).requires_grad_()
+    fwd_bwd("oracle sym_solve_update 256^3 N=3", lambda x, m, v: x - 0.5 * P.sym_solve(m, v, 0.1 * one), [x, m, g0], vecs(shape, 3, f32, 6))
+    fwd_bwd("oracle sym_outer 256^3 N=3", P.sym_outer, [x], vecs(shape, 6, f32, 5))
+    del m, x, g0
+    torch.cuda.empty_cache()
+    shape = (192, 192, 192)
+    m = field(shape, 6, f32, 1).requires_grad_()
+    fwd_bwd("oracle sym_to_full 192^3 N=6", P.sym_to_full, [m], vecs(shape + (6,), 6, f32, 2))
+    del m
+    torch.cuda.empty_cache()
+
+    say()
+    say("== Gauss-Newton backward kernels: algorithmic bytes / time, against the copy peak ==")
+    say("   matmul backward (J, H, g in; dJ and / or dH out), outer backward (2N + NN) s, to_full backward (N^2 + NN) s")
+    say(f"{'kernel':44s} {'dtype':8s} {'batch':>10s} {'us':>10s} {'GB/s':>8s} {'of peak':>8s} path")
+
+    def row(label, dtype, batch, fn, nelem):
+        ms = ev_time(fn)
+        path = lib.nfm_last_path_was_tma()
+        gbs = nelem * torch.tensor([], dtype=dtype).element_size() * batch / ms / 1e6
+        say(f"{label:44s} {str(dtype)[6:]:8s} {batch:10d} {ms * 1e3:10.1f} {gbs:8.0f} {gbs / peak:8.2f} {path}")
+
+    for dtype in (torch.float32, torch.float64):
+        s = torch.tensor([], dtype=dtype).element_size()
+        for k, d in ((3, 3), (6, 6), (10, 3), (10, 10)):
+            mode1 = k == d and k <= 3
+            kh, ko = (d, k) if mode1 else (k, d)
+            hh, oo = kh * (kh + 1) // 2, ko * (ko + 1) // 2
+            batch = int(2e9 // ((2 * k * d + 2 * hh + oo) * s))
+            j, h, g = jacobian((batch,), k, d, dtype, 1), field((batch,), kh, dtype, 2), vecs((batch,), oo, dtype, 3)
+            for which, name, nout in ((1, "dJ", k * d), (2, "dH", hh), (3, "dJ+dH", k * d + hh)):
+                row(f"matmul backward k={k} d={d} {name}", dtype, batch, lambda: A.matmul_backward(j, h, g, which),
+                    k * d + hh + oo + nout)
+            del j, h, g
+            torch.cuda.empty_cache()
+        for n in (3, 6, 10):
+            nn = n * (n + 1) // 2
+            batch = int(2e9 // ((2 * n + nn) * s))
+            x, g = vecs((batch,), n, dtype, 1), vecs((batch,), nn, dtype, 2)
+            row(f"outer backward N={n}", dtype, batch, lambda: A.outer_backward(x, g), 2 * n + nn)
+            del x, g
+            batch = int(2e9 // ((n * n + nn) * s))
+            g = vecs((batch, n), n, dtype, 3)
+            row(f"to_full backward N={n}", dtype, batch, lambda: A.to_full_backward(g), n * n + nn)
+            del g
+            torch.cuda.empty_cache()
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__)
     ap.add_argument("--out", default=None)
     ap.add_argument("--dense", action="store_true", help="measure the dense routines instead of the packed ones")
+    ap.add_argument("--gn", action="store_true", help="measure the Gauss-Newton builders instead of the packed solves")
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("grad_timing needs a CUDA device")
@@ -193,8 +293,8 @@ def main():
     peak = copy_peak()
     say(f"measured copy peak (2 GiB device-to-device copy, read + write bytes): {peak:.0f} GB/s")
     say()
-    if args.dense:
-        dense(peak)
+    if args.dense or args.gn:
+        (dense if args.dense else gn)(peak)
         if args.out:
             with open(args.out, "w") as fh:
                 fh.write("\n".join(LINES) + "\n")
