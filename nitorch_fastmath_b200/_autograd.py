@@ -69,28 +69,12 @@ def _layout_len(layout: int, n: int) -> int:
     return {_lib.LAYOUT_SCALED_IDENTITY: 1, _lib.LAYOUT_DIAG: n, _lib.LAYOUT_SYM: n * (n + 1) // 2}[layout]
 
 
-def _launch(name: str, n: int, out_len: int, batch, operands, *args, before=(), dtype, device) -> Tensor:
-    """Run one backward kernel over ``batch``: every operand (trailing dim = its record) is
-    broadcast to ``batch`` and handed over as (pointer, batch stride); ``before`` / ``args`` are
-    the scalar arguments ahead of / between the operands and the output."""
-    out = torch.empty((*batch, out_len), dtype=dtype, device=device)
-    nb = D.batch_count(batch)
-    if nb > 0 and out_len > 0:
-        ops = [D.as_operand(t, batch, 1, dtype) for t in operands]
-        ptrs = [x for o in ops for x in (o.ptr, o.stride)]
-        with D.device_of(device):
-            rc = getattr(_lib.load(), name)(D.dtype_code(dtype), n, *before, nb, *ptrs, *args, out.data_ptr(), out_len,
-                                           D.current_stream_ptr(device))
-        _lib.check(rc, name)
-    return out
-
-
 def outer2(u: Tensor, w: Tensor, layout: int, sign: int) -> Tensor:
     """``sign * S(u, w)`` in ``layout``: records of 1 / N / N(N+1)/2 over the broadcast batch of u, w."""
     n = u.shape[-1]
     batch = tuple(torch.broadcast_shapes(u.shape[:-1], w.shape[:-1]))
-    return _launch("nfm_sym_outer2", n, _layout_len(layout, n), batch, [u, w], sign,
-                   before=(layout,), dtype=u.dtype, device=u.device)
+    return D.launch("nfm_sym_outer2", (n, layout), batch, [(u, 1), (w, 1)], (sign,), rec=(_layout_len(layout, n),),
+                    dtype=u.dtype, device=u.device, skip_empty=True)
 
 
 def invert_backward(inv: Tensor, grad: Tensor, diag_only: bool) -> Tensor:
@@ -98,16 +82,16 @@ def invert_backward(inv: Tensor, grad: Tensor, diag_only: bool) -> Tensor:
     nn = inv.shape[-1]
     n = D.packed_order(nn)
     batch = tuple(torch.broadcast_shapes(inv.shape[:-1], grad.shape[:-1]))
-    return _launch("nfm_sym_invert_backward", n, nn, batch, [inv, grad],
-                   before=(int(bool(diag_only)),), dtype=inv.dtype, device=inv.device)
+    return D.launch("nfm_sym_invert_backward", (n, int(bool(diag_only))), batch, [(inv, 1), (grad, 1)], rec=(nn,),
+                    dtype=inv.dtype, device=inv.device, skip_empty=True)
 
 
 def det_backward(mat: Tensor, grad: Tensor) -> Tensor:
     """Gradient of ``sym_det`` with respect to the packed matrix; ``grad`` has the batch shape."""
     nn = mat.shape[-1]
     batch = tuple(torch.broadcast_shapes(mat.shape[:-1], grad.shape))
-    return _launch("nfm_sym_det_backward", D.packed_order(nn), nn, batch, [mat, grad.unsqueeze(-1)],
-                   dtype=mat.dtype, device=mat.device)
+    return D.launch("nfm_sym_det_backward", (D.packed_order(nn),), batch, [(mat, 1), (grad.unsqueeze(-1), 1)], rec=(nn,),
+                    dtype=mat.dtype, device=mat.device, skip_empty=True)
 
 
 def _work_device(dev: torch.device) -> torch.device:
@@ -326,16 +310,16 @@ def dense_det_backward(a: Tensor, g: Tensor) -> Tensor:
     """g * adj(A)^T for (..., n, n) matrices and (...) incoming gradients."""
     n = a.shape[-1]
     batch = _batch((a, 2), (g, 0))
-    return _launch("nfm_batch_det_backward", n, n * n, batch, [a.flatten(-2), g.unsqueeze(-1)],
-                   dtype=a.dtype, device=a.device).view(*batch, n, n)
+    return D.launch("nfm_batch_det_backward", (n,), batch, [(a.flatten(-2), 1), (g.unsqueeze(-1), 1)], rec=(n * n,),
+                    dtype=a.dtype, device=a.device, skip_empty=True).view(*batch, n, n)
 
 
 def dense_inv_backward(y: Tensor, g: Tensor, sym: bool) -> Tensor:
     """-Y^T G Y^T, or -Y (G + G^T) Y / 2 when ``sym``, from the inverse Y."""
     n = y.shape[-1]
     batch = _batch((y, 2), (g, 2))
-    return _launch("nfm_batch_inv_backward", n, n * n, batch, [y.flatten(-2), g.flatten(-2)], before=(int(sym),),
-                   dtype=y.dtype, device=y.device).view(*batch, n, n)
+    return D.launch("nfm_batch_inv_backward", (n, int(sym)), batch, [(y.flatten(-2), 1), (g.flatten(-2), 1)],
+                    rec=(n * n,), dtype=y.dtype, device=y.device, skip_empty=True).view(*batch, n, n)
 
 
 def dense_outer(u: Tensor, w: Tensor, rows: bool, sym: bool, sign: int) -> Tensor:
@@ -346,8 +330,9 @@ def dense_outer(u: Tensor, w: Tensor, rows: bool, sym: bool, sign: int) -> Tenso
     batch = _batch((u, 2), (w, 2))
     if k == 0:
         return torch.zeros((*batch, m, n), dtype=u.dtype, device=u.device)
-    return _launch("nfm_batch_outer", m, m * n, batch, [u.flatten(-2), w.flatten(-2)],
-                   before=(n, k, int(rows), int(sym), sign), dtype=u.dtype, device=u.device).view(*batch, m, n)
+    return D.launch("nfm_batch_outer", (m, n, k, int(rows), int(sym), sign), batch,
+                    [(u.flatten(-2), 1), (w.flatten(-2), 1)], rec=(m * n,), dtype=u.dtype, device=u.device,
+                    skip_empty=True).view(*batch, m, n)
 
 
 def dense_tsolve(a: Tensor, b: Tensor, right: bool, algo: int) -> Tensor:
@@ -355,15 +340,16 @@ def dense_tsolve(a: Tensor, b: Tensor, right: bool, algo: int) -> Tensor:
     n = a.shape[-1]
     k = b.shape[-2] if right else b.shape[-1]
     batch = _batch((a, 2), (b, 2))
-    return _launch("nfm_batch_tsolve", n, n * k, batch, [a.flatten(-2), b.flatten(-2)], before=(k, int(right), algo),
-                   dtype=a.dtype, device=a.device).view(*batch, *b.shape[-2:])
+    return D.launch("nfm_batch_tsolve", (n, k, int(right), algo), batch, [(a.flatten(-2), 1), (b.flatten(-2), 1)],
+                    rec=(n * k,), dtype=a.dtype, device=a.device, skip_empty=True).view(*batch, *b.shape[-2:])
 
 
 def dense_tmatvec(a: Tensor, v: Tensor) -> Tensor:
     """``A^T v`` for A: (..., m, n), v: (..., m)."""
     m, n = a.shape[-2:]
     batch = _batch((a, 2), (v, 1))
-    return _launch("nfm_batch_tmatvec", m, n, batch, [a.flatten(-2), v], before=(n,), dtype=a.dtype, device=a.device)
+    return D.launch("nfm_batch_tmatvec", (m, n), batch, [(a.flatten(-2), 1), (v, 1)], rec=(n,), dtype=a.dtype,
+                    device=a.device, skip_empty=True)
 
 
 class _BatchDet(torch.autograd.Function):
@@ -482,20 +468,6 @@ def rmdiv(a, b, method, out) -> Tensor:
 # Gauss-Newton builders: sym_matmul, sym_outer, sym_to_full, sym_matmul_solve, sym_solve_update
 # ---------------------------------------------------------------------------
 
-def _mode(k: int, d: int) -> int:
-    """J H J^T for k == d <= 3 (the reference's unrolled branches), J^T H J otherwise."""
-    return 1 if (k == d and k <= 3) else 0
-
-
-def _packed_h(j: Tensor, h: Tensor) -> Tensor:
-    """A diagonal Hessian (k values) padded to packed form here, outside the Functions, so that
-    its gradient is the diagonal of the packed one (the backward of torch.cat)."""
-    k = j.shape[-2]
-    if h.shape[-1] == k and k > 1:
-        return torch.cat([h, h.new_zeros((*h.shape[:-1], k * (k - 1) // 2))], -1)
-    return h
-
-
 def matmul_backward(j: Tensor, h: Tensor, g: Tensor, which: int):
     """(dJ, dH) of ``sym_matmul`` from J (..., k, d), packed H and the packed incoming gradient;
     ``which`` bit 0 asks for dJ, bit 1 for dH (None where not asked).  With both, one record
@@ -504,8 +476,8 @@ def matmul_backward(j: Tensor, h: Tensor, g: Tensor, which: int):
     kd, kk = k * d, h.shape[-1]
     batch = _batch((j, 2), (h, 1), (g, 1))
     out_len = (kd if which & 1 else 0) + (kk if which & 2 else 0)
-    out = _launch("nfm_sym_matmul_backward", k, out_len, batch, [j.flatten(-2), h, g], before=(d, _mode(k, d), which),
-                  dtype=h.dtype, device=h.device)
+    out = D.launch("nfm_sym_matmul_backward", (k, d, S._mode(k, d), which), batch, [(j.flatten(-2), 1), (h, 1), (g, 1)],
+                   rec=(out_len,), dtype=h.dtype, device=h.device, skip_empty=True)
     return (out[..., :kd].unflatten(-1, (k, d)) if which & 1 else None,
             out[..., out_len - kk:] if which & 2 else None)
 
@@ -513,14 +485,15 @@ def matmul_backward(j: Tensor, h: Tensor, g: Tensor, which: int):
 def outer_backward(x: Tensor, g: Tensor) -> Tensor:
     """Gradient of ``sym_outer``: 2 G^ x."""
     n = x.shape[-1]
-    return _launch("nfm_sym_outer_backward", n, n, _batch((x, 1), (g, 1)), [x, g], dtype=x.dtype, device=x.device)
+    return D.launch("nfm_sym_outer_backward", (n,), _batch((x, 1), (g, 1)), [(x, 1), (g, 1)], rec=(n,), dtype=x.dtype,
+                    device=x.device, skip_empty=True)
 
 
 def to_full_backward(g: Tensor) -> Tensor:
     """Gradient of ``sym_to_full`` from the (..., n, n) incoming gradient: G_ii, G_ij + G_ji."""
     n = g.shape[-1]
-    return _launch("nfm_sym_to_full_backward", n, n * (n + 1) // 2, tuple(g.shape[:-2]), [g.flatten(-2)],
-                   dtype=g.dtype, device=g.device)
+    return D.launch("nfm_sym_to_full_backward", (n,), tuple(g.shape[:-2]), [(g.flatten(-2), 1)], rec=(n * (n + 1) // 2,),
+                    dtype=g.dtype, device=g.device, skip_empty=True)
 
 
 class _SymMatmul(torch.autograd.Function):
@@ -544,7 +517,7 @@ class _SymMatmul(torch.autograd.Function):
 
 def matmul(j, h) -> Tensor:
     j, h = torch.as_tensor(j), torch.as_tensor(h)
-    return _SymMatmul.apply(j, _packed_h(j, h))
+    return _SymMatmul.apply(j, S._packed_h(j, h))
 
 
 class _SymOuter(torch.autograd.Function):
@@ -621,7 +594,7 @@ class _MatmulSolve(torch.autograd.Function):
 def matmul_solve(j, h, g, diag, out) -> Tensor:
     _check_out(out, "sym_matmul_solve")
     j, h, g = torch.as_tensor(j), torch.as_tensor(h), torch.as_tensor(g)
-    return _MatmulSolve.apply(j, _packed_h(j, h), g, diag)
+    return _MatmulSolve.apply(j, S._packed_h(j, h), g, diag)
 
 
 class _SolveUpdate(torch.autograd.Function):

@@ -12,6 +12,7 @@ pass; documented in DESIGN.md).
 """
 from __future__ import annotations
 
+import itertools
 import math
 from typing import Optional, Sequence, Tuple
 
@@ -50,9 +51,10 @@ def common_device(*tensors) -> torch.device:
     return dev
 
 
-def require_cuda(dev: torch.device) -> None:
-    if dev.type != "cuda":
-        raise RuntimeError("internal: device path called with non-CUDA tensors")
+def check_order(n: int) -> int:
+    if not 1 <= n <= _lib.MAX_N:
+        raise ValueError(f"matrix order {n} is outside the supported range 1..{_lib.MAX_N}")
+    return n
 
 
 def _record_contiguous(t: torch.Tensor, rec_ndim: int) -> bool:
@@ -191,8 +193,62 @@ def outer_views(t: Optional[torch.Tensor], batch_shape: Tuple[int, ...], rec_ndi
     return t.expand(*batch_shape, *rec_shape)[idx]
 
 
+def outer_loop(batch: Tuple[int, ...], operands: Sequence[Tuple[Optional[torch.Tensor], int]],
+               out: Optional[torch.Tensor], rec: Tuple[int, ...], dtype: torch.dtype, device: torch.device,
+               call) -> Optional[torch.Tensor]:
+    """Partially broadcast operands (see ``outer_split``): ``call(*operand views, out view)`` once per
+    index of the leading batch dims, on views, so nothing is materialised and each call sees dense or
+    fully broadcast operands.  Returns ``out`` (or a new ``dtype`` tensor) filled, or None when no
+    split applies and the caller launches once."""
+    split = outer_split(batch, operands) if batch_count(batch) > 0 else 0
+    if not split:
+        return None
+    shape = (*batch, *rec)
+    full = out if (out is not None and out.dtype == dtype and tuple(out.shape) == shape) else \
+        torch.empty(shape, dtype=dtype, device=device)
+    for idx in itertools.product(*[range(k) for k in batch[:split]]):
+        call(*[outer_views(t, batch, nd, idx) for t, nd in operands], full[idx])
+    if out is not None and full is not out:
+        out.copy_(full)
+        return out
+    return full
+
+
 def batch_count(batch_shape: Sequence[int]) -> int:
     return math.prod(batch_shape)
+
+
+def launch(fn_name: str, head: Sequence, batch: Tuple[int, ...],
+           operands: Sequence[Tuple[Optional[torch.Tensor], int]], tail: Sequence = (), *,
+           rec: Tuple[int, ...], out: Optional[torch.Tensor] = None, dtype: torch.dtype, device: torch.device,
+           struct: bool = False, skip_empty: bool = False, what: Optional[str] = None) -> torch.Tensor:
+    """Run the device entry ``fn_name(dtype code, *head, nb, *operands, *tail, out, stream)`` over
+    ``batch`` on ``device`` and return its ``(*batch, *rec)`` result (``out`` when given).
+
+    Each ``(tensor, rec_ndim)`` operand is broadcast to ``batch`` and passed as (pointer, batch
+    stride), an absent one as (NULL, 0).  With ``struct`` the ``fn_name + "_ex"`` entry is called
+    with ``nfm_operand`` pointers, which also carry an element stride, so strided 1-D records are
+    passed without a copy; an absent operand is a NULL struct.  An ``out`` the library cannot write
+    through (another dtype, batch dims that do not collapse) is written through a temporary and
+    copied back.  The call is skipped when the batch is empty, or with ``skip_empty`` when the result
+    is; errors are reported as ``what`` (default ``fn_name``)."""
+    o, res, copy_back = out_operand(out, batch + rec, len(rec), dtype, device, struct)
+    nb = math.prod(batch)
+    if nb > 0 and not (skip_empty and res.numel() == 0):
+        # ``ops`` keeps every Operand, and with it any converted or materialised copy, alive until
+        # the call has been enqueued: the pointers below would otherwise dangle
+        ops = [None if t is None else as_operand(t, batch, nd, dtype, struct) for t, nd in operands]
+        if struct:
+            args = [None if x is None else x.c_struct() for x in ops] + [*tail, o.c_struct()]
+        else:
+            args = [v for x in ops for v in ((None, 0) if x is None else (x.ptr, x.stride))] + [*tail, o.ptr, o.stride]
+        fn = getattr(_lib.load(), fn_name + "_ex" if struct else fn_name)
+        with device_of(device):
+            rc = fn(dtype_code(dtype), *head, nb, *args, current_stream_ptr(device))
+        _lib.check(rc, what or fn_name)
+    if copy_back:
+        res.copy_(o.tensor)
+    return res
 
 
 def current_stream_ptr(device: torch.device) -> int:

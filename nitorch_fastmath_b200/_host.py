@@ -57,6 +57,18 @@ def offload_device() -> torch.device:
     return torch.device("cuda", torch.cuda.current_device())
 
 
+def uploaded(call, *tensors: Optional[torch.Tensor], out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The route for CPU operands that are not streamed: upload ``tensors`` whole to the current
+    CUDA device, run ``call`` (the device path) on them and bring its result back, into ``out`` or
+    as a new CPU tensor."""
+    dev = offload_device()
+    r = call(*[None if t is None else t.to(dev, non_blocking=True) for t in tensors])
+    if out is not None:
+        out.copy_(r)
+        return out
+    return r.cpu()
+
+
 def is_plain(t: Optional[torch.Tensor]) -> bool:
     return t is None or (t.device.type == "cpu" and t.is_contiguous())
 

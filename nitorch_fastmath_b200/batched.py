@@ -20,15 +20,7 @@ __all__ = ['batchmatvec', 'batchdet', 'batchinv']
 def _square_order(a: Tensor) -> int:
     if a.dim() < 2 or a.shape[-1] != a.shape[-2]:
         raise ValueError(f"expected (..., n, n) matrices, got {tuple(a.shape)}")
-    n = a.shape[-1]
-    if not 1 <= n <= _lib.MAX_N:
-        raise ValueError(f"matrix order {n} is outside the supported range 1..{_lib.MAX_N}")
-    return n
-
-
-def _upload(*tensors):
-    dev = _host.offload_device()
-    return [t.to(dev, non_blocking=True) for t in tensors]
+    return D.check_order(a.shape[-1])
 
 
 def _plain_host(*tensors) -> bool:
@@ -53,15 +45,15 @@ def batchdet(a: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
     -------
     d : (...) tensor
     """
-    if getattr(a, "requires_grad", False) and torch.is_grad_enabled():
+    if A.needs_grad(a) and torch.is_grad_enabled():
         return A.batchdet(a, out)
     return _batchdet(a, out=out)
 
 
 def _batchdet(a: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
     a = torch.as_tensor(a)
+    n = _square_order(a)
     if a.device.type != "cuda":
-        n = _square_order(a)
         nb = a.numel() // (n * n)
         D.check_out_shape(out, a.shape[:-2])
         if _plain_host(a) and nb > 0 and (out is None or _plain_host(a, out)):
@@ -71,25 +63,9 @@ def _batchdet(a: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
                            lambda fn, ws, wsb, chunk, nbuf, streams: fn(code, n, nb, a.data_ptr(), res.data_ptr(), ws, wsb,
                                                                          chunk, nbuf, streams))
             return res
-        r = batchdet(*_upload(a))
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r.cpu()
-    n = _square_order(a)
-    cdt = D.compute_dtype(a)
-    batch = tuple(a.shape[:-2])
-    nb = D.batch_count(batch)
-    o, res, copy_back = D.out_operand(out, batch, 0, cdt, a.device)
-    if nb > 0:
-        m = D.as_operand(a, batch, 2, cdt)
-        with D.device_of(a.device):
-            rc = _lib.load().nfm_batch_det(D.dtype_code(cdt), n, nb, m.ptr, m.stride, o.ptr, o.stride,
-                                           D.current_stream_ptr(a.device))
-        _lib.check(rc, "nfm_batch_det")
-    if copy_back:
-        res.copy_(o.tensor)
-    return res
+        return _host.uploaded(_batchdet, a, out=out)
+    return D.launch("nfm_batch_det", (n,), tuple(a.shape[:-2]), [(a, 2)], rec=(), out=out,
+                    dtype=D.compute_dtype(a), device=a.device)
 
 
 def batchinv(a: Tensor, *, method: str = 'auto', regularise: bool = True, out: Optional[Tensor] = None) -> Tensor:
@@ -112,7 +88,7 @@ def batchinv(a: Tensor, *, method: str = 'auto', regularise: bool = True, out: O
     Differentiable (``nfm_batch_inv_backward``); for orders 2 and 3 the determinant shift of
     ``regularise`` is treated as a constant.
     """
-    if getattr(a, "requires_grad", False) and torch.is_grad_enabled():
+    if A.needs_grad(a) and torch.is_grad_enabled():
         return A.batchinv(a, method, regularise, out)
     return _batchinv(a, method=method, regularise=regularise, out=out)
 
@@ -123,8 +99,8 @@ def _batchinv(a: Tensor, *, method: str = 'auto', regularise: bool = True, out: 
     algo = {'auto': _lib.ALGO_AUTO, 'lu': _lib.ALGO_LU, 'chol': _lib.ALGO_LDL, 'ldl': _lib.ALGO_LDL}.get(kind)
     if algo is None:
         raise ValueError(f"unknown method {method!r}")
+    n = _square_order(a)
     if a.device.type != "cuda":
-        n = _square_order(a)
         nb = a.numel() // (n * n)
         D.check_out_shape(out, a.shape)
         if _plain_host(a) and nb > 0 and (out is None or _plain_host(a, out)):
@@ -134,25 +110,9 @@ def _batchinv(a: Tensor, *, method: str = 'auto', regularise: bool = True, out: 
                            lambda fn, ws, wsb, chunk, nbuf, streams: fn(code, n, algo, int(bool(regularise)), nb, a.data_ptr(),
                                                                          res.data_ptr(), ws, wsb, chunk, nbuf, streams))
             return res
-        r = batchinv(*_upload(a), method=method, regularise=regularise)
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r.cpu()
-    n = _square_order(a)
-    cdt = D.compute_dtype(a)
-    batch = tuple(a.shape[:-2])
-    nb = D.batch_count(batch)
-    o, res, copy_back = D.out_operand(out, (*batch, n, n), 2, cdt, a.device)
-    if nb > 0:
-        m = D.as_operand(a, batch, 2, cdt)
-        with D.device_of(a.device):
-            rc = _lib.load().nfm_batch_inv(D.dtype_code(cdt), n, algo, int(bool(regularise)), nb, m.ptr, m.stride,
-                                           o.ptr, o.stride, D.current_stream_ptr(a.device))
-        _lib.check(rc, "nfm_batch_inv")
-    if copy_back:
-        res.copy_(o.tensor)
-    return res
+        return _host.uploaded(lambda m: _batchinv(m, method=method, regularise=regularise), a, out=out)
+    return D.launch("nfm_batch_inv", (n, algo, int(bool(regularise))), tuple(a.shape[:-2]), [(a, 2)], rec=(n, n),
+                    out=out, dtype=D.compute_dtype(a), device=a.device)
 
 
 def batchmatvec(mat: Tensor, vec: Tensor, *, out: Optional[Tensor] = None) -> Tensor:
@@ -169,7 +129,7 @@ def batchmatvec(mat: Tensor, vec: Tensor, *, out: Optional[Tensor] = None) -> Te
     -------
     matvec : (..., m) tensor
     """
-    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(mat, vec) and torch.is_grad_enabled():
         return A.batchmatvec(mat, vec, out)
     return _batchmatvec(mat, vec, out=out)
 
@@ -179,25 +139,10 @@ def _batchmatvec(mat: Tensor, vec: Tensor, *, out: Optional[Tensor] = None) -> T
     dev = D.common_device(mat, vec)
     if dev.type != "cuda":
         D.check_out_shape(out, (*torch.broadcast_shapes(mat.shape[:-2], vec.shape[:-1]), mat.shape[-2]))
-        r = batchmatvec(*_upload(mat, vec))
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r.cpu()
+        return _host.uploaded(_batchmatvec, mat, vec, out=out)
     m_, n = mat.shape[-2:]
     if vec.shape[-1] != n:
         raise ValueError(f"mat is (..., {m_}, {n}) but vec is (..., {vec.shape[-1]})")
     cdt = D.compute_dtype(mat, vec)
     batch = tuple(torch.broadcast_shapes(mat.shape[:-2], vec.shape[:-1]))
-    nb = D.batch_count(batch)
-    o, res, copy_back = D.out_operand(out, (*batch, m_), 1, cdt, dev)
-    if nb > 0:
-        a = D.as_operand(mat, batch, 2, cdt)
-        v = D.as_operand(vec, batch, 1, cdt)
-        with D.device_of(dev):
-            rc = _lib.load().nfm_batch_matvec(D.dtype_code(cdt), m_, n, nb, a.ptr, a.stride, v.ptr, v.stride,
-                                              o.ptr, o.stride, D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_batch_matvec")
-    if copy_back:
-        res.copy_(o.tensor)
-    return res
+    return D.launch("nfm_batch_matvec", (m_, n), batch, [(mat, 2), (vec, 1)], rec=(m_,), out=out, dtype=cdt, device=dev)

@@ -36,7 +36,7 @@ def lmdiv(a: Tensor, b: Tensor, method: str = 'lu', rcond: float = 1e-15, out: O
 
     a : `(..., n, n)`, b : `(..., n, k)` -> `(..., n, k)`.  Differentiable in both operands.
     """
-    if (getattr(a, "requires_grad", False) or getattr(b, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(a, b) and torch.is_grad_enabled():
         return A.lmdiv(a, b, method, out)
     return _lmdiv(a, b, method, out)
 
@@ -48,7 +48,7 @@ def _lmdiv(a: Tensor, b: Tensor, method: str = 'lu', out: Optional[Tensor] = Non
     algo = _algo(method)
     dev = D.common_device(a, b)
     if dev.type != "cuda":
-        cuda = _host.offload_device()
+        _host.offload_device()   # raises when there is no CUDA device: no CPU path
         n, k = a.shape[-1], b.shape[-1]
         if b.dim() >= 2 and b.shape[-2] == n:     # anything else is rejected by the device call
             D.check_out_shape(out, (*torch.broadcast_shapes(a.shape[:-2], b.shape[:-2]), n, k))
@@ -64,31 +64,15 @@ def _lmdiv(a: Tensor, b: Tensor, method: str = 'lu', out: Optional[Tensor] = Non
                            lambda fn, ws, wsb, chunk, nbuf, streams: fn(code, n, k, algo, nb, a.data_ptr(), b.data_ptr(),
                                                                          res.data_ptr(), ws, wsb, chunk, nbuf, streams))
             return res
-        r = lmdiv(a.to(cuda), b.to(cuda), method=method).cpu()
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r
-    n = a.shape[-1]
-    if not 1 <= n <= _lib.MAX_N:
-        raise ValueError(f"matrix order {n} is outside the supported range 1..{_lib.MAX_N}")
+        return _host.uploaded(lambda da, db: _lmdiv(da, db, method), a, b, out=out)
+    n = D.check_order(a.shape[-1])
     if b.shape[-2] != n:
         raise ValueError("a and b have incompatible shapes")
     k = b.shape[-1]
     cdt = D.compute_dtype(a, b)
     batch = tuple(torch.broadcast_shapes(a.shape[:-2], b.shape[:-2]))
-    nb = D.batch_count(batch)
-    o, res, copy_back = D.out_operand(out, (*batch, n, k), 2, cdt, dev)
-    if nb > 0 and k > 0:
-        ao = D.as_operand(a, batch, 2, cdt)
-        bo = D.as_operand(b, batch, 2, cdt)
-        with D.device_of(dev):
-            rc = _lib.load().nfm_batch_solve(D.dtype_code(cdt), n, k, algo, nb, ao.ptr, ao.stride, bo.ptr, bo.stride,
-                                             o.ptr, o.stride, D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_batch_solve")
-    if copy_back:
-        res.copy_(o.tensor)
-    return res
+    return D.launch("nfm_batch_solve", (n, k, algo), batch, [(a, 2), (b, 2)], rec=(n, k), out=out, dtype=cdt,
+                    device=dev, skip_empty=True)
 
 
 def rmdiv(a: Tensor, b: Tensor, method: str = 'lu', rcond: float = 1e-15, out: Optional[Tensor] = None) -> Tensor:
@@ -98,7 +82,7 @@ def rmdiv(a: Tensor, b: Tensor, method: str = 'lu', rcond: float = 1e-15, out: O
     a : `(..., k, n)`, b : `(..., n, n)` -> `(..., k, n)`.  Solved natively as ``b^T x_r = a_r`` for every
     row ``r`` (``nfm_batch_rsolve``): neither operand is transposed or copied.  Differentiable in both operands.
     """
-    if (getattr(a, "requires_grad", False) or getattr(b, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(a, b) and torch.is_grad_enabled():
         return A.rmdiv(a, b, method, out)
     return _rmdiv(a, b, method, out)
 
@@ -110,34 +94,18 @@ def _rmdiv(a: Tensor, b: Tensor, method: str = 'lu', out: Optional[Tensor] = Non
     algo = _algo(method)
     dev = D.common_device(a, b)
     if dev.type != "cuda":
-        cuda = _host.offload_device()
+        _host.offload_device()   # raises when there is no CUDA device: no CPU path
         if a.dim() >= 2 and a.shape[-1] == b.shape[-1]:     # anything else is rejected by the device call
             D.check_out_shape(out, (*torch.broadcast_shapes(a.shape[:-2], b.shape[:-2]), a.shape[-2], b.shape[-1]))
-        r = rmdiv(a.to(cuda), b.to(cuda), method=method).cpu()
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r
-    n = b.shape[-1]
-    if not 1 <= n <= _lib.MAX_N:
-        raise ValueError(f"matrix order {n} is outside the supported range 1..{_lib.MAX_N}")
+        return _host.uploaded(lambda da, db: _rmdiv(da, db, method), a, b, out=out)
+    n = D.check_order(b.shape[-1])
     if a.shape[-1] != n:
         raise ValueError("a and b have incompatible shapes")
     k = a.shape[-2]
     cdt = D.compute_dtype(a, b)
     batch = tuple(torch.broadcast_shapes(a.shape[:-2], b.shape[:-2]))
-    nb = D.batch_count(batch)
-    o, res, copy_back = D.out_operand(out, (*batch, k, n), 2, cdt, dev)
-    if nb > 0 and k > 0:
-        ao = D.as_operand(a, batch, 2, cdt)
-        bo = D.as_operand(b, batch, 2, cdt)
-        with D.device_of(dev):
-            rc = _lib.load().nfm_batch_rsolve(D.dtype_code(cdt), n, k, algo, nb, bo.ptr, bo.stride, ao.ptr, ao.stride,
-                                              o.ptr, o.stride, D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_batch_rsolve")
-    if copy_back:
-        res.copy_(o.tensor)
-    return res
+    return D.launch("nfm_batch_rsolve", (n, k, algo), batch, [(b, 2), (a, 2)], rec=(k, n), out=out, dtype=cdt,
+                    device=dev, skip_empty=True)
 
 
 def inv(a: Tensor, method: str = 'lu', rcond: float = 1e-15, out: Optional[Tensor] = None) -> Tensor:

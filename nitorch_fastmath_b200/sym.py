@@ -29,7 +29,6 @@ Signatures are the union of the reference's in-repo implementation
 """
 from __future__ import annotations
 
-import itertools
 import os
 from typing import Optional, Sequence, Union
 
@@ -64,17 +63,6 @@ def _algo(method: Optional[str]) -> int:
         raise ValueError(f"unknown method {method!r}; use one of 'auto', 'ldl', 'lu', 'warp'") from None
 
 
-def _check_n(n: int) -> None:
-    if not 1 <= n <= _lib.MAX_N:
-        raise ValueError(f"matrix order {n} is outside the supported range 1..{_lib.MAX_N}")
-
-
-def _to_device_inputs(*tensors):
-    """CPU operands are uploaded whole (general path for non-plain host tensors)."""
-    dev = _host.offload_device()
-    return [None if t is None else t.to(dev, non_blocking=True) for t in tensors], dev
-
-
 # ---------------------------------------------------------------------------
 # matvec family
 # ---------------------------------------------------------------------------
@@ -85,7 +73,7 @@ def _matvec(inp: Optional[Tensor], mat: Tensor, vec: Tensor, sign: int,
             and D.plain_cuda(vec, mat, inp, out) and (out is None or out.shape == vec.shape)):
         # fast path: dense CUDA fields with the same batch dims
         n = vec.shape[-1]
-        _check_n(n)
+        D.check_order(n)
         nn = mat.shape[-1]
         layout = D.detect_layout(nn, n)
         if inp is not None and inp.shape[-1] != n:
@@ -105,7 +93,7 @@ def _matvec(inp: Optional[Tensor], mat: Tensor, vec: Tensor, sign: int,
     dev = D.common_device(*tensors)
     cdt = D.compute_dtype(*tensors, dtype=dtype)
     n = vec.shape[-1]
-    _check_n(n)
+    D.check_order(n)
     layout = D.detect_layout(mat.shape[-1], n)
     shapes = [mat.shape[:-1], vec.shape[:-1]] + ([inp.shape[:-1]] if inp is not None else [])
     if inp is not None and inp.shape[-1] != n:
@@ -129,37 +117,14 @@ def _matvec(inp: Optional[Tensor], mat: Tensor, vec: Tensor, sign: int,
                     code, n, nb, mat.data_ptr(), vec.data_ptr(), inp.data_ptr() if inp is not None else None,
                     sign, res.data_ptr(), ws, wsb, chunk, nbuf, streams))
             return res
-        (dm, dv, di), cuda_dev = _to_device_inputs(mat, vec, inp)
-        r = _matvec(di, dm, dv, sign, dtype, None)
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r.cpu()
+        return _host.uploaded(lambda m, v, i: _matvec(i, m, v, sign, dtype, None), mat, vec, inp, out=out)
 
-    split = D.outer_split(batch, [(mat, 1), (vec, 1), (inp, 1)]) if nb > 0 else 0
-    if split:
-        # partially broadcast operands: one launch per index of the leading batch dims, on views
-        full = out if (out is not None and out.dtype == cdt and tuple(out.shape) == (*batch, n)) else \
-            torch.empty((*batch, n), dtype=cdt, device=dev)
-        for idx in itertools.product(*[range(k) for k in batch[:split]]):
-            _matvec(D.outer_views(inp, batch, 1, idx), D.outer_views(mat, batch, 1, idx),
-                    D.outer_views(vec, batch, 1, idx), sign, cdt, full[idx])
-        if out is not None and full is not out:
-            out.copy_(full)
-            return out
-        return full
-    o, res, copy_back = D.out_operand(out, (*batch, n), 1, cdt, dev, allow_estride=True)
-    if nb > 0:
-        m = D.as_operand(mat, batch, 1, cdt, allow_estride=True)
-        v = D.as_operand(vec, batch, 1, cdt, allow_estride=True)
-        i = D.as_operand(inp, batch, 1, cdt, allow_estride=True) if inp is not None else None
-        with D.device_of(dev):
-            rc = _lib.load().nfm_sym_matvec_ex(
-                code, n, layout, nb, m.c_struct(), v.c_struct(), i.c_struct() if i is not None else None, sign,
-                o.c_struct(), D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_sym_matvec")
-    if copy_back:
-        res.copy_(o.tensor)
+    res = D.outer_loop(batch, [(mat, 1), (vec, 1), (inp, 1)], out, (n,), cdt, dev,
+                       lambda m, v, i, o: _matvec(i, m, v, sign, cdt, o))
+    if res is not None:
+        return res
+    res = D.launch("nfm_sym_matvec", (n, layout), batch, [(mat, 1), (vec, 1), (inp, 1)], (sign,),
+                   rec=(n,), out=out, dtype=cdt, device=dev, struct=True)
     if out is None and dtype is None:
         want = tensors[0].dtype
         for t in tensors[1:]:
@@ -186,7 +151,7 @@ def sym_matvec(mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None, ou
     -------
     matvec : `(..., M) tensor`, dtype = promotion of the inputs
     """
-    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(mat, vec) and torch.is_grad_enabled():
         return A.matvec(None, mat, vec, 0, dtype, out)
     return _matvec(None, mat, vec, 0, dtype, out)
 
@@ -194,16 +159,14 @@ def sym_matvec(mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None, ou
 def sym_addmatvec(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None,
                   out: Optional[Tensor] = None) -> Tensor:
     """``inp + mat @ vec``  (reference name: sym.py:31)."""
-    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
-            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(inp, mat, vec) and torch.is_grad_enabled():
         return A.matvec(inp, mat, vec, +1, dtype, out)
     return _matvec(torch.as_tensor(inp), mat, vec, +1, dtype, out)
 
 
 def sym_addmatvec_(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None) -> Tensor:
     """In-place ``inp += mat @ vec``; returns ``inp``  (sym.py:31)."""
-    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
-            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(inp, mat, vec) and torch.is_grad_enabled():
         return A.matvec(inp, mat, vec, +1, inp.dtype if dtype is None else dtype, None, inplace=True)
     return _matvec(inp, mat, vec, +1, inp.dtype if dtype is None else dtype, inp)
 
@@ -211,16 +174,14 @@ def sym_addmatvec_(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.
 def sym_submatvec(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None,
                   out: Optional[Tensor] = None) -> Tensor:
     """``inp - mat @ vec``  (sym.py:32)."""
-    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
-            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(inp, mat, vec) and torch.is_grad_enabled():
         return A.matvec(inp, mat, vec, -1, dtype, out)
     return _matvec(torch.as_tensor(inp), mat, vec, -1, dtype, out)
 
 
 def sym_submatvec_(inp: Tensor, mat: Tensor, vec: Tensor, dtype: Optional[torch.dtype] = None) -> Tensor:
     """In-place ``inp -= mat @ vec``; returns ``inp``  (sym.py:32)."""
-    if (getattr(inp, "requires_grad", False) or getattr(mat, "requires_grad", False)
-            or getattr(vec, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(inp, mat, vec) and torch.is_grad_enabled():
         return A.matvec(inp, mat, vec, -1, inp.dtype if dtype is None else dtype, None, inplace=True)
     return _matvec(inp, mat, vec, -1, inp.dtype if dtype is None else dtype, inp)
 
@@ -290,8 +251,7 @@ def sym_solve(mat: Tensor, vec: Tensor,
     -------
     result : `(..., M) tensor` with ``vec``'s dtype (as the reference).
     """
-    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
-            or getattr(diag, "requires_grad", False) or getattr(eps, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(mat, vec, diag, eps) and torch.is_grad_enabled():
         return A.solve(mat, vec, diag, dtype, out, eps, method)
     return _solve(mat, vec, diag, dtype, out, eps=eps, method=method)
 
@@ -306,7 +266,7 @@ def _solve(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = N
             and D.plain_cuda(vec, mat, out) and (out is None or out.shape == vec.shape)):
         # fast path: dense CUDA fields with the same batch dims
         n = vec.shape[-1]
-        _check_n(n)
+        D.check_order(n)
         nn = mat.shape[-1]
         layout = D.detect_layout(nn, n)
         dev = vec.device
@@ -327,7 +287,7 @@ def _solve(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = N
     cdt = D.compute_dtype(mat, vec, dtype=dtype)
     res_dtype = dtype if dtype is not None else vec.dtype   # reference: result has vec's dtype (half types compute in fp32)
     n = vec.shape[-1]
-    _check_n(n)
+    D.check_order(n)
     layout = D.detect_layout(mat.shape[-1], n)
     reg = _as_diag(diag, n, cdt, dev)
     shapes = [mat.shape[:-1], vec.shape[:-1]] + ([reg.shape[:-1]] if reg is not None else [])
@@ -354,39 +314,14 @@ def _solve(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = N
                     code, n, algo, nb, mat.data_ptr(), vec.data_ptr(), reg.data_ptr() if reg is not None else None,
                     res.data_ptr(), ws, wsb, chunk, nbuf, streams))
             return res
-        (dm, dv), cuda_dev = _to_device_inputs(mat, vec)
-        r = _solve(dm, dv, None if reg is None else reg.to(cuda_dev), dtype=dtype, method=method)
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r.cpu()
+        return _host.uploaded(lambda m, v, r: _solve(m, v, r, dtype=dtype, method=method), mat, vec, reg, out=out)
 
-    split = D.outer_split(batch, [(mat, 1), (vec, 1), (reg, 1)]) if nb > 0 else 0
-    if split:
-        # partially broadcast operands: one launch per index of the leading batch dims, on views
-        # (nothing is materialised; each launch sees dense / fully broadcast operands)
-        full = out if (out is not None and out.dtype == cdt and tuple(out.shape) == (*batch, n)) else \
-            torch.empty((*batch, n), dtype=cdt, device=dev)
-        for idx in itertools.product(*[range(k) for k in batch[:split]]):
-            _solve(D.outer_views(mat, batch, 1, idx), D.outer_views(vec, batch, 1, idx),
-                   D.outer_views(reg, batch, 1, idx), dtype=cdt, out=full[idx], method=method)
-        if out is not None and full is not out:
-            out.copy_(full)
-            return out
-        return full if (out is not None or full.dtype == res_dtype) else full.to(res_dtype)
-    o, res, copy_back = D.out_operand(out if (out is None or out.dtype == cdt) else None, (*batch, n), 1, cdt, dev,
-                                      allow_estride=True)
-    if nb > 0:
-        m = D.as_operand(mat, batch, 1, cdt, allow_estride=True)
-        v = D.as_operand(vec, batch, 1, cdt, allow_estride=True)
-        r = D.as_operand(reg, batch, 1, cdt, allow_estride=True) if reg is not None else None
-        with D.device_of(dev):
-            rc = _lib.load().nfm_sym_solve_ex(
-                code, n, layout, algo, nb, m.c_struct(), v.c_struct(), r.c_struct() if r is not None else None,
-                o.c_struct(), D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_sym_solve")
-    if copy_back:
-        res.copy_(o.tensor)
+    res = D.outer_loop(batch, [(mat, 1), (vec, 1), (reg, 1)], out, (n,), cdt, dev,
+                       lambda m, v, r, o: _solve(m, v, r, dtype=cdt, out=o, method=method))
+    if res is not None:
+        return res if (out is not None or res.dtype == res_dtype) else res.to(res_dtype)
+    res = D.launch("nfm_sym_solve", (n, layout, algo), batch, [(mat, 1), (vec, 1), (reg, 1)],
+                   rec=(n,), out=out if (out is None or out.dtype == cdt) else None, dtype=cdt, device=dev, struct=True)
     if out is not None and out.dtype != cdt:
         out.copy_(res)
         return out
@@ -398,8 +333,7 @@ def _solve(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = N
 def sym_solve_(mat: Tensor, vec: Tensor, diag=None, dtype: Optional[torch.dtype] = None, *,
                eps=None, method: Optional[str] = None) -> Tensor:
     r"""In-place ``vec <- mat \ vec``; returns ``vec``  (reference name sym.py:33)."""
-    if (getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
-            or getattr(diag, "requires_grad", False) or getattr(eps, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(mat, vec, diag, eps) and torch.is_grad_enabled():
         return A.solve(mat, vec, diag, dtype, None, eps, method, inplace=True)
     return _solve(mat, vec, diag, dtype=dtype, out=vec, eps=eps, method=method)
 
@@ -420,8 +354,7 @@ def sym_solve_update(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alph
     reference's per-voxel regulariser ``(..., M)`` (or anything broadcastable to it).
     Differentiable with respect to ``x``, ``mat``, ``vec`` and a tensor ``diag``.
     """
-    if (getattr(x, "requires_grad", False) or getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
-            or getattr(diag, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(x, mat, vec, diag) and torch.is_grad_enabled():
         return A.solve_update(x, mat, vec, lam, alpha, out, diag, method)
     return _solve_update(x, mat, vec, lam, alpha, out, diag=diag, method=method)
 
@@ -434,7 +367,7 @@ def _solve_update(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alpha: 
     if dev.type != "cuda":
         raise RuntimeError("sym_solve_update takes CUDA tensors")
     n = vec.shape[-1]
-    _check_n(n)
+    D.check_order(n)
     if mat.shape[-1] != n * (n + 1) // 2 or x.shape[-1] != n:
         raise ValueError("sym_solve_update takes a packed symmetric mat and x, vec of the same trailing size")
     cdt = D.compute_dtype(x, mat, vec)
@@ -444,31 +377,32 @@ def _solve_update(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alpha: 
     reg = _as_diag(diag, n, cdt, dev)
     shapes = [x.shape[:-1], mat.shape[:-1], vec.shape[:-1]] + ([reg.shape[:-1]] if reg is not None else [])
     batch = tuple(torch.broadcast_shapes(*shapes))
-    nb = D.batch_count(batch)
-    o, res, copy_back = D.out_operand(out, (*batch, n), 1, cdt, dev)
-    if nb > 0:
-        m = D.as_operand(mat, batch, 1, cdt)
-        v = D.as_operand(vec, batch, 1, cdt)
-        xo = D.as_operand(x, batch, 1, cdt)
-        r = D.as_operand(reg, batch, 1, cdt) if reg is not None else None
-        with D.device_of(dev):
-            rc = _lib.load().nfm_sym_solve_update_reg(
-                D.dtype_code(cdt), n, algo, nb, m.ptr, m.stride, v.ptr, v.stride, xo.ptr, xo.stride,
-                None if r is None else r.ptr, 0 if r is None else r.stride, float(lam), float(alpha), o.ptr, o.stride,
-                D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_sym_solve_update")
-    if copy_back:
-        res.copy_(o.tensor)
-    return res
+    return D.launch("nfm_sym_solve_update_reg", (n, algo), batch, [(mat, 1), (vec, 1), (x, 1), (reg, 1)],
+                    (float(lam), float(alpha)), rec=(n,), out=out, dtype=cdt, device=dev, what="nfm_sym_solve_update")
 
 
 def sym_solve_update_(x: Tensor, mat: Tensor, vec: Tensor, lam: float = 0.0, alpha: float = 1.0, *,
                       diag: Optional[Tensor] = None, method: Optional[str] = None) -> Tensor:
     r"""In-place ``x -= alpha * (mat + lam*I + diag(d)) \ vec``; returns ``x``."""
-    if (getattr(x, "requires_grad", False) or getattr(mat, "requires_grad", False) or getattr(vec, "requires_grad", False)
-            or getattr(diag, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(x, mat, vec, diag) and torch.is_grad_enabled():
         return A.solve_update(x, mat, vec, lam, alpha, None, diag, method, inplace=True)
     return _solve_update(x, mat, vec, lam, alpha, out=x, diag=diag, method=method)
+
+
+def _mode(k: int, d: int) -> int:
+    """C ABI ``mode`` of the J/H products: 1 (J H J^T) for k == d <= 3, the reference's unrolled
+    branches (_impl/sym.py:532-593); 0 (J^T H J) otherwise."""
+    return 1 if (k == d and k <= 3) else 0
+
+
+def _packed_h(j: Tensor, h: Tensor) -> Tensor:
+    """A diagonal Hessian (k values; reference jhjn accepts it: _impl/sym.py:603-606) in packed form with
+    zero off-diagonals.  The autograd wrappers pad it before their Function, so that its gradient is
+    the diagonal of the packed one (the backward of torch.cat)."""
+    k = j.shape[-2]
+    if h.shape[-1] == k and k > 1:
+        return torch.cat([h, h.new_zeros((*h.shape[:-1], k * (k - 1) // 2))], -1)
+    return h
 
 
 def sym_matmul_solve(j: Tensor, h: Tensor, g: Tensor, diag=None, out: Optional[Tensor] = None) -> Tensor:
@@ -482,8 +416,7 @@ def sym_matmul_solve(j: Tensor, h: Tensor, g: Tensor, diag=None, out: Optional[T
     for ``k == d <= 3`` (the reference's unrolled branches).  Not a function of the reference.
     Differentiable with respect to ``j``, ``h``, ``g`` and a tensor ``diag``.
     """
-    if (getattr(j, "requires_grad", False) or getattr(h, "requires_grad", False) or getattr(g, "requires_grad", False)
-            or getattr(diag, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(j, h, g, diag) and torch.is_grad_enabled():
         return A.matmul_solve(j, h, g, diag, out)
     return _matmul_solve(j, h, g, diag, out)
 
@@ -496,32 +429,17 @@ def _matmul_solve(j: Tensor, h: Tensor, g: Tensor, diag=None, out: Optional[Tens
     k, d = j.shape[-2:]
     if not ((1 <= k <= 6 and 1 <= d <= 6) or (1 <= k <= _lib.MAX_N and 1 <= d <= 3)):
         raise ValueError("sym_matmul_solve supports 1 <= k, d <= 6, or k <= 10 with d <= 3 (use sym_matmul + sym_solve otherwise)")
-    if h.shape[-1] == k and k > 1:
-        h = torch.cat([h, h.new_zeros((*h.shape[:-1], k * (k - 1) // 2))], -1)
+    h = _packed_h(j, h)
     if h.shape[-1] != k * (k + 1) // 2:
         raise ValueError("h must be compact symmetric (k*(k+1)//2 coefficients) or diagonal (k coefficients)")
-    mode = 1 if (k == d and k <= 3) else 0
     if g.shape[-1] != d:
         raise ValueError(f"g must have {d} trailing values")
     cdt = D.compute_dtype(j, h, g)
     reg = _as_diag(diag, d, cdt, dev)
     shapes = [j.shape[:-2], h.shape[:-1], g.shape[:-1]] + ([reg.shape[:-1]] if reg is not None else [])
     batch = tuple(torch.broadcast_shapes(*shapes))
-    nb = D.batch_count(batch)
-    o, res, copy_back = D.out_operand(out, (*batch, d), 1, cdt, dev)
-    if nb > 0:
-        jo = D.as_operand(j, batch, 2, cdt)
-        ho = D.as_operand(h, batch, 1, cdt)
-        go = D.as_operand(g, batch, 1, cdt)
-        r = D.as_operand(reg, batch, 1, cdt) if reg is not None else None
-        with D.device_of(dev):
-            rc = _lib.load().nfm_sym_matmul_solve(
-                D.dtype_code(cdt), k, d, mode, nb, jo.ptr, jo.stride, ho.ptr, ho.stride, go.ptr, go.stride,
-                None if r is None else r.ptr, 0 if r is None else r.stride, o.ptr, o.stride, D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_sym_matmul_solve")
-    if copy_back:
-        res.copy_(o.tensor)
-    return res
+    return D.launch("nfm_sym_matmul_solve", (k, d, _mode(k, d)), batch, [(j, 2), (h, 1), (g, 1), (reg, 1)],
+                    rec=(d,), out=out, dtype=cdt, device=dev)
 
 
 # ---------------------------------------------------------------------------
@@ -544,7 +462,7 @@ def sym_invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = N
     -------
     imat : `(..., M or M*(M+1)//2) tensor` (compact storage, same ordering)
     """
-    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+    if A.needs_grad(mat) and torch.is_grad_enabled():
         return A.invert(mat, diag, dtype, out, method)
     return _invert(mat, diag, dtype, out, method=method)
 
@@ -557,7 +475,7 @@ def _invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = None
             out is None or (D.plain_cuda(mat, out) and out.shape[-1] == (D.packed_order(mat.shape[-1]) if diag else mat.shape[-1]))):
         nn = mat.shape[-1]
         n = D.packed_order(nn)
-        _check_n(n)
+        D.check_order(n)
         no = n if diag else nn
         res = out if out is not None else (D.empty_like_phased(mat) if no == nn else
                                            torch.empty((*mat.shape[:-1], no), dtype=mat.dtype, device=mat.device))
@@ -573,7 +491,7 @@ def _invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = None
     cdt = D.compute_dtype(mat, dtype=dtype)
     nn = mat.shape[-1]
     n = D.packed_order(nn)
-    _check_n(n)
+    D.check_order(n)
     no = n if diag else nn
     batch = tuple(mat.shape[:-1])
     nb = D.batch_count(batch)
@@ -592,22 +510,10 @@ def _invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = None
                 lambda fn, ws, wsb, chunk, nbuf, streams: fn(
                     code, n, algo, int(bool(diag)), nb, mat.data_ptr(), res.data_ptr(), ws, wsb, chunk, nbuf, streams))
             return res
-        (dm,), _ = _to_device_inputs(mat)
-        r = _invert(dm, diag, dtype=dtype, method=method)
-        if out is not None:
-            out.copy_(r)
-            return out
-        return r.cpu()
+        return _host.uploaded(lambda m: _invert(m, diag, dtype=dtype, method=method), mat, out=out)
 
-    o, res, copy_back = D.out_operand(out, (*batch, no), 1, cdt, dev, allow_estride=True)
-    if nb > 0:
-        m = D.as_operand(mat, batch, 1, cdt, allow_estride=True)
-        with D.device_of(dev):
-            rc = _lib.load().nfm_sym_invert_ex(code, n, algo, int(bool(diag)), nb, m.c_struct(), o.c_struct(),
-                                               D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_sym_invert")
-    if copy_back:
-        res.copy_(o.tensor)
+    res = D.launch("nfm_sym_invert", (n, algo, int(bool(diag))), batch, [(mat, 1)], rec=(no,), out=out,
+                   dtype=cdt, device=dev, struct=True)
     if out is None and dtype is None and mat.dtype != res.dtype and mat.dtype.is_floating_point:
         res = res.to(mat.dtype)
     return res
@@ -615,7 +521,7 @@ def _invert(mat: Tensor, diag: bool = False, dtype: Optional[torch.dtype] = None
 
 def sym_invert_(mat: Tensor, dtype: Optional[torch.dtype] = None, *, method: Optional[str] = None) -> Tensor:
     """In-place inversion; returns ``mat``  (reference name sym.py:34)."""
-    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+    if A.needs_grad(mat) and torch.is_grad_enabled():
         return A.invert(mat, False, dtype, None, method, inplace=True)
     return _invert(mat, False, dtype=dtype, out=mat, method=method)
 
@@ -624,37 +530,20 @@ def sym_invert_(mat: Tensor, dtype: Optional[torch.dtype] = None, *, method: Opt
 # remaining public names of nitorch_fastmath/sym.py:29
 # ---------------------------------------------------------------------------
 
-def _unary(fn_name: str, x: Tensor, n: int, out_shape, rec_ndim_out: int) -> Tensor:
-    dev = x.device
-    if dev.type != "cuda":
-        _host.offload_device()   # raises when there is no CUDA device: no CPU path
-        (dx,), _ = _to_device_inputs(x)
-        return _unary(fn_name, dx, n, out_shape, rec_ndim_out).cpu()
-    cdt = D.compute_dtype(x)
-    batch = tuple(x.shape[:-1])
-    nb = D.batch_count(batch)
-    o, res, _ = D.out_operand(None, tuple(out_shape), rec_ndim_out, cdt, dev)
-    if nb > 0:
-        m = D.as_operand(x, batch, 1, cdt)
-        with D.device_of(dev):
-            rc = getattr(_lib.load(), fn_name)(D.dtype_code(cdt), n, nb, m.ptr, m.stride, o.ptr, o.stride,
-                                               D.current_stream_ptr(dev))
-        _lib.check(rc, fn_name)
-    return res
-
-
 def sym_to_full(mat: Tensor) -> Tensor:
     """Compact symmetric -> full `(..., M, M)`  (reference _impl/sym.py:16-60)."""
-    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+    if A.needs_grad(mat) and torch.is_grad_enabled():
         return A.to_full(mat)
     return _to_full(mat)
 
 
 def _to_full(mat: Tensor) -> Tensor:
     mat = torch.as_tensor(mat)
-    n = D.packed_order(mat.shape[-1])
-    _check_n(n)
-    return _unary("nfm_sym_to_full", mat, n, (*mat.shape[:-1], n, n), 2)
+    n = D.check_order(D.packed_order(mat.shape[-1]))
+    if mat.device.type != "cuda":
+        return _host.uploaded(_to_full, mat)
+    return D.launch("nfm_sym_to_full", (n,), tuple(mat.shape[:-1]), [(mat, 1)], rec=(n, n),
+                    dtype=D.compute_dtype(mat), device=mat.device)
 
 
 def sym_diag(mat: Tensor) -> Tensor:
@@ -665,31 +554,35 @@ def sym_diag(mat: Tensor) -> Tensor:
 
 def sym_outer(x: Tensor) -> Tensor:
     """Symmetric outer product ``x x^T`` in compact storage (reference _impl/sym.py:496-528)."""
-    if getattr(x, "requires_grad", False) and torch.is_grad_enabled():
+    if A.needs_grad(x) and torch.is_grad_enabled():
         return A.outer(x)
     return _outer(x)
 
 
 def _outer(x: Tensor) -> Tensor:
     x = torch.as_tensor(x)
-    n = x.shape[-1]
-    _check_n(n)
-    return _unary("nfm_sym_outer", x, n, (*x.shape[:-1], n * (n + 1) // 2), 1)
+    n = D.check_order(x.shape[-1])
+    if x.device.type != "cuda":
+        return _host.uploaded(_outer, x)
+    return D.launch("nfm_sym_outer", (n,), tuple(x.shape[:-1]), [(x, 1)], rec=(n * (n + 1) // 2,),
+                    dtype=D.compute_dtype(x), device=x.device)
 
 
 def sym_det(mat: Tensor) -> Tensor:
     """Determinant of a compact symmetric matrix `(...)`  (reference _impl/sym.py:401-452;
     the reference's batched N >= 3 result is wrong (:434), this one is not)."""
-    if getattr(mat, "requires_grad", False) and torch.is_grad_enabled():
+    if A.needs_grad(mat) and torch.is_grad_enabled():
         return A.det(mat)
     return _det(mat)
 
 
 def _det(mat: Tensor) -> Tensor:
     mat = torch.as_tensor(mat)
-    n = D.packed_order(mat.shape[-1])
-    _check_n(n)
-    return _unary("nfm_sym_det", mat, n, tuple(mat.shape[:-1]), 0)
+    n = D.check_order(D.packed_order(mat.shape[-1]))
+    if mat.device.type != "cuda":
+        return _host.uploaded(_det, mat)
+    return D.launch("nfm_sym_det", (n,), tuple(mat.shape[:-1]), [(mat, 1)], rec=(),
+                    dtype=D.compute_dtype(mat), device=mat.device)
 
 
 def sym_matmul(j: Tensor, h: Tensor) -> Tensor:
@@ -701,7 +594,7 @@ def sym_matmul(j: Tensor, h: Tensor) -> Tensor:
     :math:`J H J^T`; this drop-in reproduces that (C ABI ``mode=1``).
     Differentiable with respect to ``j`` and ``h`` (also a diagonal ``h``).
     """
-    if (getattr(j, "requires_grad", False) or getattr(h, "requires_grad", False)) and torch.is_grad_enabled():
+    if A.needs_grad(j, h) and torch.is_grad_enabled():
         return A.matmul(j, h)
     return _matmul(j, h)
 
@@ -710,28 +603,14 @@ def _matmul(j: Tensor, h: Tensor) -> Tensor:
     j, h = torch.as_tensor(j), torch.as_tensor(h)
     dev = D.common_device(j, h)
     if dev.type != "cuda":
-        _host.offload_device()   # raises when there is no CUDA device: no CPU path
-        (dj, dh), _ = _to_device_inputs(j, h)
-        return _matmul(dj, dh).cpu()
+        return _host.uploaded(_matmul, j, h)
     k, d = j.shape[-2:]
     if not (1 <= k <= _lib.MAX_N and 1 <= d <= _lib.MAX_N):
         raise ValueError(f"sym_matmul supports 1 <= k, d <= {_lib.MAX_N}")
-    if h.shape[-1] == k and k > 1:
-        # diagonal Hessian (reference jhjn accepts it: _impl/sym.py:603-606): packed form with zero off-diagonals
-        h = torch.cat([h, h.new_zeros((*h.shape[:-1], k * (k - 1) // 2))], -1)
+    h = _packed_h(j, h)
     if h.shape[-1] != k * (k + 1) // 2:
         raise ValueError("h must be compact symmetric (k*(k+1)//2 coefficients) or diagonal (k coefficients)")
     cdt = h.dtype if h.dtype in (torch.float32, torch.float64) else D.compute_dtype(j, h)
-    mode = 1 if (k == d and k <= 3) else 0
     batch = tuple(torch.broadcast_shapes(j.shape[:-2], h.shape[:-1]))
-    nb = D.batch_count(batch)
-    do = d * (d + 1) // 2
-    o, res, _ = D.out_operand(None, (*batch, do), 1, cdt, dev)
-    if nb > 0:
-        jo = D.as_operand(j, batch, 2, cdt)
-        ho = D.as_operand(h, batch, 1, cdt)
-        with D.device_of(dev):
-            rc = _lib.load().nfm_sym_matmul(D.dtype_code(cdt), k, d, mode, nb, jo.ptr, jo.stride, ho.ptr, ho.stride,
-                                            o.ptr, o.stride, D.current_stream_ptr(dev))
-        _lib.check(rc, "nfm_sym_matmul")
-    return res
+    return D.launch("nfm_sym_matmul", (k, d, _mode(k, d)), batch, [(j, 2), (h, 1)], rec=(d * (d + 1) // 2,),
+                    dtype=cdt, device=dev)
