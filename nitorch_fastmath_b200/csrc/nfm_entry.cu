@@ -391,6 +391,8 @@ int nfm_batch_matvec(int dtype, int m, int n, int64_t batch, const void* mat, in
   }
   if (mat == nullptr || vec == nullptr || out == nullptr) return fail(NFM_E_BADARG, "NULL operand");
   if (mat_stride < 0 || vec_stride < 0 || out_stride < 0) return fail(NFM_E_BADARG, "negative batch stride");
+  t_last_path_tma = 0;
+  reset_launch_record();
   int rc = dtype == NFM_F32 ? batch_matvec_rt<float>(m, n, 0, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s)
                             : batch_matvec_rt<double>(m, n, 0, batch, mat, mat_stride, vec, vec_stride, out, out_stride, s);
   if (rc) set_error("matvec kernel launch failed: %s", cudaGetErrorString(cudaError_t(rc)));

@@ -104,6 +104,8 @@ int nfm_sym_matmul(int dtype, int k, int d, int mode, int64_t batch, const void*
   if (batch < 0 || !jac || !hess || !out || jac_stride < 0 || hess_stride < 0 || out_stride < 0) { set_error("bad argument"); return NFM_E_BADARG; }
   auto st = static_cast<cudaStream_t>(stream);
   if (!fused_shape_built(k, d) || (mode == 1 && k > 3)) {  // run-time-sized kernel beyond the templated shapes
+    t_last_path_tma = 0;
+    reset_launch_record();
     const int rc = dtype == NFM_F32 ? sym_matmul_rt<float>(k, d, mode, batch, jac, jac_stride, hess, hess_stride, out, out_stride, st)
                                     : sym_matmul_rt<double>(k, d, mode, batch, jac, jac_stride, hess, hess_stride, out, out_stride, st);
     if (rc) set_error("sym_matmul kernel launch failed: %s", cudaGetErrorString(cudaError_t(rc)));

@@ -395,6 +395,10 @@ __global__ void __launch_bounds__(THREADS)
       else zero_record(r2[j]);
     }
 
+    // the barrier below hands the stage to the async proxy (its TMA refill): order this thread's
+    // generic-proxy loads from it before that write, or a load still in flight can return the
+    // next tile's bytes (DESIGN.md section 4)
+    fence_proxy_async();
     // the output buffer we are about to overwrite was last read by the bulk
     // store issued two tiles ago: allow one store (group) still pending
     if (tid < kIssuers) bulk_wait_read<1>();

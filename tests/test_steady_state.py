@@ -200,6 +200,30 @@ def _det_backward(mat, grad, n):
     return out * grad.double()[..., None]
 
 
+def _ghat(g, n):
+    """The full symmetric form of a packed gradient with the off-diagonals halved."""
+    f = _unpack(g.double(), n)
+    return (f + torch.diag_embed(f.diagonal(0, -1, -2))) / 2
+
+
+def _pack2(m):
+    """M_ii, 2 M_ij (i < j) of a symmetric M."""
+    return _pack(2 * m - torch.diag_embed(m.diagonal(0, -1, -2)))
+
+
+def _matmul_backward(i, k, d, which):
+    """dJ (flattened) and / or dH of J^T H J (J H J^T for k = d <= 3), one record [dJ | dH]."""
+    j = i["j"].double()
+    mode1 = k == d and k <= 3
+    h, gh = _unpack(i["h"].double(), d if mode1 else k), _ghat(i["g"], k if mode1 else d)
+    parts = []
+    if which & 1:
+        parts.append((2 * gh @ j @ h if mode1 else 2 * h @ j @ gh).flatten(-2))
+    if which & 2:
+        parts.append(_pack2(j.transpose(-1, -2) @ gh @ j if mode1 else j @ gh @ j.transpose(-1, -2)))
+    return torch.cat(parts, -1)
+
+
 # --------------------------------------------------------------------------
 # the case table
 # --------------------------------------------------------------------------
@@ -406,13 +430,107 @@ def _dense_cases():
     return cases
 
 
+MATMUL_SHAPES = ((1, 1), (2, 2), (3, 3), (4, 4), (6, 6), (3, 2), (2, 3), (10, 3))
+
+
+def _grad_cases():
+    """The backward kernels of the dense routines and of the Gauss-Newton builders (_autograd.py)."""
+    from nitorch_fastmath_b200 import _autograd as A
+    from nitorch_fastmath_b200 import _lib
+    cases = []
+    for dt in DTYPES:
+        t = "f32" if dt == torch.float32 else "f64"
+        es = torch.finfo(dt).bits // 8
+        for n in range(1, 11):
+            nn = n * (n + 1) // 2
+            for sym in (False, True):
+                def g_inv(b, s, n=n, dt=dt, sym=sym):
+                    return dict(y=dense_spd(b, n, dt, s) if sym else dense(b, n, dt, s), g=vecs(b, n, dt, s + 1, k=n))
+
+                def r_inv(i, sym=sym):
+                    y, g = i["y"].double(), i["g"].double()
+                    if sym:
+                        return -y @ ((g + g.transpose(-1, -2)) / 2) @ y
+                    return -y.transpose(-1, -2) @ g @ y.transpose(-1, -2)
+
+                # fp64 n = 9, 10: the ring of the smallest tile does not fit shared memory (DESIGN section 6 item 8)
+                cases.append(Case(f"dense_inv_backward_{'sym_' if sym else ''}{t}_n{n}", dt, g_inv,
+                                  lambda i, sym=sym: A.dense_inv_backward(i["y"], i["g"], sym), r_inv, rec=2, scale=10,
+                                  extra=dict(strided=dt == torch.float64 and n >= 9)))
+            # orders <= 3 closed-form cofactors on the tile kernel; from 4 pivoted, on the warp pool from 256 B of input
+            cases.append(Case(f"dense_det_backward_{t}_n{n}", dt,
+                              lambda b, s, n=n, dt=dt: dict(a=dense(b, n, dt, s), g=vecs(b, 1, dt, s + 1)[:, 0].contiguous()),
+                              lambda i: A.dense_det_backward(i["a"], i["g"]),
+                              lambda i: i["g"].double()[..., None, None] * torch.linalg.det(i["a"].double())[..., None, None]
+                              * torch.linalg.inv(i["a"].double()).transpose(-1, -2), rec=2, scale=10,
+                              extra=dict(path=3 if n >= 4 and (n * n + 1) * es >= 256 else 1)))
+            for kk, rows, sym, sign in ((1, False, False, 1), (2, True, True, -1), (3, False, True, -1), (4, True, False, -1)):
+                def g_out(b, s, n=n, dt=dt, kk=kk, rows=rows):
+                    return dict(u=vecs(b, kk if rows else n, dt, s, k=n if rows else kk),
+                                w=vecs(b, kk if rows else n, dt, s + 1, k=n if rows else kk))
+
+                def r_out(i, rows=rows, sym=sym, sign=sign):
+                    u, w = i["u"].double(), i["w"].double()
+                    m = u.transpose(-1, -2) @ w if rows else u @ w.transpose(-1, -2)
+                    return sign * ((m + m.transpose(-1, -2)) / 2 if sym else m)
+
+                cases.append(Case(f"dense_outer_k{kk}_{'rows' if rows else 'left'}_{'sym' if sym else 'plain'}_"
+                                  f"{'p' if sign > 0 else 'm'}_{t}_n{n}", dt, g_out,
+                                  lambda i, rows=rows, sym=sym, sign=sign: A.dense_outer(i["u"], i["w"], rows, sym, sign),
+                                  r_out, rec=2, scale=10, extra=dict(mag=True)))
+            # A^-T B: one right-hand side (the one-row right division, many-right-hand-sides kernel), 2-4 (register
+            # kernels with the transposed flag), more than 4 (the many-right-hand-sides kernel, transposed)
+            for name, kk, right, algo in (("lu_k1", 1, False, _lib.ALGO_LU), ("lu_k3", 3, False, _lib.ALGO_LU),
+                                          ("chol_k2", 2, False, _lib.ALGO_LDL), ("lu_right_k2", 2, True, _lib.ALGO_LU),
+                                          ("lu_k5", 5, False, _lib.ALGO_LU)):
+                def g_ts(b, s, n=n, dt=dt, kk=kk, right=right, algo=algo):
+                    a = dense_spd(b, n, dt, s) if algo == _lib.ALGO_LDL else dense(b, n, dt, s)
+                    return dict(a=a, b=vecs(b, kk, dt, s + 1, k=n) if right else vecs(b, n, dt, s + 1, k=kk))
+
+                def r_ts(i, right=right):
+                    a = i["a"].double()
+                    if right:   # B A^-T = (A^-1 B^T)^T
+                        return torch.linalg.solve(a, i["b"].double().transpose(-1, -2)).transpose(-1, -2)
+                    return torch.linalg.solve(a.transpose(-1, -2), i["b"].double())
+
+                cases.append(Case(f"tsolve_{name}_{t}_n{n}", dt, g_ts,
+                                  lambda i, right=right, algo=algo: A.dense_tsolve(i["a"], i["b"], right, algo), r_ts,
+                                  rec=2, scale=10, extra=dict(many=kk == 1 or kk > 4)))
+            cases.append(Case(f"tmatvec_{t}_n{n}", dt, lambda b, s, n=n, dt=dt: dict(a=dense(b, n, dt, s), v=vecs(b, n, dt, s + 1)),
+                              lambda i: A.dense_tmatvec(i["a"], i["v"]),
+                              lambda i: (i["a"].double().transpose(-1, -2) @ i["v"].double()[..., None])[..., 0], scale=10))
+            cases.append(Case(f"outer_backward_{t}_n{n}", dt,
+                              lambda b, s, n=n, nn=nn, dt=dt: dict(x=vecs(b, n, dt, s), g=vecs(b, nn, dt, s + 1)),
+                              lambda i: A.outer_backward(i["x"], i["g"]),
+                              lambda i, n=n: 2 * (_ghat(i["g"], n) @ i["x"].double()[..., None])[..., 0], scale=10))
+            cases.append(Case(f"to_full_backward_{t}_n{n}", dt, lambda b, s, n=n, dt=dt: dict(g=vecs(b, n, dt, s, k=n)),
+                              lambda i: A.to_full_backward(i["g"]),
+                              lambda i: _pack2(i["g"].double() + i["g"].double().transpose(-1, -2)) / 2, scale=10))
+        for k, d in MATMUL_SHAPES:
+            mode1 = k == d and k <= 3
+            kh, ko = (d, k) if mode1 else (k, d)
+            for which in (1, 2, 3):
+                def g_mb(b, s, k=k, d=d, kh=kh, ko=ko, dt=dt):
+                    j = 0.3 * vecs(b, k, dt, s, k=d) + 2 * torch.eye(k, d, device=DEV, dtype=dt)
+                    return dict(j=j, h=spd(b, kh, dt, s + 1), g=vecs(b, ko * (ko + 1) // 2, dt, s + 2))
+
+                def run_mb(i, which=which):
+                    dj, dh = A.matmul_backward(i["j"], i["h"], i["g"], which)
+                    return torch.cat([p for p in (None if dj is None else dj.flatten(-2), dh) if p is not None], -1)
+
+                cases.append(Case(f"matmul_backward_w{which}_{t}_k{k}_d{d}", dt, g_mb, run_mb,
+                                  lambda i, k=k, d=d, which=which: _matmul_backward(i, k, d, which), scale=10,
+                                  extra=dict(mag=True)))
+    return cases
+
+
 _CASES = None
 
 
 def all_cases():
     global _CASES
     if _CASES is None:
-        _CASES = {c.name: c for c in _sym_cases() + _dense_cases()}
+        _CASES = {c.name: c for c in _sym_cases() + _dense_cases() + _grad_cases()}
     return _CASES
 
 
@@ -558,6 +676,13 @@ def worst_error(case, ins, out):
         if case.extra.get("dot"):      # a sum of products: error relative to the sum of their magnitudes
             den = (sl["u"].double() * sl["w"].double()).abs().sum(-1, keepdim=True)
             err = ((out[c:c + CHUNK].double() - want).abs() / den.clamp_min(1e-300)).max()
+        elif case.extra.get("mag"):    # sums of products of random signs: norm-wise, relative to the same
+            # formula on the magnitudes of the inputs (a record whose entries all nearly cancel has no exact digits)
+            den = case.ref({k: v.abs() for k, v in sl.items()})
+            dims = tuple(range(-case.rec, 0))
+            num = (out[c:c + CHUNK].double() - want).pow(2).sum(dims).sqrt()
+            err = (num / den.pow(2).sum(dims).sqrt().clamp_min(1e-300)).max()
+            del den
         else:
             err = _rel(out[c:c + CHUNK], want, case.rec, sl.get(case.addend) if case.addend else None)
         worst = torch.maximum(worst, err)
@@ -591,14 +716,17 @@ def run_case(case):
         warp = case.extra.get("warp")
         if warp:
             assert path == 2 and sh["kind"] == 0, (case.name, path, sh)
+        elif case.extra.get("strided"):
+            assert path == 0 and sh["kind"] == 0, (case.name, path, sh)
         elif _dense_aligned(ins) and not (case.extra.get("many") and sh["kind"] == 0):
             # (the many-right-hand-sides kernel stages only when three warps' buffers fit shared memory)
             assert path != 0, f"{case.name} ({label}, batch {batch}) fell off the TMA path: {sh}"
+            assert path == case.extra.get("path", path), (case.name, label, path, sh)
         if label.startswith("small"):
             small_batch = batch
             if sh_expected is not None and label != "none":
                 assert _geom(sh) == _geom(sh_expected)
-        if label != "none" and not warp:
+        if label != "none" and not warp and not case.extra.get("strided"):
             want_w = 1 if label.endswith("w1") else 2
             assert _wraps(sh) >= want_w, (case.name, label, sh)
             if sh["kind"] == 4:   # whole warp tiles; the < 32 systems after them go to the one-thread kernel
@@ -690,7 +818,8 @@ def test_more_than_2_31_elements():
 
 SWITCH_CASES = ["solve_S_auto_none_f32_n3", "invert_auto_f32_n6", "batchinv_f64_n4", "addmatvec_E_f32_n7",
                 "batchinv_f64_n8", "batchinv_f64_n9", "batchinv_f64_n10", "solvevec_f32_n10",
-                "lmdiv_lu_k5_f64_n4", "lmdiv_lu_k12_f32_n6", "rmdiv_k1_f64_n8"]
+                "lmdiv_lu_k5_f64_n4", "lmdiv_lu_k12_f32_n6", "rmdiv_k1_f64_n8",
+                "dense_inv_backward_f32_n4", "matmul_backward_w3_f32_k6_d6", "tsolve_lu_k1_f64_n8"]
 
 
 def _digest(t):
